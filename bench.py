@@ -62,6 +62,10 @@ def parse():
                     help="after the headline measurement also time BASELINE north_star's point (concert hall ~5 M triangles, "
                          "10 485 760 path pairs, depth 32, sharded over the N GPUs) and report it under 'north_star'; auto = at N = 8")
     ap.add_argument("--north-star-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one computed to DIR (either --impl): histogram.npy "
+                         "(float64 energies, [sources][bands][bins]) and ir.npy (float32 impulse responses, "
+                         "[sources][channels][samples])")
     return ap.parse_args()
 
 
@@ -151,11 +155,18 @@ def cpu_oracle_rate(args, n_paths, threads, repeats=1, seed=SEED0):
         t0 = time.perf_counter()
         per_source = max(1, n_paths // len(sc.sources))      # n_paths = path pairs over all sources
         h, st = S.trace(cfg, sc.sources, sc.listener, per_source, args.depth, seed + r, n_threads=threads)
-        for si in range(len(sc.sources)):
-            po.build_ir(cfg, h[si], per_source)
+        irs = [po.build_ir(cfg, h[si], per_source) for si in range(len(sc.sources))]
         times.append(time.perf_counter() - t0)
-    st["hist"] = h                                           # of the last repeat (seed + repeats - 1): bench parity check
+    st["hist"], st["ir"] = h, np.stack(irs)                  # of the last repeat (seed + repeats - 1): parity check, dump
     return times, st
+
+
+def write_outputs(out_dir, hist, ir):
+    """--dump-outputs: histogram.npy = the Q32.32 histogram / 2^32 (float64, [sources][bands][bins]), ir.npy = the impulse
+    responses (float32, [sources][channels][samples]).  At most 64 sources x (64 KB + 384 KB), well under 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "histogram.npy"), np.asarray(hist, dtype=np.uint64).astype(np.float64) / 2.0 ** 32)
+    np.save(os.path.join(out_dir, "ir.npy"), np.ascontiguousarray(ir, dtype=np.float32))
 
 
 def run_reference(args):
@@ -166,6 +177,8 @@ def run_reference(args):
     sample = min(args.paths, 1 << 17)
     cpu_oracle_rate(args, sample, threads, repeats=max(1, min(args.warmup, 1)))
     times, st = cpu_oracle_rate(args, sample, threads, repeats=args.steps)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, st["hist"], st["ir"])
     total = sum(times)
     v = sample * args.steps / total
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -344,6 +357,13 @@ class Workload:
                          "source": prof.get("source")}
         return r
 
+    def dump_outputs(self, out_dir):
+        """rank 0, after time_device: the context's copy of the last timed step's histogram (summed over the ranks at N > 1)
+        and the impulse responses rebuilt from it by the same IR kernels (deterministic: the floats the step left on the
+        device, which the timed step does not read back)"""
+        ir = self.ctx.build_ir(0)[None] if self.NS == 1 else self.ctx.build_ir_all(self.NS)
+        write_outputs(out_dir, self.ctx.get_histogram(), ir)
+
     def close(self):
         self.ctx.close()
 
@@ -381,6 +401,8 @@ def run_b200(args):
     sc, ctx, D, NS_, B, Kb = wl.sc, wl.ctx, wl.D, wl.NS, wl.B, wl.Kb
     P_total = wl.P_total
     dev_ms, launches, clocks = wl.time_device(K, W)
+    if args.dump_outputs and rank == 0:
+        wl.dump_outputs(args.dump_outputs)
     value = P_total * K / (dev_ms * 1e-3)
     st = wl.stage_times(min(K, 5))
     roofline = wl.roofline(args, st, clocks)

@@ -170,6 +170,24 @@ def test_update_source_whole_reference_loop(po, scene_fn, seeds):
         assert any_ir
 
 
+@pytest.mark.parametrize("scene_fn, seed, tag", [(pin_scene, 1, "pin_seed1"), (closet_scene, 5, "closet_seed5")])
+def test_update_source_against_stored_reference_output(oracle, scene_fn, seed, tag):
+    """The same comparison without the reference tree: the oracle against the output of the reference's UpdateSource stored
+    in tests/golden/ref_ue_v1.npz (ray count, EnergyBuffer, and the IR where the reference produced one)."""
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_ue_v1.npz"))
+    verts, tri_mat, ab, src, lis = scene_fn()
+    S = oracle.Scene(verts, tri_mat, ab[:, 2:3].copy(), use_bvh=False)
+    h, st = S.trace(oracle.ue_pin_config(), [src], lis, 1000, 512, seed)
+    assert st["ext_rays"] + st["shadow_rays"] == int(g[tag + "_traces"])
+    e_ref = g[tag + "_energy"]
+    e_or = h[0, 0].astype(np.float64) / 2.0 ** 32 / 1000
+    assert e_ref.sum() > 0 and np.abs(e_ref - e_or).sum() / e_or.sum() < 2e-5
+    if tag + "_ir0" in g:
+        ir_ref = g[tag + "_ir0"]
+        ir_or = oracle.build_ir_from_energy(oracle.ue_pin_config(bin_ms=49.0 / 48.0), e_or.astype(np.float32))
+        assert ir_ref.any() and np.linalg.norm(ir_or[0] - ir_ref) / np.linalg.norm(ir_ref) < 1e-5
+
+
 def test_flush_energy_buffer_keeps_old_energy_in_the_engine(po):
     """FlushEnergyBuffer is EnergyBuffer.SetNumZeroed(NumBins) (COMP.h:76-79): the engine zero-fills only NEW elements, so once
     the buffer has its size a 'flush' clears nothing -- which is why the second flush at SUB.cpp:191 does not blank the IR in
