@@ -243,7 +243,7 @@ int fs_scene_set_triangles(fs_ctx* ctx, const float* verts, const uint32_t* tri_
         if (!(verts[i] == verts[i]) || fabsf(verts[i]) > 1e18f) return fail(ctx, FS_ERR_INVALID, "non-finite vertex");
     cudaFree(ctx->d_verts); cudaFree(ctx->d_tri_mat);
     ctx->d_verts = nullptr; ctx->d_tri_mat = nullptr;
-    ctx->n_tris = n_tris; ctx->committed = false; ctx->tris_set = false;
+    ctx->n_tris = n_tris; ctx->committed = false; ctx->tris_set = false; ctx->verts_dirty = false;
     if (n_tris) {
         CK(cudaMalloc(&ctx->d_verts, sizeof(float) * 9 * n_tris));
         CK(cudaMalloc(&ctx->d_tri_mat, sizeof(uint32_t) * n_tris));
@@ -415,6 +415,49 @@ int fs_scene_commit(fs_ctx* ctx)
     ctx->stats.bvh_max_leaf = ctx->bvh.max_leaf;
     apply_l2_policy(ctx);
     ctx->committed = true;
+    ctx->verts_dirty = false;
+    return FS_OK;
+}
+
+static bool host_is_pinned(const void* p);
+
+int fs_scene_update_vertices(fs_ctx* ctx, const float* verts, uint64_t first_tri, uint64_t n_tris)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!ctx->tris_set) return fail(ctx, FS_ERR_STATE, "fs_scene_update_vertices: call fs_scene_set_triangles first");
+    if (n_tris && !verts) return fail(ctx, FS_ERR_INVALID, "fs_scene_update_vertices: null array");
+    if (first_tri > ctx->n_tris || n_tris > ctx->n_tris - first_tri)
+        return fail(ctx, FS_ERR_INVALID, "fs_scene_update_vertices: triangle range outside the scene");
+    for (uint64_t i = 0; i < n_tris * 9; ++i)
+        if (!(verts[i] == verts[i]) || fabsf(verts[i]) > 1e18f) return fail(ctx, FS_ERR_INVALID, "non-finite vertex");
+    if (!n_tris) return FS_OK;
+    dev_guard g(ctx->device);
+    // stream-ordered after any trace still in flight, before the next refit.  A pageable source is staged by the driver
+    // before the call returns; a page-locked one is read by the copy engine later, so wait for it (the caller may reuse
+    // the buffer as soon as this returns)
+    CK(cudaMemcpyAsync(ctx->d_verts + first_tri * 9, verts, sizeof(float) * 9 * n_tris, cudaMemcpyHostToDevice, ctx->stream));
+    if (host_is_pinned(verts)) CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->committed) ctx->verts_dirty = true;
+    return FS_OK;
+}
+
+int fs_scene_refit(fs_ctx* ctx, float* cost_ratio_out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!ctx->committed) return fail(ctx, FS_ERR_STATE, "fs_scene_refit: call fs_scene_commit first");
+    nvtx_range nv("fs_scene_refit");
+    if (ctx->tune_w8) {                 // the 8-wide nodes (experiment knob FS_TUNE_W8) are rebuilt, not refitted
+        int rc = fs_scene_commit(ctx);
+        if (rc == FS_OK && cost_ratio_out) *cost_ratio_out = 1.0f;
+        return rc;
+    }
+    dev_guard g(ctx->device);
+    uint64_t launches = 0;
+    float ratio = 1.0f;
+    CK(fs_bvh_refit(ctx->stream, ctx->d_verts, &ctx->bvh, &launches, &ratio));
+    ctx->launches.fetch_add(launches);
+    ctx->verts_dirty = false;
+    if (cost_ratio_out) *cost_ratio_out = ratio;
     return FS_OK;
 }
 
@@ -477,6 +520,7 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
 {
     nvtx_range nv("fs_trace");
     if (!ctx->committed) return fail(ctx, FS_ERR_STATE, "fs_trace: call fs_scene_commit first");
+    if (ctx->verts_dirty) return fail(ctx, FS_ERR_STATE, "fs_trace: triangles were moved; call fs_scene_refit (or fs_scene_commit) first");
     if (!src_pos || !lis_pos || n_sources == 0) return fail(ctx, FS_ERR_INVALID, "fs_trace: null positions / no source");
     if (n_paths == 0) return fail(ctx, FS_ERR_INVALID, "fs_trace: n_paths must be > 0");
     if (max_depth > 1024) return fail(ctx, FS_ERR_INVALID, "fs_trace: max_depth > 1024");
@@ -719,6 +763,7 @@ static int debug_rays(fs_ctx* ctx, const float* rays, const float* tmax, uint64_
 {
     if (!ctx) return FS_ERR_INVALID;
     if (!ctx->committed) return fail(ctx, FS_ERR_STATE, "commit the scene first");
+    if (ctx->verts_dirty) return fail(ctx, FS_ERR_STATE, "triangles were moved; call fs_scene_refit (or fs_scene_commit) first");
     if (n == 0) return FS_OK;
     dev_guard g(ctx->device);
     float *d_rays = nullptr, *d_tmax = nullptr, *d_t = nullptr; uint32_t* d_tri = nullptr; uint8_t* d_hit = nullptr;

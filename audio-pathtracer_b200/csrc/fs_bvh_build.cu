@@ -46,6 +46,14 @@ __global__ void k_init_bounds(uint32_t* bounds)
     else if (threadIdx.x >= 12 && threadIdx.x < 15) bounds[threadIdx.x] = 0u;      // scene box max
 }
 
+// raw-vertex box of one triangle: the leaf boxes of the build and of fs_bvh_refit
+__device__ __forceinline__ void tri_box(const float* __restrict__ p, float4& lo, float4& hi)
+{
+    float x0 = p[0], y0 = p[1], z0 = p[2], x1 = p[3], y1 = p[4], z1 = p[5], x2 = p[6], y2 = p[7], z2 = p[8];
+    lo = make_float4(fminf(x0, fminf(x1, x2)), fminf(y0, fminf(y1, y2)), fminf(z0, fminf(z1, z2)), 0.f);
+    hi = make_float4(fmaxf(x0, fmaxf(x1, x2)), fmaxf(y0, fmaxf(y1, y2)), fmaxf(z0, fmaxf(z1, z2)), 0.f);
+}
+
 __global__ void k_tri_bounds(const float* __restrict__ verts, uint32_t n, float4* __restrict__ tlo,
                              float4* __restrict__ thi, uint32_t* __restrict__ bounds,
                              uint32_t* __restrict__ extent_ord)
@@ -55,12 +63,11 @@ __global__ void k_tri_bounds(const float* __restrict__ verts, uint32_t n, float4
     float blx = INFINITY, bly = INFINITY, blz = INFINITY, bhx = -INFINITY, bhy = -INFINITY, bhz = -INFINITY;
     bool valid = i < n;
     if (valid) {
-        const float* p = verts + (size_t)i * 9;
-        float x0 = p[0], y0 = p[1], z0 = p[2], x1 = p[3], y1 = p[4], z1 = p[5], x2 = p[6], y2 = p[7], z2 = p[8];
-        float lx = fminf(x0, fminf(x1, x2)), ly = fminf(y0, fminf(y1, y2)), lz = fminf(z0, fminf(z1, z2));
-        float hx = fmaxf(x0, fmaxf(x1, x2)), hy = fmaxf(y0, fmaxf(y1, y2)), hz = fmaxf(z0, fmaxf(z1, z2));
-        tlo[i] = make_float4(lx, ly, lz, 0.f);
-        thi[i] = make_float4(hx, hy, hz, 0.f);
+        float4 lo, hi;
+        tri_box(verts + (size_t)i * 9, lo, hi);
+        const float lx = lo.x, ly = lo.y, lz = lo.z, hx = hi.x, hy = hi.y, hz = hi.z;
+        tlo[i] = lo;
+        thi[i] = hi;
         blx = lx; bly = ly; blz = lz; bhx = hx; bhy = hy; bhz = hz;
         cx = 0.5f * lx + 0.5f * hx; cy = 0.5f * ly + 0.5f * hy; cz = 0.5f * lz + 0.5f * hz;
         ext = fmaxf(fmaxf(fmaxf(fabsf(lx), fabsf(hx)), fmaxf(fabsf(ly), fabsf(hy))), fmaxf(fabsf(lz), fabsf(hz)));
@@ -217,6 +224,23 @@ k_sort_scatter(const uint64_t* __restrict__ keys_in, const uint32_t* __restrict_
 // ---------------------------------------------------------------------------------------------
 // tree
 // ---------------------------------------------------------------------------------------------
+// the 64 B triangle record of sorted position j and its (normal, material) record: the build (k_pack) and the refit
+// (k_refit_tris) share this arithmetic, so a refitted record is bit-identical to a freshly built one
+__device__ __forceinline__ void pack_tri(const float* __restrict__ verts, uint32_t id, uint32_t mat, uint32_t j,
+                                         float4* __restrict__ tris, float4* __restrict__ tri_nm)
+{
+    const float* p = verts + (size_t)id * 9;
+    fs_vec3 v0 = fs_mk(p[0], p[1], p[2]);
+    fs_vec3 e1 = fs_mk(p[3] - p[0], p[4] - p[1], p[5] - p[2]);
+    fs_vec3 e2 = fs_mk(p[6] - p[0], p[7] - p[1], p[8] - p[2]);
+    fs_vec3 nn = fs_tri_normal(e1, e2);
+    tris[(size_t)j * 4 + 0] = make_float4(v0.x, v0.y, v0.z, nn.x);
+    tris[(size_t)j * 4 + 1] = make_float4(e1.x, e1.y, e1.z, nn.y);
+    tris[(size_t)j * 4 + 2] = make_float4(e2.x, e2.y, e2.z, nn.z);
+    tris[(size_t)j * 4 + 3] = make_float4(__uint_as_float(id), __uint_as_float(mat), 0.f, 0.f);
+    tri_nm[j] = make_float4(nn.x, nn.y, nn.z, __uint_as_float(mat));
+}
+
 __global__ void k_pack(const float* __restrict__ verts, const uint32_t* __restrict__ mats,
                        const uint32_t* __restrict__ sorted_ids, uint32_t n,
                        const float4* __restrict__ tlo, const float4* __restrict__ thi,
@@ -227,19 +251,10 @@ __global__ void k_pack(const float* __restrict__ verts, const uint32_t* __restri
     uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= n) return;
     uint32_t id = sorted_ids[j];
-    const float* p = verts + (size_t)id * 9;
-    fs_vec3 v0 = fs_mk(p[0], p[1], p[2]);
-    fs_vec3 e1 = fs_mk(p[3] - p[0], p[4] - p[1], p[5] - p[2]);
-    fs_vec3 e2 = fs_mk(p[6] - p[0], p[7] - p[1], p[8] - p[2]);
-    fs_vec3 nn = fs_tri_normal(e1, e2);
     const uint32_t mat = mats[id];
-    tris[(size_t)j * 4 + 0] = make_float4(v0.x, v0.y, v0.z, nn.x);
-    tris[(size_t)j * 4 + 1] = make_float4(e1.x, e1.y, e1.z, nn.y);
-    tris[(size_t)j * 4 + 2] = make_float4(e2.x, e2.y, e2.z, nn.z);
-    tris[(size_t)j * 4 + 3] = make_float4(__uint_as_float(id), __uint_as_float(mat), 0.f, 0.f);
+    pack_tri(verts, id, mat, j, tris, tri_nm);
     tri_orig[j] = id;
     tri_mat[j] = mat;
-    tri_nm[j] = make_float4(nn.x, nn.y, nn.z, __uint_as_float(mat));
     bb_lo[(n - 1) + j] = tlo[id];
     bb_hi[(n - 1) + j] = thi[id];
 }
@@ -521,12 +536,13 @@ __device__ __forceinline__ uint4 quant_box(float lox, float hix, float loy, floa
 // big, often-hit boxes are the ones that get resolved one level further.  collapse = 0: the four grandchildren
 // (a leaf child leaves a slot empty).  Child references stay BVH2 node indices, so every BVH2 node can be emitted
 // independently; the ones no wide node refers to are simply never visited.
-struct cbox { float lx, hx, ly, hy, lz, hz; int ref; };
+// src: where the box was loaded from, BVH2 node * 2 + side (the provenance of a wide-node slot, see fs_bvh_refit)
+struct cbox { float lx, hx, ly, hy, lz, hz; int ref, src; };
 __device__ __forceinline__ void load_children(const float4* __restrict__ nodes, int i, cbox& a, cbox& b)
 {
     const float4 n0 = nodes[(size_t)i * 4], n1 = nodes[(size_t)i * 4 + 1], n2 = nodes[(size_t)i * 4 + 2], n3 = nodes[(size_t)i * 4 + 3];
-    a.lx = n0.x; a.hx = n0.y; a.ly = n0.z; a.hy = n0.w; a.lz = n2.x; a.hz = n2.y; a.ref = __float_as_int(n3.x);
-    b.lx = n1.x; b.hx = n1.y; b.ly = n1.z; b.hy = n1.w; b.lz = n2.z; b.hz = n2.w; b.ref = __float_as_int(n3.y);
+    a.lx = n0.x; a.hx = n0.y; a.ly = n0.z; a.hy = n0.w; a.lz = n2.x; a.hz = n2.y; a.ref = __float_as_int(n3.x); a.src = 2 * i;
+    b.lx = n1.x; b.hx = n1.y; b.ly = n1.z; b.hy = n1.w; b.lz = n2.z; b.hz = n2.w; b.ref = __float_as_int(n3.y); b.src = 2 * i + 1;
 }
 __device__ __forceinline__ float cbox_area(const cbox& c)
 {
@@ -535,7 +551,7 @@ __device__ __forceinline__ float cbox_area(const cbox& c)
 }
 
 __global__ void k_emit4(uint32_t n_inner, const float4* __restrict__ nodes, const float* __restrict__ grid,
-                        uint4* __restrict__ wnodes, int collapse)
+                        uint4* __restrict__ wnodes, int* __restrict__ wsrc, int collapse)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_inner) return;
@@ -558,8 +574,10 @@ __global__ void k_emit4(uint32_t n_inner, const float4* __restrict__ nodes, cons
         if (r1 >= 0) { load_children(nodes, r1, c[1], c[k]); ++k; }
         if (r0 >= 0) { load_children(nodes, r0, c[0], c[k]); ++k; }
     }
-    for (int j = 0; j < 4; ++j)
+    for (int j = 0; j < 4; ++j) {
         wnodes[(size_t)i * 4 + j] = (j < k) ? quant_box(c[j].lx, c[j].hx, c[j].ly, c[j].hy, c[j].lz, c[j].hz, c[j].ref, grid) : EMPTY;
+        wsrc[(size_t)i * 4 + j] = (j < k) ? c[j].src : -1;
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -583,7 +601,8 @@ __global__ void k_wide_count(const uint4* __restrict__ src, const int* __restric
     cnt[t] = c;
 }
 
-__global__ void k_wide_place(const uint4* __restrict__ src, uint4* __restrict__ dst, const int* __restrict__ frontier, uint32_t nf,
+__global__ void k_wide_place(const uint4* __restrict__ src, uint4* __restrict__ dst, const int* __restrict__ src_prov,
+                             int* __restrict__ dst_prov, const int* __restrict__ frontier, uint32_t nf,
                              const uint32_t* __restrict__ off, uint32_t level_base, int* __restrict__ next_frontier)
 {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -595,6 +614,7 @@ __global__ void k_wide_place(const uint4* __restrict__ src, uint4* __restrict__ 
         uint4 u = p[j];
         if (wide_is_inner(u.w)) { next_frontier[o] = (int)u.w; u.w = level_base + nf + o; ++o; }
         q[j] = u;
+        dst_prov[(size_t)(level_base + t) * 4 + j] = src_prov[(size_t)frontier[t] * 4 + j];
     }
 }
 
@@ -712,15 +732,17 @@ __device__ __forceinline__ int dp_cut(const float4* __restrict__ nodes, const fl
 
 // the 4-wide nodes with the children chosen by the table instead of greedily (FS_TUNE_COLLAPSE bit 4)
 __global__ void k_emit4_dp(uint32_t n_inner, const float4* __restrict__ nodes, const float* __restrict__ T, const float* __restrict__ grid,
-                           uint4* __restrict__ wnodes)
+                           uint4* __restrict__ wnodes, int* __restrict__ wsrc)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_inner) return;
     const uint4 EMPTY = make_uint4(0x0000ffffu, 0x0000ffffu, 0x0000ffffu, 0x7fffffffu);
     cbox c[4];
     const int k = dp_cut<4>(nodes, T, (int)i, c);
-    for (int j = 0; j < 4; ++j)
+    for (int j = 0; j < 4; ++j) {
         wnodes[(size_t)i * 4 + j] = (j < k) ? quant_box(c[j].lx, c[j].hx, c[j].ly, c[j].hy, c[j].lz, c[j].hz, c[j].ref, grid) : EMPTY;
+        wsrc[(size_t)i * 4 + j] = (j < k) ? c[j].src : -1;
+    }
 }
 
 // T = null: greedy collapse (open the inner child with the largest box until there are eight slots)
@@ -854,7 +876,7 @@ __device__ __forceinline__ cbox cbox_union(const cbox& a, const cbox& b, int ref
 {
     cbox u;
     u.lx = fminf(a.lx, b.lx); u.hx = fmaxf(a.hx, b.hx); u.ly = fminf(a.ly, b.ly); u.hy = fmaxf(a.hy, b.hy);
-    u.lz = fminf(a.lz, b.lz); u.hz = fmaxf(a.hz, b.hz); u.ref = ref;
+    u.lz = fminf(a.lz, b.lz); u.hz = fmaxf(a.hz, b.hz); u.ref = ref; u.src = -1;
     return u;
 }
 
@@ -939,16 +961,19 @@ __global__ void k_sah_cost(uint32_t n_inner, const float4* __restrict__ nodes, d
 }
 
 // single-triangle scene: root whose second child is a far-away point box (never entered in practice)
-__global__ void k_emit_single(const float4* __restrict__ bb_lo, const float4* __restrict__ bb_hi,
-                              float4* __restrict__ nodes)
+__device__ __forceinline__ void emit_single(float4 l0, float4 h0, float4* __restrict__ nodes)
 {
-    float4 l0 = bb_lo[0], h0 = bb_hi[0];
     float pad = box_pad(l0, h0);
     const float F = 1e30f;
     nodes[0] = make_float4(l0.x - pad, h0.x + pad, l0.y - pad, h0.y + pad);
     nodes[1] = make_float4(F, F, F, F);
     nodes[2] = make_float4(l0.z - pad, h0.z + pad, F, F);
     nodes[3] = make_float4(__int_as_float(~0), __int_as_float(~0), 0.f, 0.f);
+}
+__global__ void k_emit_single(const float4* __restrict__ bb_lo, const float4* __restrict__ bb_hi,
+                              float4* __restrict__ nodes)
+{
+    emit_single(bb_lo[0], bb_hi[0], nodes);
 }
 
 // BFS copy of the top of the tree; children inside the copy get FS_TOP_FLAG | local index.
@@ -981,6 +1006,91 @@ __global__ void k_leaf_stats(int n, const int2* __restrict__ ranges, uint32_t* _
     if (i >= n - 1) return;
     int cnt = ranges[i].y - ranges[i].x + 1;
     if (cnt <= leaf_max) atomicMax(max_leaf, (uint32_t)cnt);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Refit (fs_bvh_refit): the committed topology with boxes recomputed from moved triangles.  Every box of the build is
+// box_pad(unpadded box) and every unpadded box a fminf / fmaxf union of raw triangle bounds: exact and independent of
+// the order of the union, so refitting unchanged triangles reproduces the committed arrays bit for bit.
+// ---------------------------------------------------------------------------------------------
+__global__ void k_refit_tris(uint32_t n, const float* __restrict__ verts, const uint32_t* __restrict__ tri_orig,
+                             const uint32_t* __restrict__ tri_mat, float4* __restrict__ tris, float4* __restrict__ tri_nm)
+{
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    pack_tri(verts, tri_orig[j], tri_mat[j], j, tris, tri_nm);
+}
+
+// unpadded box of child reference r: a leaf ~(j << 3 | cnt - 1) is the union of the raw bounds of sorted triangles
+// j .. j + cnt - 1, an inner child the box its own thread stored before it released this node
+__device__ __forceinline__ void refit_child(int r, const float* __restrict__ verts, const uint32_t* __restrict__ tri_orig,
+                                            const float4* ubox, float4& lo, float4& hi)
+{
+    if (r >= 0) { lo = __ldcg(ubox + 2 * (size_t)r); hi = __ldcg(ubox + 2 * (size_t)r + 1); return; }
+    const uint32_t e = (uint32_t)~r, first = e >> 3, cnt = (e & 7u) + 1u;
+    tri_box(verts + (size_t)tri_orig[first] * 9, lo, hi);
+    for (uint32_t k = 1; k < cnt; ++k) {
+        float4 l, h;
+        tri_box(verts + (size_t)tri_orig[first + k] * 9, l, h);
+        lo = make_float4(fminf(lo.x, l.x), fminf(lo.y, l.y), fminf(lo.z, l.z), 0.f);
+        hi = make_float4(fmaxf(hi.x, h.x), fmaxf(hi.y, h.y), fmaxf(hi.z, h.z), 0.f);
+    }
+}
+
+// bottom-up over the BVH2 with one arrival counter per node (as k_wide_dp): a thread starts at every node without inner
+// children; the last of a node's inner children to finish carries on with the parent.  Child entries are written in the
+// float form of k_ploc_merge / k_emit; the child references (node word 3) are left alone.
+__global__ void k_refit_nodes(uint32_t n_inner, const float* __restrict__ verts, const uint32_t* __restrict__ tri_orig,
+                              const int* __restrict__ parent, const uint32_t* __restrict__ need, uint32_t* __restrict__ arrive,
+                              float4* __restrict__ nodes, float4* ubox)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_inner || need[i] != 0u) return;
+    int n = (int)i;
+    for (;;) {
+        const float4 n3 = nodes[(size_t)n * 4 + 3];
+        float4 l0, h0, l1, h1;
+        refit_child(__float_as_int(n3.x), verts, tri_orig, ubox, l0, h0);
+        refit_child(__float_as_int(n3.y), verts, tri_orig, ubox, l1, h1);
+        const float p0 = box_pad(l0, h0), p1 = box_pad(l1, h1);
+        nodes[(size_t)n * 4 + 0] = make_float4(l0.x - p0, h0.x + p0, l0.y - p0, h0.y + p0);
+        nodes[(size_t)n * 4 + 1] = make_float4(l1.x - p1, h1.x + p1, l1.y - p1, h1.y + p1);
+        nodes[(size_t)n * 4 + 2] = make_float4(l0.z - p0, h0.z + p0, l1.z - p1, h1.z + p1);
+        __stcg(ubox + 2 * (size_t)n, make_float4(fminf(l0.x, l1.x), fminf(l0.y, l1.y), fminf(l0.z, l1.z), 0.f));
+        __stcg(ubox + 2 * (size_t)n + 1, make_float4(fmaxf(h0.x, h1.x), fmaxf(h0.y, h1.y), fmaxf(h0.z, h1.z), 0.f));
+        __threadfence();
+        const int p = parent[n];
+        if (p < 0) break;
+        if (atomicAdd(arrive + p, 1u) + 1u < need[p]) break;
+        __threadfence();
+        n = p;
+    }
+}
+
+// single-triangle scene: the root of k_emit_single, from the moved triangle
+__global__ void k_refit_single(const float* __restrict__ verts, const uint32_t* __restrict__ tri_orig, float4* __restrict__ nodes)
+{
+    float4 lo, hi;
+    tri_box(verts + (size_t)tri_orig[0] * 9, lo, hi);
+    emit_single(lo, hi, nodes);
+}
+
+// every slot of the wide nodes re-quantised from the BVH2 child entry it was made from (wsrc = node * 2 + side); the
+// child reference (u.w) and the empty slots stay as they are
+__global__ void k_requant4(uint32_t n_slots, const float4* __restrict__ nodes, const int* __restrict__ wsrc,
+                           const float* __restrict__ grid, uint4* __restrict__ wnodes)
+{
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n_slots) return;
+    const int src = wsrc[s];
+    if (src < 0) return;
+    cbox a, b;
+    load_children(nodes, src >> 1, a, b);
+    const cbox& c = (src & 1) ? b : a;
+    const uint4 q = quant_box(c.lx, c.hx, c.ly, c.hy, c.lz, c.hz, 0, grid);
+    uint4 u = wnodes[s];
+    u.x = q.x; u.y = q.y; u.z = q.z;
+    wnodes[s] = u;
 }
 
 }  // namespace
@@ -1093,13 +1203,15 @@ fail:
 }
 
 // sparse (one wide node per BVH2 node) -> dense breadth-first array; *dense_out is allocated here
-static cudaError_t wide_compact(cudaStream_t st, uint32_t n_inner, const uint4* sparse, uint4** dense_out, uint32_t* n_wide_out,
-                                uint64_t* launches)
+// (the slot provenance sparse_prov is carried along into *dense_prov_out, also allocated here)
+static cudaError_t wide_compact(cudaStream_t st, uint32_t n_inner, const uint4* sparse, const int* sparse_prov, uint4** dense_out,
+                                int** dense_prov_out, uint32_t* n_wide_out, uint64_t* launches)
 {
     cudaError_t err = cudaSuccess;
     int* fr[2] = {nullptr, nullptr};
     uint32_t *cnt = nullptr, *off = nullptr, *tile_sums = nullptr, *total = nullptr;
     uint4* dense = nullptr;
+    int* dense_prov = nullptr;
     const int TPB = 256;
     uint32_t nf = 1, base = 0;
     int pp = 0;
@@ -1109,22 +1221,23 @@ static cudaError_t wide_compact(cudaStream_t st, uint32_t n_inner, const uint4* 
     BCHECK(cudaMalloc(&tile_sums, 4ull * ((n_inner + SCAN_TILE - 1) / SCAN_TILE + 2)));
     BCHECK(cudaMalloc(&total, 4));
     BCHECK(cudaMalloc(&dense, sizeof(uint4) * 4ull * n_inner));
+    BCHECK(cudaMalloc(&dense_prov, sizeof(int) * 4ull * n_inner));
     BCHECK(cudaMemcpyAsync(fr[0], &zero, 4, cudaMemcpyHostToDevice, st));
     while (nf) {
         const uint32_t g = (nf + TPB - 1) / TPB;
         uint32_t next = 0;
         k_wide_count<<<g, TPB, 0, st>>>(sparse, fr[pp], nf, cnt); ++*launches;
         scan_u32(st, cnt, off, nf, tile_sums, total, launches);
-        k_wide_place<<<g, TPB, 0, st>>>(sparse, dense, fr[pp], nf, off, base, fr[pp ^ 1]); ++*launches;
+        k_wide_place<<<g, TPB, 0, st>>>(sparse, dense, sparse_prov, dense_prov, fr[pp], nf, off, base, fr[pp ^ 1]); ++*launches;
         BCHECK(cudaMemcpyAsync(&next, total, 4, cudaMemcpyDeviceToHost, st));
         BCHECK(cudaStreamSynchronize(st));
         base += nf; nf = next; pp ^= 1;
         if (base + nf > n_inner) { err = cudaErrorUnknown; goto fail; }     // cannot happen for a tree
     }
     BCHECK(cudaGetLastError());
-    *dense_out = dense; dense = nullptr; *n_wide_out = base;
+    *dense_out = dense; dense = nullptr; *dense_prov_out = dense_prov; dense_prov = nullptr; *n_wide_out = base;
 fail:
-    cudaFree(fr[0]); cudaFree(fr[1]); cudaFree(cnt); cudaFree(off); cudaFree(tile_sums); cudaFree(total); cudaFree(dense);
+    cudaFree(fr[0]); cudaFree(fr[1]); cudaFree(cnt); cudaFree(off); cudaFree(tile_sums); cudaFree(total); cudaFree(dense); cudaFree(dense_prov);
     return err;
 }
 
@@ -1227,6 +1340,7 @@ cudaError_t fs_bvh_build(cudaStream_t st, const float* d_verts, const uint32_t* 
     BCHECK(cudaMalloc(&queue, 4ull * FS_TOP_CAP));
     BCHECK(cudaMalloc(&out->nodes, sizeof(float4) * 4ull * n_inner));
     BCHECK(cudaMalloc(&out->wnodes, sizeof(uint4) * 4ull * n_inner));
+    BCHECK(cudaMalloc(&out->wsrc, sizeof(int) * 4ull * n_inner));
     BCHECK(cudaMalloc(&grid, sizeof(float) * 8));
     BCHECK(cudaMalloc(&out->tris, sizeof(float4) * 4ull * n));
     BCHECK(cudaMalloc(&out->tri_orig, 4ull * n));
@@ -1341,20 +1455,21 @@ cudaError_t fs_bvh_build(cudaStream_t st, const float* d_verts, const uint32_t* 
             (e4 = cudaMemsetAsync(arr, 0, 4ull * n_inner, st)) == cudaSuccess) {
             k_w8_parents<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, out->nodes, par, need);
             k_wide_dp<4><<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, out->nodes, par, need, arr, T4);
-            k_emit4_dp<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, out->nodes, T4, grid, out->wnodes);
+            k_emit4_dp<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, out->nodes, T4, grid, out->wnodes, out->wsrc);
             *launches += 3;
             e4 = cudaStreamSynchronize(st);
         }
         cudaFree(T4); cudaFree(par); cudaFree(need); cudaFree(arr);
         BCHECK(e4);
     } else {
-        k_emit4<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, out->nodes, grid, out->wnodes, collapse & 1); ++*launches;
+        k_emit4<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, out->nodes, grid, out->wnodes, out->wsrc, collapse & 1); ++*launches;
     }
     out->n_wide = n_inner;
     if (!(collapse & 2)) {                          // FS_TUNE_COLLAPSE bit 1 keeps the sparse layout (A/B)
-        uint4* dense = nullptr; uint32_t n_wide = 0;
-        BCHECK(wide_compact(st, n_inner, out->wnodes, &dense, &n_wide, launches));
+        uint4* dense = nullptr; int* dense_prov = nullptr; uint32_t n_wide = 0;
+        BCHECK(wide_compact(st, n_inner, out->wnodes, out->wsrc, &dense, &dense_prov, &n_wide, launches));
         cudaFree(out->wnodes); out->wnodes = dense; out->n_wide = n_wide;
+        cudaFree(out->wsrc); out->wsrc = dense_prov;
     }
     {
         cudaResourceDesc rd; memset(&rd, 0, sizeof(rd));
@@ -1403,5 +1518,60 @@ void fs_bvh_free(fs_bvh_device* b)
     if (b->wnodes_tex) cudaDestroyTextureObject(b->wnodes_tex);
     cudaFree(b->w8nodes); cudaFree(b->tris8); cudaFree(b->tri8_map);
     cudaFree(b->nodes); cudaFree(b->wnodes); cudaFree(b->tris); cudaFree(b->tri_orig); cudaFree(b->tri_mat); cudaFree(b->tri_nm); cudaFree(b->top_nodes);
+    cudaFree(b->wsrc);
+    cudaFree(b->rf.parent); cudaFree(b->rf.need); cudaFree(b->rf.arrive); cudaFree(b->rf.ubox); cudaFree(b->rf.queue); cudaFree(b->rf.misc);
     memset(b, 0, sizeof(*b));
+}
+
+// Refit of a committed tree (see fs_internal.h).  Stream-ordered on `st`; the one synchronisation is the read-back of the
+// quantisation grid and the two costs.  The 8-wide nodes (FS_TUNE_W8) are not refitted: the caller rebuilds them.
+cudaError_t fs_bvh_refit(cudaStream_t st, const float* d_verts, fs_bvh_device* b, uint64_t* launches, float* cost_ratio)
+{
+    cudaError_t err = cudaSuccess;
+    const uint32_t n = b->n_tris, n_inner = b->n_inner;
+    const int TPB = 256;
+    fs_bvh_device::refit_scratch& r = b->rf;
+    struct { double cost[2]; float grid[8]; uint32_t n_top; } h;
+    if (cost_ratio) *cost_ratio = 1.0f;
+    if (n == 0) return cudaSuccess;
+    if (!r.misc) {
+        // first refit: the topology tables, and the cost of the tree as committed before anything overwrites it
+        BCHECK(cudaMalloc(&r.parent, 4ull * n_inner));
+        BCHECK(cudaMalloc(&r.need, 4ull * n_inner));
+        BCHECK(cudaMalloc(&r.arrive, 4ull * n_inner));
+        BCHECK(cudaMalloc(&r.ubox, sizeof(float4) * 2ull * n_inner));
+        BCHECK(cudaMalloc(&r.queue, 4ull * FS_TOP_CAP));
+        BCHECK(cudaMalloc(&r.misc, sizeof(h)));
+        // -1 everywhere first: the inner nodes inside a multi-triangle leaf (LBVH) have no parent; their subtrees are
+        // refitted as trees of their own, which keeps the whole node array equal to a fresh build's
+        BCHECK(cudaMemsetAsync(r.parent, 0xff, 4ull * n_inner, st));
+        BCHECK(cudaMemsetAsync(r.misc, 0, sizeof(h), st));
+        k_w8_parents<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, b->nodes, r.parent, r.need);
+        k_sah_cost<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, b->nodes, (double*)r.misc);
+        *launches += 2;
+        BCHECK(cudaMemcpyAsync(&r.cost0, r.misc, sizeof(double), cudaMemcpyDeviceToHost, st));
+    }
+    BCHECK(cudaMemsetAsync(r.arrive, 0, 4ull * n_inner, st));
+    BCHECK(cudaMemsetAsync((double*)r.misc + 1, 0, sizeof(double), st));
+    k_refit_tris<<<(n + TPB - 1) / TPB, TPB, 0, st>>>(n, d_verts, b->tri_orig, b->tri_mat, b->tris, b->tri_nm);
+    if (n == 1) k_refit_single<<<1, 1, 0, st>>>(d_verts, b->tri_orig, b->nodes);
+    else k_refit_nodes<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, d_verts, b->tri_orig, r.parent, r.need, r.arrive, b->nodes, r.ubox);
+    k_sah_cost<<<(n_inner + TPB - 1) / TPB, TPB, 0, st>>>(n_inner, b->nodes, (double*)r.misc + 1);
+    {
+        float* d_grid = (float*)((char*)r.misc + offsetof(decltype(h), grid));
+        k_quant_grid<<<1, 32, 0, st>>>(b->nodes, d_grid);
+        const uint32_t n_slots = 4u * b->n_wide;
+        k_requant4<<<(n_slots + TPB - 1) / TPB, TPB, 0, st>>>(n_slots, b->nodes, b->wsrc, d_grid, b->wnodes);
+        k_top_treelet<<<1, 32, 0, st>>>(b->nodes, n_inner, FS_TOP_CAP, b->top_nodes,
+                                        (uint32_t*)((char*)r.misc + offsetof(decltype(h), n_top)), r.queue);
+    }
+    *launches += 6;
+    BCHECK(cudaGetLastError());
+    BCHECK(cudaMemcpyAsync(&h, r.misc, sizeof(h), cudaMemcpyDeviceToHost, st));
+    BCHECK(cudaStreamSynchronize(st));
+    for (int a = 0; a < 3; ++a) { b->qbase[a] = h.grid[a]; b->qscale[a] = h.grid[3 + a]; }
+    b->n_top = h.n_top;
+    if (cost_ratio) *cost_ratio = r.cost0 > 0.0 ? (float)(h.cost[1] / r.cost0) : 1.0f;
+fail:
+    return err;
 }

@@ -32,6 +32,17 @@ struct fs_bvh_device {
     uint32_t* tri8_map;          // position in tris8 -> position in tris (the index hit records carry)
     uint32_t n_w8;
     float extent;
+    int* wsrc;                   // [n_wide][4] provenance of each wide-node slot: BVH2 node * 2 + side (-1: empty slot)
+    // fs_bvh_refit scratch, allocated at the first refit (callers that never refit pay nothing)
+    struct refit_scratch {
+        int* parent;             // [n_inner] BVH2 parent (-1: root)
+        uint32_t* need;          // [n_inner] inner children
+        uint32_t* arrive;        // [n_inner] arrival counters of the bottom-up pass
+        float4* ubox;            // [n_inner][2] unpadded box of every inner node
+        int* queue;              // [FS_TOP_CAP] k_top_treelet
+        void* misc;              // double cost[2] (as committed, refitted) | float grid[8] | uint32 n_top
+        double cost0;            // surface-area cost of the tree as committed
+    } rf;
 };
 
 cudaError_t fs_bvh_build(cudaStream_t st, const float* d_verts, const uint32_t* d_mats, uint64_t n_tris,
@@ -40,6 +51,10 @@ cudaError_t fs_bvh_build(cudaStream_t st, const float* d_verts, const uint32_t* 
                                                     bit 2 also build the 8-wide compressed nodes, bit 3 greedy instead of optimal 8-wide collapse,
                                                     bit 4 optimal (dynamic programme) instead of greedy 4-wide collapse*/);
 void fs_bvh_free(fs_bvh_device* b);
+// Refits the committed tree `b` to new positions of its triangles (d_verts, same count and order as at the build): topology
+// kept, triangle records, BVH2 boxes, quantisation grid, 4-wide node boxes and the treelet recomputed; one host
+// synchronisation (the grid).  *cost_ratio = surface-area cost of the refitted BVH2 / that of the tree as committed.
+cudaError_t fs_bvh_refit(cudaStream_t st, const float* d_verts, fs_bvh_device* b, uint64_t* launches, float* cost_ratio);
 
 // device-side counters of one trace call
 struct fs_dev_counters {
@@ -134,6 +149,7 @@ struct fs_ctx {
     std::vector<float> mat_absorption;
     std::vector<float> mat_transmission, mat_scattering, mat_thickness_cm;
     bool mats_set, tris_set, committed;
+    bool verts_dirty;           // fs_scene_update_vertices on a committed scene, not yet refitted: the tree no longer bounds the triangles
     fs_bvh_device bvh;
     // trace: batches alternate between lanes -- while one batch's traversal launch drains its slowest rays, the other
     // lane's kernels fill the SMs

@@ -230,6 +230,25 @@ int fs_multi_scene_commit(fs_multi* m)
     if (rc) for (auto& e : errs) if (!e.empty()) { mfail(rc, e); break; }
     return rc;
 }
+int fs_multi_scene_update_vertices(fs_multi* m, const float* verts, uint64_t first_tri, uint64_t n_tris)
+{
+    if (!m) return FS_ERR_INVALID;
+    std::vector<std::string> errs(m->n);
+    int rc = on_all(m, [&](uint32_t i) { int r = fs_scene_update_vertices(m->ctx[i], verts, first_tri, n_tris); if (r) errs[i] = fs_last_error(m->ctx[i]); return r; });
+    if (rc) for (auto& e : errs) if (!e.empty()) { mfail(rc, e); break; }
+    return rc;
+}
+// every device refits its own copy (identical trees, identical results); the cost ratio is device 0's
+int fs_multi_scene_refit(fs_multi* m, float* cost_ratio_out)
+{
+    if (!m) return FS_ERR_INVALID;
+    std::vector<std::string> errs(m->n);
+    std::vector<float> ratio(m->n, 1.0f);
+    int rc = on_all(m, [&](uint32_t i) { int r = fs_scene_refit(m->ctx[i], &ratio[i]); if (r) errs[i] = fs_last_error(m->ctx[i]); return r; });
+    if (rc) for (auto& e : errs) if (!e.empty()) { mfail(rc, e); break; }
+    if (rc == FS_OK && cost_ratio_out) *cost_ratio_out = ratio[0];
+    return rc;
+}
 
 // One IR update's trace over all devices (UpdateSource, SUB.cpp:128-195, for n_sources sources): shard, trace, peer-store,
 // sum.  On return the work is ENQUEUED; the reduced histogram is context 0's (stream-ordered: fs_build_ir* on context 0

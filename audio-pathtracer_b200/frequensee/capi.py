@@ -26,6 +26,7 @@ FLAG_IR_NORMALIZE = 1024
 ABI_SYMBOLS = [
     "fs_default_config", "fs_create", "fs_destroy", "fs_last_error", "fs_set_stream", "fs_synchronize",
     "fs_scene_set_triangles", "fs_scene_set_materials", "fs_scene_set_materials_ex", "fs_scene_commit",
+    "fs_scene_update_vertices", "fs_scene_refit",
     "fs_trace", "fs_update", "fs_trace_range_device", "fs_trace_range", "fs_trace_debug",
     "fs_debug_closest_hits", "fs_debug_any_hits",
     "fs_build_ir", "fs_build_ir_to", "fs_build_ir_all", "fs_build_ir_bands", "fs_build_ir_from_energy", "fs_set_histogram", "fs_set_histogram_device",
@@ -35,6 +36,7 @@ ABI_SYMBOLS = [
     "fs_debug_rfft", "fs_get_stats",
     "fs_multi_create", "fs_multi_destroy", "fs_multi_last_error", "fs_multi_device_count", "fs_multi_context",
     "fs_multi_scene_set_triangles", "fs_multi_scene_set_materials", "fs_multi_scene_set_materials_ex", "fs_multi_scene_commit",
+    "fs_multi_scene_update_vertices", "fs_multi_scene_refit",
     "fs_multi_trace", "fs_multi_last_ms", "fs_multi_synchronize",
 ]
 
@@ -147,6 +149,8 @@ def load():
     L.fs_scene_set_materials.argtypes = [vp, vp, u32, u32]
     L.fs_scene_set_materials_ex.argtypes = [vp, vp, vp, vp, vp, u32, u32]
     L.fs_scene_commit.argtypes = [vp]
+    L.fs_scene_update_vertices.argtypes = [vp, vp, u64, u64]
+    L.fs_scene_refit.argtypes = [vp, C.POINTER(C.c_float)]
     L.fs_trace.argtypes = [vp, vp, u32, vp, u64, u32, u64, vp]
     L.fs_update.argtypes = [vp, vp, u32, vp, u64, u32, u64, vp, vp]
     L.fs_trace_range_device.argtypes = [vp, vp, u32, vp, u64, u64, u64, u32, u64, vp, i32]
@@ -189,6 +193,8 @@ def load():
     L.fs_multi_scene_set_materials.argtypes = [vp, vp, u32, u32]
     L.fs_multi_scene_set_materials_ex.argtypes = [vp, vp, vp, vp, vp, u32, u32]
     L.fs_multi_scene_commit.argtypes = [vp]
+    L.fs_multi_scene_update_vertices.argtypes = [vp, vp, u64, u64]
+    L.fs_multi_scene_refit.argtypes = [vp, C.POINTER(C.c_float)]
     L.fs_multi_trace.argtypes = [vp, vp, u32, vp, u64, u32, u64, vp]
     L.fs_multi_last_ms.argtypes = [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     L.fs_multi_synchronize.argtypes = [vp]
@@ -268,6 +274,18 @@ class Context:
         self._ck(self.L.fs_scene_set_materials_ex(self.h, absorption.ctypes.data, *[a.ctypes.data if a is not None else None for a in opt],
                                                    absorption.shape[0], absorption.shape[1]))
         self._ck(self.L.fs_scene_commit(self.h))
+
+    def update_vertices(self, verts, first_tri=0):
+        """moves triangles [first_tri, first_tri + len(verts)) of the scene (same count, same materials); on a committed
+        scene the move takes effect at refit() (or a full commit)"""
+        verts = np.ascontiguousarray(verts, dtype=np.float32).reshape(-1, 3, 3)
+        self._ck(self.L.fs_scene_update_vertices(self.h, verts.ctypes.data, first_tri, len(verts)))
+
+    def refit(self):
+        """refits the committed BVH to the moved triangles; returns its surface-area cost over that of the tree as committed"""
+        r = C.c_float(1.0)
+        self._ck(self.L.fs_scene_refit(self.h, C.byref(r)))
+        return r.value
 
     def set_stream(self, stream_ptr):
         self._ck(self.L.fs_set_stream(self.h, C.c_void_p(stream_ptr)))
@@ -495,6 +513,16 @@ class MultiContext:
         self._ck(self.L.fs_multi_scene_set_triangles(self.h, verts.ctypes.data, tri_mat.ctypes.data, len(verts)))
         self._ck(self.L.fs_multi_scene_set_materials(self.h, absorption.ctypes.data, absorption.shape[0], absorption.shape[1]))
         self._ck(self.L.fs_multi_scene_commit(self.h))
+
+    def update_vertices(self, verts, first_tri=0):
+        verts = np.ascontiguousarray(verts, dtype=np.float32).reshape(-1, 3, 3)
+        self._ck(self.L.fs_multi_scene_update_vertices(self.h, verts.ctypes.data, first_tri, len(verts)))
+
+    def refit(self):
+        """every device refits its copy; returns device 0's cost ratio"""
+        r = C.c_float(1.0)
+        self._ck(self.L.fs_multi_scene_refit(self.h, C.byref(r)))
+        return r.value
 
     def trace(self, src_pos, lis_pos, n_paths, max_depth, seed, want_hist=True):
         src, lis = Context._pos(src_pos, lis_pos)

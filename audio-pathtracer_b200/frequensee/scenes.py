@@ -301,6 +301,75 @@ def concert_hall(seed=5, target_tris=5_000_000, n_bands=8):
                  {"seed": seed, "size": tuple(size)})
 
 
+# ---------------------------------------------------------------------------------------------
+# moving geometry: two rooms joined by a doorway with a hinged door
+# ---------------------------------------------------------------------------------------------
+def door_rooms(seed=11, n_bands=8, wall_tess=16, n_blobs=4):
+    """Two 6 x 8 x 3 m rooms side by side (x < 6 and x > 6.2), a 0.2 m dividing wall with a 1.0 x 2.1 m doorway at
+    y = 3.5 .. 4.5, and a 4 cm wooden door hinged on the vertical line (6.1, 3.5).  The source is in the first room, the
+    listener in the second; each room holds a few upholstered blobs and cabinets.  meta["door"] = (first triangle, count)
+    of the door, the last part of the scene; door_verts() swings it.  Surfaces are opaque (no transmission by default), so
+    with the door closed no path connects the two rooms and the listener's histogram is empty."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    X0, W, X1, Y, Z = 6.0, 0.2, 12.2, 8.0, 3.0
+    y0, y1, zd = 3.5, 4.5, 2.1
+    src = np.array([2.0, 2.0, 1.4])
+    lis = np.array([10.0, 6.0, 1.6])
+    parts, mats = [], []
+
+    def add(t, m):
+        parts.append(t)
+        mats.append(np.full(len(t), m, dtype=np.uint32) if np.isscalar(m) else m)
+
+    t, face = box((0, 0, 0), (X1, Y, Z), wall_tess)
+    add(t, np.array([6, 6, 2, 6, 3, 6], dtype=np.uint32)[face])
+    for x in (X0, X0 + W):                                          # the two faces of the dividing wall around the doorway
+        add(patch([x, 0, 0], [0, y0, 0], [0, 0, Z], 6, 6), 6)
+        add(patch([x, y1, 0], [0, Y - y1, 0], [0, 0, Z], 6, 6), 6)
+        add(patch([x, y0, zd], [0, y1 - y0, 0], [0, 0, Z - zd], 2, 2), 6)
+    add(patch([X0, y0, 0], [W, 0, 0], [0, 0, zd], 2, 6), 6)        # jambs and lintel
+    add(patch([X0, y1, 0], [W, 0, 0], [0, 0, zd], 2, 6), 6)
+    add(patch([X0, y0, zd], [W, 0, 0], [0, y1 - y0, 0], 2, 2), 6)
+    for lo_x, hi_x in ((0.0, X0), (X0 + W, X1)):                   # furniture, clear of the source, listener and door swing
+        placed = 0
+        while placed < n_blobs:
+            r = rng.uniform(0.25, 0.5)
+            c = np.array([rng.uniform(lo_x + r + 0.1, hi_x - r - 0.1), rng.uniform(r + 0.1, Y - r - 0.1), rng.uniform(r, 1.2)])
+            if min(np.linalg.norm(c - src), np.linalg.norm(c - lis), np.linalg.norm(c[:2] - [X0 + W / 2, 4.0])) < r + 1.4:
+                continue
+            add(uv_sphere(c, r, 20, 40, (1.0, 1.0, rng.uniform(0.6, 1.0))), int(rng.choice([5, 4, 3])))
+            placed += 1
+        for _ in range(3):
+            w = rng.uniform(0.4, 1.0, size=2)
+            h = rng.uniform(0.6, 2.0)
+            lo = np.array([rng.uniform(lo_x + 0.1, hi_x - w[0] - 0.1), rng.choice([0.1, Y - w[1] - 0.1]), 0.02])
+            add(box(lo, lo + [w[0], w[1], h], 3)[0], int(rng.choice([1, 7])))
+    first = sum(len(p) for p in parts)
+    door, _ = box((X0 + W / 2 - 0.02, y0, 0.0), (X0 + W / 2 + 0.02, y1, zd), 6)
+    add(door, 1)
+    verts = np.concatenate(parts, axis=0)
+    tri_mat = np.concatenate(mats)
+    return Scene("door_rooms", verts, tri_mat, absorption_table(n_bands), [src], lis,
+                 {"seed": seed, "size": (X1, Y, Z), "door": (first, len(door)), "hinge": (X0 + W / 2, y0)})
+
+
+def door_verts(scene, angle_deg):
+    """the scene's vertices with the door rotated by angle_deg about its hinge (positive: it swings into the listener's
+    room); 0 = closed, the door as built"""
+    verts = scene.verts.copy()
+    if angle_deg == 0:
+        return verts
+    first, n = scene.meta["door"]
+    hx, hy = scene.meta["hinge"]
+    a = np.deg2rad(angle_deg)
+    d = verts[first:first + n].astype(np.float64)
+    dx, dy = d[..., 0] - hx, d[..., 1] - hy
+    d[..., 0] = hx + dx * np.cos(a) + dy * np.sin(a)
+    d[..., 1] = hy - dx * np.sin(a) + dy * np.cos(a)
+    verts[first:first + n] = d.astype(np.float32)
+    return verts
+
+
 def by_name(name, **kw):
     return {"shoebox": shoebox, "furnished_room": furnished_room, "mine_tunnels": mine_tunnels,
-            "concert_hall": concert_hall}[name](**kw)
+            "concert_hall": concert_hall, "door_rooms": door_rooms}[name](**kw)

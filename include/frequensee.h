@@ -191,6 +191,24 @@ int fs_scene_set_materials_ex(fs_ctx* ctx, const float* absorption, const float*
 /* builds the BVH on the device: Morton codes, radix sort, PLOC agglomeration (search radius chosen by surface-area cost),
  * 4-wide quantised nodes in a dense breadth-first array.  One-time cost per scene: 0.2 s for 1 M triangles. */
 int fs_scene_commit(fs_ctx* ctx);
+/* moving geometry.  replaces: the engine's scene query seeing WorldDynamic actors at their current transform
+ * (SUB.cpp:331-334: GeneratePath / ConnectSubpaths query Pawn + WorldStatic + WorldDynamic objects, so a door that swings is
+ * heard by the next UpdateSource).
+ * fs_scene_update_vertices overwrites the positions of triangles [first_tri, first_tri + n_tris) of the scene set by
+ * fs_scene_set_triangles (verts: [n_tris][3][3] float metres; same count, same material ids).  Copies at call time,
+ * enqueued on the context stream.  FS_ERR_STATE before fs_scene_set_triangles; FS_ERR_INVALID for a range outside the scene
+ * or a non-finite / > 1e18 coordinate (checked before anything is copied: a rejected call changes nothing).
+ * On a committed scene the positions take effect at the next fs_scene_refit (or fs_scene_commit = full rebuild); until
+ * then fs_trace*, fs_update and fs_debug_*_hits return FS_ERR_STATE. */
+int fs_scene_update_vertices(fs_ctx* ctx, const float* verts, uint64_t first_tri, uint64_t n_tris);
+/* Refits the committed BVH to the current triangle positions: topology kept, every box and triangle record recomputed,
+ * the quantisation grid re-derived.  Results are bit-identical to a fresh fs_scene_commit of the same positions (the
+ * closest hit does not depend on the tree); only the traversal cost changes as the tree degrades.  FS_ERR_STATE if the
+ * scene is not committed.  One host synchronisation (the grid is read back: trace parameters carry it by value).
+ * cost_ratio_out (may be NULL): surface-area cost of the refitted BVH2 over that of the tree as committed, so the caller
+ * can decide when a full fs_scene_commit pays off.  With the experiment knob FS_TUNE_W8 (8-wide nodes) this is a full
+ * fs_scene_commit and the ratio is 1. */
+int fs_scene_refit(fs_ctx* ctx, float* cost_ratio_out);
 
 /* ---- BDPT update ---------------------------------------------------------------------------
  * replaces: UAudioRayTracingSubsystem::UpdateSource (SUB.cpp:128-195) = GenerateFullPaths
@@ -321,6 +339,9 @@ int fs_multi_scene_set_materials(fs_multi* m, const float* absorption, uint32_t 
 int fs_multi_scene_set_materials_ex(fs_multi* m, const float* absorption, const float* transmission, const float* scattering,
                                     const float* thickness_cm, uint32_t n_materials, uint32_t n_bands);
 int fs_multi_scene_commit(fs_multi* m);
+/* fs_scene_update_vertices / fs_scene_refit on every device (SUB.cpp:331-334); the ratio is that of device 0 */
+int fs_multi_scene_update_vertices(fs_multi* m, const float* verts, uint64_t first_tri, uint64_t n_tris);
+int fs_multi_scene_refit(fs_multi* m, float* cost_ratio_out);
 /* fs_trace over all devices (UpdateSource, SUB.cpp:128-195).  Enqueues and returns; hist_out (host [S][B][K]) may be NULL,
  * non-NULL synchronises. */
 int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const float lis_pos[3], uint64_t n_paths,
