@@ -1093,6 +1093,162 @@ __global__ void k_requant4(uint32_t n_slots, const float4* __restrict__ nodes, c
     wnodes[s] = u;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Parallel reinsertion on the BVH2 (Bittner et al. 2013; on the GPU: Meister & Bittner 2018).  A move takes the subtree
+// N out of its parent P (the sibling S takes P's place under the grandparent G) and puts it back as the sibling of some
+// other subtree X, reusing P as their new parent.  Unlike a rotation it can move N anywhere in the tree.  Slots are
+// child entries, slot = 2 * node + side.  One iteration:
+//   k_ri_search  one thread per candidate slot (N's box at least `thr`): the best X by the change of the surface-area
+//                cost (sum of all non-root boxes).  The removal saves area(P) plus the shrinkage of P's ancestors below
+//                the lowest common ancestor of P and X; the insertion adds area(X u N) plus the growth of X's ancestors
+//                below it.  Depth-first from the ancestors' off-path children with the branch-and-bound of Bittner et al.
+//                (whatever lies below X pays at least area(N) on top of the growth down to X).
+//   k_ri_lock    a move locks the nodes on the paths from P and from X's parent up to their common ancestor, and G:
+//                u64 atomicMax of (saving, slot), so the winner of every node is independent of the thread order
+//   k_ri_apply   moves that hold all their locks rewrite the child references of G, X's parent and P.  Disjoint lock
+//                paths keep the moves independent (no cycles: a move into N's subtree crosses P).
+// then the boxes are refitted bottom-up (k_refit_nodes: exact unions, padded as PLOC pads them).  The root stays node 0.
+// ---------------------------------------------------------------------------------------------
+#ifndef FS_REINSERT_ITERS
+#define FS_REINSERT_ITERS 32        // default iteration cap (FS_TUNE_REINSERT overrides)
+#endif
+constexpr int RI_MAXD = 64;         // ancestors of P a search may use; deeper candidates are skipped
+constexpr int RI_STACK = 128;       // search stack; a full stack drops branches (the search stays a valid heuristic)
+
+__device__ __forceinline__ cbox slot_box(const float4* __restrict__ nodes, int slot)
+{
+    cbox a, b;
+    load_children(nodes, slot >> 1, a, b);
+    return (slot & 1) ? b : a;
+}
+__device__ __forceinline__ int slot_ref(const float4* nodes, int slot)
+{
+    return ((const int*)(nodes + (size_t)(slot >> 1) * 4 + 3))[slot & 1];
+}
+
+// area histogram of the candidate slots (12 high bits of the ordered float): picks the size threshold of the candidates
+__global__ void k_ri_hist(uint32_t n_inner, const float4* __restrict__ nodes, uint32_t* __restrict__ hist)
+{
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x + 2u;
+    if (s >= 2u * n_inner) return;
+    atomicAdd(hist + (f2ord(cbox_area(slot_box(nodes, (int)s))) >> 20), 1u);
+}
+
+__global__ void k_ri_search(uint32_t n_inner, const float4* __restrict__ nodes, const int* __restrict__ parent, float thr,
+                            float min_gain, float* __restrict__ mv_gain, int* __restrict__ mv_dst)
+{
+    const int s = (int)(blockIdx.x * blockDim.x + threadIdx.x) + 2;       // the root's slots never move (P = root has no G)
+    if (s >= 2 * (int)n_inner) return;
+    mv_dst[s] = -1;
+    const int P = s >> 1;
+    cbox a, b;
+    load_children(nodes, P, a, b);
+    const cbox N = (s & 1) ? b : a, S = (s & 1) ? a : b;
+    const float aN = cbox_area(N);
+    if (!(aN >= thr)) return;
+    struct ent { int slot; float c, g; };
+    ent st[RI_STACK];
+    int sp = 0;
+    // up from P: the off-path child of every ancestor, with the saving of the removal when that ancestor is the common one
+    cbox cur = S;                   // the box of the current ancestor once N has left it
+    float g = 0.0f;
+    for (int c = P, d = 0;; ++d) {
+        const int u = parent[c];
+        if (u < 0) break;
+        if (d == RI_MAXD) return;
+        cbox l, r;
+        load_children(nodes, u, l, r);
+        const int cs = (l.ref == c) ? 0 : 1;
+        const cbox& cb = cs ? r : l;
+        const cbox& ob = cs ? l : r;
+        g += (c == P) ? cbox_area(cb) : cbox_area(cb) - cbox_area(cur);
+        cur = cbox_union(cur, ob, 0);
+        st[sp++] = ent{2 * u + (cs ^ 1), 0.0f, g};
+        c = u;
+    }
+    for (int i = 0, j = sp - 1; i < j; ++i, --j) { const ent t = st[i]; st[i] = st[j]; st[j] = t; }   // nearest first off the stack
+    if (S.ref >= 0) {               // inside S (S itself is where N is now): S grows by N
+        const float c0 = cbox_area(cbox_union(S, N, 0)) - cbox_area(S), aP = st[sp - 1].g;
+        st[sp++] = ent{2 * S.ref, c0, aP};
+        st[sp++] = ent{2 * S.ref + 1, c0, aP};
+    }
+    float best = -min_gain * aN; int bdst = -1;       // a move must save a little more than float noise
+    while (sp) {
+        const ent e = st[--sp];
+        if (e.c + aN - e.g >= best) continue;
+        const cbox X = slot_box(nodes, e.slot);
+        const float u = cbox_area(cbox_union(X, N, 0));
+        const float tot = e.c + u - e.g;
+        if (tot < best) { best = tot; bdst = e.slot; }
+        if (X.ref >= 0) {
+            const float c2 = e.c + u - cbox_area(X);
+            if (c2 + aN - e.g < best && sp + 2 <= RI_STACK) {
+                st[sp++] = ent{2 * X.ref + 1, c2, e.g};
+                st[sp++] = ent{2 * X.ref, c2, e.g};
+            }
+        }
+    }
+    mv_gain[s] = -best;
+    mv_dst[s] = bdst;
+}
+
+// the lock set of move (slot s -> slot dst): P .. common ancestor, X's parent .. below it, and G; visits each node with f
+template <typename F>
+__device__ __forceinline__ void ri_lockset(const int* __restrict__ parent, int s, int dst, F f)
+{
+    int up[RI_MAXD + 2]; int d = 0;
+    for (int c = s >> 1; c >= 0 && d < RI_MAXD + 2; c = parent[c]) up[d++] = c;      // P, G, ..., root (the search bounded it)
+    int lca = 0;
+    for (int v = dst >> 1; v >= 0; v = parent[v]) {
+        bool on = false;
+        for (int k = 0; k < d; ++k) if (up[k] == v) { on = true; break; }
+        if (on) { lca = v; break; }
+        f(v);
+    }
+    for (int k = 0; k < d; ++k) { f(up[k]); if (up[k] == lca) break; }
+    if (d > 1) f(up[1]);
+}
+
+__device__ __forceinline__ unsigned long long ri_key(float gain, int s)
+{
+    return ((unsigned long long)__float_as_uint(gain) << 32) | (unsigned long long)(uint32_t)s;     // gain > 0: ordered as uint
+}
+
+__global__ void k_ri_lock(uint32_t n_inner, const int* __restrict__ parent, const float* __restrict__ mv_gain,
+                          const int* __restrict__ mv_dst, unsigned long long* __restrict__ lock)
+{
+    const int s = (int)(blockIdx.x * blockDim.x + threadIdx.x) + 2;
+    if (s >= 2 * (int)n_inner || mv_dst[s] < 0) return;
+    const unsigned long long key = ri_key(mv_gain[s], s);
+    ri_lockset(parent, s, mv_dst[s], [&](int v) { atomicMax(lock + v, key); });
+}
+
+__device__ __forceinline__ void set_ref(float4* nodes, int slot, int ref)
+{
+    ((int*)(nodes + (size_t)(slot >> 1) * 4 + 3))[slot & 1] = ref;
+}
+
+__global__ void k_ri_apply(uint32_t n_inner, const int* __restrict__ parent, const float* __restrict__ mv_gain,
+                           const int* __restrict__ mv_dst, const unsigned long long* __restrict__ lock, float4* nodes,
+                           uint32_t* __restrict__ n_moved)
+{
+    const int s = (int)(blockIdx.x * blockDim.x + threadIdx.x) + 2;
+    if (s >= 2 * (int)n_inner) return;
+    const int dst = mv_dst[s];
+    if (dst < 0) return;
+    const unsigned long long key = ri_key(mv_gain[s], s);
+    bool own = true;
+    ri_lockset(parent, s, dst, [&](int v) { own = own && (lock[v] == key); });
+    if (!own) return;
+    const int P = s >> 1, G = parent[P];
+    const int Nr = slot_ref(nodes, s), Sr = slot_ref(nodes, s ^ 1), Xr = slot_ref(nodes, dst);
+    set_ref(nodes, 2 * G + (slot_ref(nodes, 2 * G) == P ? 0 : 1), Sr);
+    set_ref(nodes, dst, P);
+    set_ref(nodes, 2 * P, Nr);
+    set_ref(nodes, 2 * P + 1, Xr);
+    atomicAdd(n_moved, 1u);
+}
+
 }  // namespace
 
 
@@ -1199,6 +1355,87 @@ static cudaError_t bvh2_rotate(cudaStream_t st, uint32_t n_inner, float4* nodes,
     BCHECK(cudaGetLastError());
 fail:
     cudaFree(order); cudaFree(cnt); cudaFree(off); cudaFree(tile_sums); cudaFree(total); cudaFree(d_done);
+    return err;
+}
+
+// Up to `iters` reinsertion iterations over the BVH2 in `nodes` (see k_ri_search).  The candidates are the largest 10 %
+// of the child boxes of the tree as it comes in.  The loop stops early when an iteration moves nothing or saves less
+// than 0.01 % of the surface-area cost (on the room an iteration saves < 0.1 % from the 9th on, because few moves win all
+// their locks, yet iterations 9-32 still take another 3 % off the 4-wide nodes' summed area); an iteration that raised
+// the cost (its moves were judged on the boxes before the others moved) is undone, so the result never costs more than
+// the input.
+static cudaError_t bvh2_reinsert(cudaStream_t st, uint32_t n_inner, const float* d_verts, const uint32_t* tri_orig,
+                                 float4* nodes, int iters, uint64_t* launches)
+{
+    cudaError_t err = cudaSuccess;
+    int *parent = nullptr, *mv_dst = nullptr;
+    uint32_t *need = nullptr, *arrive = nullptr, *hist = nullptr;
+    float4 *ubox = nullptr, *backup = nullptr;
+    float* mv_gain = nullptr;
+    unsigned long long* lock = nullptr;
+    char* misc = nullptr;                         // [0] cost (double), [8] moves (u32)
+    const int TPB = 256;
+    const uint32_t n_slots = 2u * n_inner - 2u, gs = (n_slots + TPB - 1) / TPB, gi = (n_inner + TPB - 1) / TPB;
+    std::vector<uint32_t> h_hist(4096);
+    double cost0 = 0.0, prev = 0.0;
+    int it = 0;
+    uint32_t total_moves = 0;
+    float thr = 0.0f;
+    BCHECK(cudaMalloc(&parent, 4ull * n_inner)); BCHECK(cudaMalloc(&need, 4ull * n_inner)); BCHECK(cudaMalloc(&arrive, 4ull * n_inner));
+    BCHECK(cudaMalloc(&ubox, sizeof(float4) * 2ull * n_inner)); BCHECK(cudaMalloc(&backup, sizeof(float4) * 4ull * n_inner));
+    BCHECK(cudaMalloc(&lock, 8ull * n_inner));
+    BCHECK(cudaMalloc(&mv_gain, 4ull * 2 * n_inner)); BCHECK(cudaMalloc(&mv_dst, 4ull * 2 * n_inner));
+    BCHECK(cudaMalloc(&hist, 4ull * 4096)); BCHECK(cudaMalloc(&misc, 16));
+    BCHECK(cudaMemsetAsync(hist, 0, 4ull * 4096, st));
+    BCHECK(cudaMemsetAsync(misc, 0, 16, st));
+    k_ri_hist<<<gs, TPB, 0, st>>>(n_inner, nodes, hist);
+    k_sah_cost<<<gi, TPB, 0, st>>>(n_inner, nodes, (double*)misc);
+    *launches += 2;
+    BCHECK(cudaMemcpyAsync(h_hist.data(), hist, 4ull * 4096, cudaMemcpyDeviceToHost, st));
+    BCHECK(cudaMemcpyAsync(&cost0, misc, 8, cudaMemcpyDeviceToHost, st));
+    BCHECK(cudaStreamSynchronize(st));
+    {
+        uint64_t acc = 0;
+        for (int bin = 4095; bin >= 0; --bin) {
+            acc += h_hist[bin];
+            if (acc * 10 >= n_slots) { thr = ord2f((uint32_t)bin << 20); break; }
+        }
+    }
+    prev = cost0;
+    for (it = 0; it < iters; ++it) {
+        struct { double cost; uint32_t moved; } h;
+        BCHECK(cudaMemsetAsync(lock, 0, 8ull * n_inner, st));
+        BCHECK(cudaMemsetAsync(misc, 0, 16, st));
+        k_w8_parents<<<gi, TPB, 0, st>>>(n_inner, nodes, parent, need);
+        k_ri_search<<<gs, TPB, 0, st>>>(n_inner, nodes, parent, thr, 1e-5f, mv_gain, mv_dst);
+        k_ri_lock<<<gs, TPB, 0, st>>>(n_inner, parent, mv_gain, mv_dst, lock);
+        BCHECK(cudaMemcpyAsync(backup, nodes, sizeof(float4) * 4ull * n_inner, cudaMemcpyDeviceToDevice, st));
+        k_ri_apply<<<gs, TPB, 0, st>>>(n_inner, parent, mv_gain, mv_dst, lock, nodes, (uint32_t*)(misc + 8));
+        BCHECK(cudaMemsetAsync(arrive, 0, 4ull * n_inner, st));
+        k_w8_parents<<<gi, TPB, 0, st>>>(n_inner, nodes, parent, need);
+        k_refit_nodes<<<gi, TPB, 0, st>>>(n_inner, d_verts, tri_orig, parent, need, arrive, nodes, ubox);
+        k_sah_cost<<<gi, TPB, 0, st>>>(n_inner, nodes, (double*)misc);
+        *launches += 7;
+        BCHECK(cudaMemcpyAsync(&h, misc, sizeof(h), cudaMemcpyDeviceToHost, st));
+        BCHECK(cudaStreamSynchronize(st));
+        BCHECK(cudaGetLastError());
+        if (h.moved == 0) break;
+        if (h.cost > prev) {
+            BCHECK(cudaMemcpyAsync(nodes, backup, sizeof(float4) * 4ull * n_inner, cudaMemcpyDeviceToDevice, st));
+            BCHECK(cudaStreamSynchronize(st));
+            break;
+        }
+        total_moves += h.moved;
+        const bool small = prev - h.cost < 1e-4 * prev;
+        prev = h.cost;
+        if (small) { ++it; break; }
+    }
+    if (getenv("FS_VERBOSE"))
+        fprintf(stderr, "[frequensee] reinsertion: %d iterations, %u moves, surface-area cost %.6g -> %.6g (%.2f %%)\n", it,
+                total_moves, cost0, prev, cost0 > 0.0 ? 100.0 * (prev - cost0) / cost0 : 0.0);
+fail:
+    cudaFree(parent); cudaFree(need); cudaFree(arrive); cudaFree(ubox); cudaFree(backup); cudaFree(lock);
+    cudaFree(mv_gain); cudaFree(mv_dst); cudaFree(hist); cudaFree(misc);
     return err;
 }
 
@@ -1438,6 +1675,12 @@ cudaError_t fs_bvh_build(cudaStream_t st, const float* d_verts, const uint32_t* 
                     fprintf(stderr, "[frequensee] %d rotation sweeps: %u rotations, surface-area cost %.6g\n", sweeps, n_rot, h_c);
                 }
             }
+        }
+        {
+            // FS_TUNE_REINSERT = most reinsertion iterations (0: off)
+            int iters = FS_REINSERT_ITERS;
+            if (const char* e = getenv("FS_TUNE_REINSERT")) { int v = atoi(e); if (v >= 0 && v <= 256) iters = v; }
+            if (iters && n >= 4096) BCHECK(bvh2_reinsert(st, n_inner, d_verts, out->tri_orig, out->nodes, iters, launches));
         }
     } else {
         k_karras<<<gb, TPB, 0, st>>>(keys0, (int)n, children, ranges, parent); ++*launches;
