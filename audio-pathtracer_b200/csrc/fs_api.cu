@@ -186,7 +186,7 @@ void fs_destroy(fs_ctx* ctx)
     cudaFree(ctx->d_bsdf_tab); cudaFree(ctx->d_lobes);
     fs_bvh_free(&ctx->bvh);
     cudaFree(ctx->d_verts); cudaFree(ctx->d_tri_mat); cudaFree(ctx->d_refl_over_pi);
-    cudaFree(ctx->d_hist); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg);
+    cudaFree(ctx->d_hist); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
     cudaFree(ctx->d_amp); cudaFree(ctx->d_energy);
     for (cudaEvent_t e : ctx->kev) cudaEventDestroy(e);
     for (cudaEvent_t e : ctx->tev) cudaEventDestroy(e);
@@ -503,6 +503,62 @@ static int ensure_hist(fs_ctx* ctx, uint32_t n_sources)
     return FS_OK;
 }
 
+// bookkeeping of the histogram that fs_build_ir* read: its source count and the path count of every source (per_source:
+// host [n_sources] after fs_trace_sources*, null = n_paths for all)
+static void set_hist_counts(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, const uint64_t* per_source)
+{
+    ctx->hist_n_paths = n_paths; ctx->hist_cur_sources = n_sources;
+    if (per_source) ctx->hist_src_paths.assign(per_source, per_source + n_sources);
+    else ctx->hist_src_paths.clear();
+}
+static uint64_t hist_paths(const fs_ctx* ctx, uint32_t source)
+{
+    return source < ctx->hist_src_paths.size() ? ctx->hist_src_paths[source] : ctx->hist_n_paths;
+}
+
+// per-source budgets (fs_trace_sources*) in the form trace_common takes: packed positions, offsets, depths, maxima
+struct fs_src_table {
+    std::vector<float> pos;          // [S][3]
+    std::vector<uint64_t> off;       // [S+1]: off[s] = first work index of source s, off[S] = G
+    std::vector<uint32_t> depth;     // [S]
+    std::vector<uint64_t> n_paths;   // [S]
+    uint64_t n_max; uint32_t d_max;
+};
+
+// validates a per-source call completely before anything is enqueued (the context is left as it was on every error)
+static int prepare_sources(fs_ctx* ctx, const char* who, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3],
+                           fs_src_table* t)
+{
+    std::string w(who);
+    if (!ctx->committed) return fail(ctx, FS_ERR_STATE, (w + ": call fs_scene_commit first").c_str());
+    if (ctx->verts_dirty) return fail(ctx, FS_ERR_STATE, (w + ": triangles were moved; call fs_scene_refit (or fs_scene_commit) first").c_str());
+    if (!src || !lis_pos || n_sources == 0) return fail(ctx, FS_ERR_INVALID, (w + ": null sources / listener or no source").c_str());
+    if ((uint64_t)n_sources * ctx->cfg.n_bins >= 0xffffffffull) return fail(ctx, FS_ERR_INVALID, (w + ": n_sources * n_bins too large").c_str());
+    const uint32_t flags = ctx->cfg.flags;
+    const uint32_t lim = (flags & FS_FLAG_MIS) ? 32u : (flags & FS_FLAG_CONNECT_ALL) ? 63u : 1024u;
+    t->pos.resize(3ull * n_sources); t->off.resize(n_sources + 1ull); t->depth.resize(n_sources); t->n_paths.resize(n_sources);
+    t->n_max = 0; t->d_max = 0;
+    uint64_t G = 0;
+    for (uint32_t s = 0; s < n_sources; ++s) {
+        const fs_source_desc& d = src[s];
+        if (d.n_paths == 0) return fail(ctx, FS_ERR_INVALID, (w + ": n_paths of source " + std::to_string(s) + " is 0").c_str());
+        if (d.max_depth > lim)
+            return fail(ctx, FS_ERR_INVALID, (w + ": max_depth of source " + std::to_string(s) + " > " + std::to_string(lim) +
+                                              " (the limit of this flag mode)").c_str());
+        if ((flags & FS_FLAG_SHARE_LISTENER) && d.max_depth != src[0].max_depth)
+            return fail(ctx, FS_ERR_INVALID, (w + ": FS_FLAG_SHARE_LISTENER needs the same max_depth for every source "
+                                                  "(one shared listener walk serves one ray budget)").c_str());
+        if (G + d.n_paths < G) return fail(ctx, FS_ERR_INVALID, (w + ": total path count overflows").c_str());
+        for (int a = 0; a < 3; ++a) t->pos[3ull * s + a] = d.pos[a];
+        t->off[s] = G; t->depth[s] = d.max_depth; t->n_paths[s] = d.n_paths;
+        G += d.n_paths;
+        if (d.n_paths > t->n_max) t->n_max = d.n_paths;
+        if (d.max_depth > t->d_max) t->d_max = d.max_depth;
+    }
+    t->off[n_sources] = G;
+    return FS_OK;
+}
+
 // the listener cache is [max_depth + 2][n_paths] float4; without room for it the shared keying still holds, the listener
 // subpaths are then simply traced in place by every batch
 static bool lis_cache_fits(fs_ctx* ctx, uint64_t n_paths, uint32_t max_depth)
@@ -514,9 +570,11 @@ static bool lis_cache_fits(fs_ctx* ctx, uint64_t n_paths, uint32_t max_depth)
     return need < 0.25 * (double)free_b;
 }
 
+// tab (per-source budgets, fs_trace_sources*): src_pos = tab->pos, n_paths = the largest budget, max_depth = the largest depth,
+// the work range is [0, G) with G = tab->off[S]; null = uniform budgets, G = n_sources * n_paths
 static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3],
                         uint64_t n_paths, uint64_t g_first, uint64_t g_count, uint32_t max_depth, uint64_t seed,
-                        unsigned long long* d_hist, fs_path_dbg* d_dbg)
+                        unsigned long long* d_hist, fs_path_dbg* d_dbg, const fs_src_table* tab = nullptr)
 {
     nvtx_range nv("fs_trace");
     if (!ctx->committed) return fail(ctx, FS_ERR_STATE, "fs_trace: call fs_scene_commit first");
@@ -524,7 +582,8 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
     if (!src_pos || !lis_pos || n_sources == 0) return fail(ctx, FS_ERR_INVALID, "fs_trace: null positions / no source");
     if (n_paths == 0) return fail(ctx, FS_ERR_INVALID, "fs_trace: n_paths must be > 0");
     if (max_depth > 1024) return fail(ctx, FS_ERR_INVALID, "fs_trace: max_depth > 1024");
-    if (g_first + g_count > (uint64_t)n_sources * n_paths) return fail(ctx, FS_ERR_INVALID, "fs_trace: work range exceeds n_sources * n_paths");
+    const uint64_t G = tab ? tab->off[n_sources] : (uint64_t)n_sources * n_paths;
+    if (g_first + g_count > G || g_first + g_count < g_first) return fail(ctx, FS_ERR_INVALID, "fs_trace: work range exceeds the sources' paths");
     if ((uint64_t)n_sources * ctx->cfg.n_bins >= 0xffffffffull) return fail(ctx, FS_ERR_INVALID, "fs_trace: n_sources * n_bins too large");
     // an overflow of the PREVIOUS trace that nobody has looked at yet: report it now if its flag has landed; if it is
     // still in flight the device flag is left set (reset_ovf = 0) so that this call's copy carries it
@@ -537,6 +596,16 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
         ctx->src_cap = n_sources;
     }
     CK(cudaMemcpyAsync(ctx->d_src_pos, src_pos, sizeof(float) * 3 * n_sources, cudaMemcpyHostToDevice, ctx->stream));
+    if (tab) {
+        if (ctx->src_tab_cap < n_sources) {
+            cudaFree(ctx->d_src_tab); ctx->d_src_tab = nullptr; ctx->src_tab_cap = 0;
+            CK(cudaMalloc(&ctx->d_src_tab, 12ull * n_sources + 8ull));
+            ctx->src_tab_cap = n_sources;
+        }
+        CK(cudaMemcpyAsync(ctx->d_src_tab, tab->off.data(), 8ull * (n_sources + 1ull), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync((char*)ctx->d_src_tab + 8ull * (n_sources + 1ull), tab->depth.data(), 4ull * n_sources,
+                           cudaMemcpyHostToDevice, ctx->stream));
+    }
     // equal batches: every bounce of a batch is a pair of launches whose cost has a fixed part (launch + the tail of the
     // slowest rays), so 1.25 M pairs run as 1 x 1.25 M or 2 x 0.63 M, never as 1 M + a 0.25 M remainder.
     // Batches alternate between up to tune_streams lanes (own stream + own wavefront buffers): a traversal launch ends
@@ -588,6 +657,7 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
     for (uint32_t l = 0; l < n_lanes; ++l) CK(fs_wave_alloc(ctx, &ctx->lanes[l], cap, max_depth));
     fs_trace_params tp;
     fill_params(ctx, &tp, lis_pos, n_paths, max_depth, seed);
+    tp.n_src = n_sources;
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
     ctx->kev_used = 0; ctx->tev_used = 0; ctx->stats.extend_launches = 0; ctx->stats.persistent_launches = 0;
     CK(fs_wave_reset_counters(ctx, reset_ovf));
@@ -610,6 +680,11 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
             CK(fs_wave_trace_batch(ctx, &ctx->lanes[0], tp, d_hist, nullptr));
         }
         tp.lis_mode = 2;
+    }
+    // per-source budgets: set after the listener pass, which traces max n_s listener subpaths of one uniform source
+    if (tab) {
+        tp.src_off = (const uint64_t*)ctx->d_src_tab;
+        tp.src_depth = (const uint32_t*)((const char*)ctx->d_src_tab + 8ull * (n_sources + 1ull));
     }
     if (n_lanes > 1) {
         CK(cudaEventRecord(ctx->ev_fork, ctx->stream));
@@ -698,7 +773,7 @@ int fs_trace(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float 
     rc = trace_common(ctx, src_pos, n_sources, lis_pos, n_paths, 0, (uint64_t)n_sources * n_paths, max_depth, seed,
                       ctx->d_hist, nullptr);
     if (rc) return rc;
-    ctx->hist_n_paths = n_paths; ctx->hist_cur_sources = n_sources;
+    set_hist_counts(ctx, n_sources, n_paths, nullptr);
     if (hist_out) {
         CK(cudaMemcpyAsync(hist_out, ctx->d_hist, 8 * hn, cudaMemcpyDeviceToHost, ctx->stream));
         return finish_stats(ctx);
@@ -731,7 +806,7 @@ int fs_trace_range(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const 
     CK(cudaMemcpyAsync(ctx->d_hist, hist_inout, 8 * hn, cudaMemcpyHostToDevice, ctx->stream));
     rc = trace_common(ctx, src_pos, n_sources, lis_pos, n_paths, g_first, g_count, max_depth, seed, ctx->d_hist, nullptr);
     if (rc) return rc;
-    ctx->hist_n_paths = n_paths; ctx->hist_cur_sources = n_sources;
+    set_hist_counts(ctx, n_sources, n_paths, nullptr);
     CK(cudaMemcpyAsync(hist_inout, ctx->d_hist, 8 * hn, cudaMemcpyDeviceToHost, ctx->stream));
     return finish_stats(ctx);
 }
@@ -753,7 +828,7 @@ int fs_trace_debug(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const 
     CK(cudaMemsetAsync(ctx->d_hist, 0, 8 * hn, ctx->stream));
     rc = trace_common(ctx, src_pos, n_sources, lis_pos, n_paths, g_first, g_count, max_depth, seed, ctx->d_hist, ctx->d_dbg);
     if (rc) return rc;
-    ctx->hist_n_paths = n_paths; ctx->hist_cur_sources = n_sources;
+    set_hist_counts(ctx, n_sources, n_paths, nullptr);
     CK(cudaMemcpyAsync(dbg_out, ctx->d_dbg, sizeof(fs_path_dbg) * g_count, cudaMemcpyDeviceToHost, ctx->stream));
     return finish_stats(ctx);
 }
@@ -820,7 +895,7 @@ int fs_set_histogram(fs_ctx* ctx, const uint64_t* hist, uint32_t n_sources, uint
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemcpyAsync(ctx->d_hist, hist, 8 * hn, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    ctx->hist_n_paths = n_paths; ctx->hist_cur_sources = n_sources;
+    set_hist_counts(ctx, n_sources, n_paths, nullptr);
     return FS_OK;
 }
 
@@ -833,7 +908,25 @@ int fs_set_histogram_device(fs_ctx* ctx, const void* d_hist, uint32_t n_sources,
     if (rc) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemcpyAsync(ctx->d_hist, d_hist, 8 * hn, cudaMemcpyDeviceToDevice, ctx->stream));
-    ctx->hist_n_paths = n_paths; ctx->hist_cur_sources = n_sources;
+    set_hist_counts(ctx, n_sources, n_paths, nullptr);
+    return FS_OK;
+}
+
+int fs_set_histogram_sources_device(fs_ctx* ctx, const void* d_hist, uint32_t n_sources, const uint64_t* n_paths)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!d_hist || !n_paths || n_sources == 0) return fail(ctx, FS_ERR_INVALID, "fs_set_histogram_sources_device: bad argument");
+    uint64_t n_max = 0;
+    for (uint32_t s = 0; s < n_sources; ++s) {
+        if (n_paths[s] == 0) return fail(ctx, FS_ERR_INVALID, "fs_set_histogram_sources_device: a path count is 0");
+        if (n_paths[s] > n_max) n_max = n_paths[s];
+    }
+    dev_guard g(ctx->device);
+    int rc = ensure_hist(ctx, n_sources);
+    if (rc) return rc;
+    const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
+    CK(cudaMemcpyAsync(ctx->d_hist, d_hist, 8 * hn, cudaMemcpyDeviceToDevice, ctx->stream));
+    set_hist_counts(ctx, n_sources, n_max, n_paths);
     return FS_OK;
 }
 
@@ -910,8 +1003,8 @@ static int ir_common(fs_ctx* ctx, uint32_t hist_source, uint32_t source, const f
         d_energy = ctx->d_energy;
     }
     const unsigned long long* hsrc = ctx->d_hist ? ctx->d_hist + (size_t)hist_source * c.n_bands * c.n_bins : nullptr;
-    if (per_band) CK(fs_ir_build_bands(ctx, hsrc, ctx->hist_n_paths, noise_seed, s->ir));
-    else CK(fs_ir_build(ctx, hsrc, ctx->hist_n_paths, d_energy, s->ir));
+    if (per_band) CK(fs_ir_build_bands(ctx, hsrc, hist_paths(ctx, hist_source), noise_seed, s->ir));
+    else CK(fs_ir_build(ctx, hsrc, hist_paths(ctx, hist_source), d_energy, s->ir));
     { std::lock_guard<std::mutex> lk(ctx->conv_mu); CK(fs_conv_update_ir(ctx, source, ctx->stream)); }
     CK(cudaEventRecord(ctx->ev_ir1, ctx->stream));
     ctx->ir_timed = true;
@@ -965,8 +1058,13 @@ int fs_build_ir_all(fs_ctx* ctx, uint32_t n_sources, float* ir_out)
     for (uint32_t s0 = 0; s0 < n_sources; s0 += FS_PTR_TABLE) {
         const uint32_t n = n_sources - s0 < FS_PTR_TABLE ? n_sources - s0 : FS_PTR_TABLE;
         fs_ptr_table tab;
-        for (uint32_t i = 0; i < n; ++i) { tab.p[i] = ctx->conv[s0 + i]->ir; tab.q[i] = nullptr; }
-        CK(fs_ir_build_multi(ctx, ctx->d_hist, s0, n, ctx->hist_n_paths, tab));
+        fs_scale_table inv;
+        for (uint32_t i = 0; i < n; ++i) {
+            tab.p[i] = ctx->conv[s0 + i]->ir; tab.q[i] = nullptr;
+            const uint64_t np = hist_paths(ctx, s0 + i);
+            inv.v[i] = np ? 1.0 / (double)np : 0.0;
+        }
+        CK(fs_ir_build_multi(ctx, ctx->d_hist, s0, n, inv, tab));
         { std::lock_guard<std::mutex> lk(ctx->conv_mu); CK(fs_conv_update_ir_multi(ctx, s0, n, ctx->stream)); }
     }
     CK(cudaEventRecord(ctx->ev_ir1, ctx->stream));
@@ -1005,6 +1103,64 @@ int fs_update(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float
     if (rc) return rc;
     if (!ir_out) return hist_out ? finish_stats(ctx) : FS_OK;      // with ir_out the IR read-back has synchronised already
     return FS_OK;
+}
+
+int fs_trace_sources(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3], uint64_t seed,
+                     uint64_t* hist_out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    nvtx_range nv("fs_trace_sources");
+    fs_src_table t;
+    int rc = prepare_sources(ctx, "fs_trace_sources", src, n_sources, lis_pos, &t);
+    if (rc) return rc;
+    dev_guard g(ctx->device);
+    if ((rc = ensure_hist(ctx, n_sources))) return rc;
+    const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
+    CK(cudaMemsetAsync(ctx->d_hist, 0, 8 * hn, ctx->stream));            // FlushEnergyBuffer, COMP.h:76-79
+    rc = trace_common(ctx, t.pos.data(), n_sources, lis_pos, t.n_max, 0, t.off[n_sources], t.d_max, seed, ctx->d_hist, nullptr, &t);
+    if (rc) return rc;
+    set_hist_counts(ctx, n_sources, t.n_max, t.n_paths.data());
+    if (hist_out) {
+        CK(cudaMemcpyAsync(hist_out, ctx->d_hist, 8 * hn, cudaMemcpyDeviceToHost, ctx->stream));
+        return finish_stats(ctx);
+    }
+    return FS_OK;
+}
+
+int fs_update_sources(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3], uint64_t seed,
+                      uint64_t* hist_out, float* ir_out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    nvtx_range nv("fs_update_sources");
+    if (n_sources > FS_MAX_SOURCES) return fail(ctx, FS_ERR_INVALID, "fs_update_sources: source id too large (< 4096)");
+    int rc = fs_trace_sources(ctx, src, n_sources, lis_pos, seed, nullptr);      // enqueued, not synchronised
+    if (rc) return rc;
+    dev_guard g(ctx->device);
+    if (hist_out) {
+        const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
+        CK(cudaMemcpyAsync(hist_out, ctx->d_hist, 8 * hn, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    rc = (n_sources == 1) ? ir_common(ctx, 0, 0, nullptr, ir_out) : fs_build_ir_all(ctx, n_sources, ir_out);
+    if (rc) return rc;
+    if (!ir_out) return hist_out ? finish_stats(ctx) : FS_OK;
+    return FS_OK;
+}
+
+int fs_trace_sources_range_device(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3],
+                                  uint64_t g_first, uint64_t g_count, uint64_t seed, void* d_hist, int zero_first)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!d_hist) return fail(ctx, FS_ERR_INVALID, "fs_trace_sources_range_device: null histogram");
+    fs_src_table t;
+    int rc = prepare_sources(ctx, "fs_trace_sources_range_device", src, n_sources, lis_pos, &t);
+    if (rc) return rc;
+    if (g_first + g_count > t.off[n_sources] || g_first + g_count < g_first)
+        return fail(ctx, FS_ERR_INVALID, "fs_trace_sources_range_device: work range exceeds the sum of the path counts");
+    dev_guard g(ctx->device);
+    const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
+    if (zero_first) CK(cudaMemsetAsync(d_hist, 0, 8 * hn, ctx->stream));
+    return trace_common(ctx, t.pos.data(), n_sources, lis_pos, t.n_max, g_first, g_count, t.d_max, seed,
+                        (unsigned long long*)d_hist, nullptr, &t);
 }
 
 int fs_build_ir_bands(fs_ctx* ctx, uint32_t hist_source, uint32_t conv_source, uint64_t noise_seed, float* ir_out)
@@ -1151,14 +1307,16 @@ int fs_get_stats(fs_ctx* ctx, fs_stats* out)
 
 // fs_multi.cu: make context 0's histogram the target of a multi-device update (allocated for n_sources, zeroed on the
 // context stream, bookkeeping of fs_trace)
-int fs_internal_hist_prepare(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, unsigned long long** d_hist_out)
+// per_source: host [n_sources] path counts of a per-source-budget update, or null (n_paths for every source)
+int fs_internal_hist_prepare(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, const uint64_t* per_source,
+                             unsigned long long** d_hist_out)
 {
     dev_guard g(ctx->device);
     int rc = ensure_hist(ctx, n_sources);
     if (rc) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemsetAsync(ctx->d_hist, 0, 8 * hn, ctx->stream));
-    ctx->hist_n_paths = n_paths; ctx->hist_cur_sources = n_sources;
+    set_hist_counts(ctx, n_sources, n_paths, per_source);
     *d_hist_out = ctx->d_hist;
     return FS_OK;
 }

@@ -75,9 +75,14 @@ struct fs_trace_params {
     fs_eval_params ep;
     uint32_t n_bins;
     float bin_ms, rr_prob, eps_offset, eps_connect, sound_speed, energy_clamp, energy_gain;
-    uint32_t max_depth;
+    uint32_t max_depth;         // per-source budgets: the largest depth (it sizes the records, queues and bounce loops)
     uint32_t seed_lo, seed_hi;
-    uint64_t n_paths;           // per source
+    uint64_t n_paths;           // per source; per-source budgets: the largest budget (stride of the listener cache)
+    // per-source budgets (fs_trace_sources): null = uniform, source of work index g = g / n_paths.  Otherwise every batch
+    // resolves each pair's (source, depth) once into fs_wave_buffers::pair_src.
+    const uint64_t* src_off;    // device [S+1]: first work index of every source, src_off[S] = G
+    const uint32_t* src_depth;  // device [S]: ray budget per subpath of every source
+    uint32_t n_src;
     uint64_t g_first;           // first global work index of this batch
     uint32_t batch;             // path pairs in this batch
     uint32_t cap;               // allocated path pairs (stride of per-node records = 2 * cap)
@@ -101,6 +106,7 @@ struct fs_wave_buffers {
     float* conn_len;            // [cap] connection segment length, indexed by path
     uint32_t* q_count;          // [max_depth+4]: [k] rays of bounce k, [D+1] connected pairs, [D+2] shadow rays
     uint32_t* q_cursor;         // [max_depth+4] work cursors of the persistent kernels
+    uint2* pair_src;            // [cap] (source, depth limit) of every pair of the batch; per-source budgets only
     uint32_t cap, depth_cap;
     // FS_FLAG_CONNECT_ALL: node positions of every subpath and the (s, t) connection rays of a batch
     float4* npos;               // [max_depth+1][2*cap]: position of node k >= 1 of subpath sp_id
@@ -159,6 +165,8 @@ struct fs_ctx {
     unsigned long long* d_hist; uint32_t hist_sources;   // [S][B][K]; hist_sources = allocated, hist_cur_sources = valid
     uint32_t hist_cur_sources;
     uint64_t hist_n_paths;
+    std::vector<uint64_t> hist_src_paths;   // per-source path counts after fs_trace_sources* (empty: every source has hist_n_paths)
+    void* d_src_tab; uint32_t src_tab_cap;  // per-source budgets on the device: [S+1] u64 offsets, then [S] u32 depths
     fs_dev_counters* d_counters;
     // traversal-stack overflow of the last trace: one 4-byte async copy into pinned memory after every fs_trace*, looked at
     // by the next call that can (sticky until reported)
@@ -201,7 +209,8 @@ cudaError_t fs_wave_debug_rays(fs_ctx* ctx, const fs_trace_params& tp, const flo
                                uint64_t n, float* d_t, uint32_t* d_tri, uint8_t* d_hit);
 
 // fs_ir.cu
-cudaError_t fs_ir_build_multi(fs_ctx* ctx, const unsigned long long* d_hist, uint32_t s0, uint32_t n, uint64_t n_paths,
+struct fs_scale_table { double v[FS_PTR_TABLE]; };   // per-source 1 / n_paths, passed by value
+cudaError_t fs_ir_build_multi(fs_ctx* ctx, const unsigned long long* d_hist, uint32_t s0, uint32_t n, const fs_scale_table& inv_scale,
                               const fs_ptr_table& d_ir);
 cudaError_t fs_conv_update_ir_multi(fs_ctx* ctx, uint32_t s0, uint32_t n, cudaStream_t st);
 cudaError_t fs_ir_build_bands(fs_ctx* ctx, const unsigned long long* d_hist_src, uint64_t n_paths, uint64_t noise_seed,

@@ -108,7 +108,7 @@ __global__ void k_ir_bands(const float* __restrict__ amp, const float* __restric
 }
 
 // ---- all sources of a multi-emitter update in one launch each (config 4: 64 sources x 58 us of tiny serial launches) ----
-__global__ void k_energy_multi(const unsigned long long* __restrict__ hist, uint32_t n_bands, uint32_t n_bins, double inv_scale,
+__global__ void k_energy_multi(const unsigned long long* __restrict__ hist, uint32_t n_bands, uint32_t n_bins, fs_scale_table inv_scale,
                                float threshold, float* __restrict__ amp /*[S][K]*/)
 {
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x, src = blockIdx.y;
@@ -116,7 +116,7 @@ __global__ void k_energy_multi(const unsigned long long* __restrict__ hist, uint
     const unsigned long long* h = hist + (size_t)src * n_bands * n_bins;
     unsigned long long sum = 0;
     for (uint32_t b = 0; b < n_bands; ++b) sum += h[(size_t)b * n_bins + k];
-    const float e = (float)(((double)sum * (1.0 / 4294967296.0)) * inv_scale);
+    const float e = (float)(((double)sum * (1.0 / 4294967296.0)) * inv_scale.v[src]);
     const float Pi4 = sqrtf(4.0f * FS_PI);
     amp[(size_t)src * n_bins + k] = (fabsf(e) >= threshold) ? e / sqrtf(e * Pi4) : 0.0f;
 }
@@ -160,8 +160,9 @@ static void ir_normalize(fs_ctx* ctx, const fs_ptr_table* tab, uint32_t n, float
 
 }  // namespace
 
-// same arithmetic as fs_ir_build, for sources [s0, s0 + n) (n <= FS_PTR_TABLE): d_ir[i] = device IR of source s0 + i
-cudaError_t fs_ir_build_multi(fs_ctx* ctx, const unsigned long long* d_hist, uint32_t s0, uint32_t n, uint64_t n_paths,
+// same arithmetic as fs_ir_build, for sources [s0, s0 + n) (n <= FS_PTR_TABLE): d_ir[i] = device IR of source s0 + i,
+// normalised by inv_scale.v[i] (1 / the path count of that source)
+cudaError_t fs_ir_build_multi(fs_ctx* ctx, const unsigned long long* d_hist, uint32_t s0, uint32_t n, const fs_scale_table& inv_scale,
                               const fs_ptr_table& d_ir)
 {
     const fs_config& c = ctx->cfg;
@@ -172,7 +173,6 @@ cudaError_t fs_ir_build_multi(fs_ctx* ctx, const unsigned long long* d_hist, uin
         ctx->amp_all_cap = FS_PTR_TABLE;
     }
     const uint32_t spb = (uint32_t)((double)c.bin_ms * 1e-3 * c.sample_rate + 0.5);
-    const double inv_scale = n_paths ? 1.0 / (double)n_paths : 0.0;
     k_energy_multi<<<dim3((c.n_bins + 255) / 256, n), 256, 0, ctx->stream>>>(d_hist + (size_t)s0 * c.n_bands * c.n_bins, c.n_bands,
                                                                             c.n_bins, inv_scale, c.ir_threshold, ctx->d_amp_all);
     k_ir_multi<<<dim3((c.sample_rate + IR_TILE - 1) / IR_TILE, n), IR_TILE, sizeof(float) * (IR_TILE + ctx->ir_window), ctx->stream>>>(

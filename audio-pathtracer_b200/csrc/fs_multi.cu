@@ -20,7 +20,8 @@
 #include <new>
 #include <thread>
 
-int fs_internal_hist_prepare(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, unsigned long long** d_hist_out);   // fs_api.cu
+int fs_internal_hist_prepare(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, const uint64_t* per_source,
+                             unsigned long long** d_hist_out);   // fs_api.cu
 
 namespace {
 
@@ -253,11 +254,11 @@ int fs_multi_scene_refit(fs_multi* m, float* cost_ratio_out)
 // One IR update's trace over all devices (UpdateSource, SUB.cpp:128-195, for n_sources sources): shard, trace, peer-store,
 // sum.  On return the work is ENQUEUED; the reduced histogram is context 0's (stream-ordered: fs_build_ir* on context 0
 // follows without a host synchronisation).  hist_out (host [S][B][K]) may be NULL; non-NULL synchronises.
-int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const float lis_pos[3], uint64_t n_paths,
-                   uint32_t max_depth, uint64_t seed, uint64_t* hist_out)
+// G: the flat work range [0, G); trace(ctx, first, count, d_hist, zero_first) traces one shard; n_paths / per_source: the
+// path counts context 0 records for its IR builders
+static int multi_trace_common(fs_multi* m, uint32_t n_sources, uint64_t G, uint64_t n_paths, const uint64_t* per_source,
+                              uint64_t* hist_out, const std::function<int(fs_ctx*, uint64_t, uint64_t, void*, int)>& trace)
 {
-    if (!m) return FS_ERR_INVALID;
-    if (!src_pos || !lis_pos || n_sources == 0 || n_paths == 0) return mfail(FS_ERR_INVALID, "fs_multi_trace: bad argument");
     cur_dev_guard guard;
     fs_ctx* c0 = m->ctx[0];
     const size_t hn = (size_t)n_sources * c0->cfg.n_bands * c0->cfg.n_bins;
@@ -276,12 +277,11 @@ int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const 
         }
         m->cap = cap;
     }
-    const uint64_t G = (uint64_t)n_sources * n_paths;
     unsigned long long* d_hist0 = nullptr;
     {   // device 0: histogram of context 0, zeroed ("Flush", COMP.h:76-79)
         cudaSetDevice(m->dev[0]);
         if (cudaEventRecord(m->ev_t0, c0->stream) != cudaSuccess) return mfail(FS_ERR_CUDA, "cudaEventRecord");
-        int rc = fs_internal_hist_prepare(c0, n_sources, n_paths, &d_hist0);
+        int rc = fs_internal_hist_prepare(c0, n_sources, n_paths, per_source, &d_hist0);
         if (rc) return mfail(rc, fs_last_error(c0));
     }
     std::vector<std::string> errs(m->n);
@@ -290,8 +290,7 @@ int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const 
         const uint64_t first = i * base + (i < rem ? i : rem), count = base + (i < rem ? 1 : 0);
         fs_ctx* c = m->ctx[i];
         cudaSetDevice(m->dev[i]);
-        int r = fs_trace_range_device(c, src_pos, n_sources, lis_pos, n_paths, first, count, max_depth, seed,
-                                      i == 0 ? (void*)d_hist0 : (void*)m->d_local[i], i == 0 ? 0 : 1);
+        int r = trace(c, first, count, i == 0 ? (void*)d_hist0 : (void*)m->d_local[i], i == 0 ? 0 : 1);
         if (r) { errs[i] = fs_last_error(c); return r; }
         if (i > 0) {
             // hand-written peer store: this device's shard histogram -> its slot of the staging buffer on device 0
@@ -331,6 +330,37 @@ int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const 
         }
     }
     return FS_OK;
+}
+
+int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const float lis_pos[3], uint64_t n_paths,
+                   uint32_t max_depth, uint64_t seed, uint64_t* hist_out)
+{
+    if (!m) return FS_ERR_INVALID;
+    if (!src_pos || !lis_pos || n_sources == 0 || n_paths == 0) return mfail(FS_ERR_INVALID, "fs_multi_trace: bad argument");
+    return multi_trace_common(m, n_sources, (uint64_t)n_sources * n_paths, n_paths, nullptr, hist_out,
+                              [&](fs_ctx* c, uint64_t first, uint64_t count, void* d_hist, int zero_first) {
+                                  return fs_trace_range_device(c, src_pos, n_sources, lis_pos, n_paths, first, count, max_depth,
+                                                               seed, d_hist, zero_first); });
+}
+
+// fs_trace_sources over all devices: the flat range [0, sum n_s) is sharded like fs_multi_trace's
+int fs_multi_trace_sources(fs_multi* m, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3], uint64_t seed,
+                           uint64_t* hist_out)
+{
+    if (!m) return FS_ERR_INVALID;
+    if (!src || !lis_pos || n_sources == 0) return mfail(FS_ERR_INVALID, "fs_multi_trace_sources: bad argument");
+    std::vector<uint64_t> counts(n_sources);
+    uint64_t G = 0, n_max = 0;
+    for (uint32_t s = 0; s < n_sources; ++s) {
+        // the full validation (depth limits, shared listener) is that of fs_trace_sources_range_device on every device
+        if (src[s].n_paths == 0) return mfail(FS_ERR_INVALID, "fs_multi_trace_sources: a source has n_paths = 0");
+        counts[s] = src[s].n_paths; G += src[s].n_paths;
+        if (src[s].n_paths > n_max) n_max = src[s].n_paths;
+    }
+    return multi_trace_common(m, n_sources, G, n_max, counts.data(), hist_out,
+                              [&](fs_ctx* c, uint64_t first, uint64_t count, void* d_hist, int zero_first) {
+                                  return fs_trace_sources_range_device(c, src, n_sources, lis_pos, first, count, seed, d_hist,
+                                                                       zero_first); });
 }
 
 // device time of the last fs_multi_trace on device 0's stream: the whole update (it ends when the slowest device has

@@ -28,6 +28,7 @@ ABI_SYMBOLS = [
     "fs_scene_set_triangles", "fs_scene_set_materials", "fs_scene_set_materials_ex", "fs_scene_commit",
     "fs_scene_update_vertices", "fs_scene_refit",
     "fs_trace", "fs_update", "fs_trace_range_device", "fs_trace_range", "fs_trace_debug",
+    "fs_trace_sources", "fs_update_sources", "fs_trace_sources_range_device", "fs_set_histogram_sources_device",
     "fs_debug_closest_hits", "fs_debug_any_hits",
     "fs_build_ir", "fs_build_ir_to", "fs_build_ir_all", "fs_build_ir_bands", "fs_build_ir_from_energy", "fs_set_histogram", "fs_set_histogram_device",
     "fs_get_histogram", "fs_get_histogram_sources", "fs_set_ir", "fs_load_float_array", "fs_save_float_array",
@@ -37,7 +38,7 @@ ABI_SYMBOLS = [
     "fs_multi_create", "fs_multi_destroy", "fs_multi_last_error", "fs_multi_device_count", "fs_multi_context",
     "fs_multi_scene_set_triangles", "fs_multi_scene_set_materials", "fs_multi_scene_set_materials_ex", "fs_multi_scene_commit",
     "fs_multi_scene_update_vertices", "fs_multi_scene_refit",
-    "fs_multi_trace", "fs_multi_last_ms", "fs_multi_synchronize",
+    "fs_multi_trace", "fs_multi_trace_sources", "fs_multi_last_ms", "fs_multi_synchronize",
 ]
 
 
@@ -117,6 +118,24 @@ PATH_DBG_DTYPE = np.dtype([
 ])
 
 
+class SourceDesc(C.Structure):
+    """fs_source_desc: one emitter of a per-source-budget update (RaycastsPerTick / RaycastBounces, COMP.h:35-66)"""
+    _fields_ = [("pos", C.c_float * 3), ("max_depth", C.c_uint32), ("n_paths", C.c_uint64)]
+
+
+def source_descs(src_pos, n_paths, depths):
+    """fs_source_desc[S] from positions [S][3], budgets [S] and depths [S]"""
+    src = np.ascontiguousarray(src_pos, dtype=np.float32).reshape(-1, 3)
+    n = np.broadcast_to(np.asarray(n_paths, dtype=np.uint64), (len(src),))
+    d = np.broadcast_to(np.asarray(depths, dtype=np.uint32), (len(src),))
+    arr = (SourceDesc * len(src))()
+    for s in range(len(src)):
+        arr[s].pos[:] = [float(v) for v in src[s]]
+        arr[s].max_depth = int(d[s])
+        arr[s].n_paths = int(n[s])
+    return arr
+
+
 class FrequenSeeError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__("frequensee error %d: %s" % (code, msg))
@@ -156,6 +175,10 @@ def load():
     L.fs_trace_range_device.argtypes = [vp, vp, u32, vp, u64, u64, u64, u32, u64, vp, i32]
     L.fs_trace_range.argtypes = [vp, vp, u32, vp, u64, u64, u64, u32, u64, vp]
     L.fs_trace_debug.argtypes = [vp, vp, u32, vp, u64, u64, u64, u32, u64, vp]
+    L.fs_trace_sources.argtypes = [vp, vp, u32, vp, u64, vp]
+    L.fs_update_sources.argtypes = [vp, vp, u32, vp, u64, vp, vp]
+    L.fs_trace_sources_range_device.argtypes = [vp, vp, u32, vp, u64, u64, u64, vp, i32]
+    L.fs_set_histogram_sources_device.argtypes = [vp, vp, u32, vp]
     L.fs_debug_closest_hits.argtypes = [vp, vp, u64, vp, vp]
     L.fs_debug_any_hits.argtypes = [vp, vp, vp, u64, vp]
     L.fs_build_ir.argtypes = [vp, u32, vp]
@@ -196,6 +219,7 @@ def load():
     L.fs_multi_scene_update_vertices.argtypes = [vp, vp, u64, u64]
     L.fs_multi_scene_refit.argtypes = [vp, C.POINTER(C.c_float)]
     L.fs_multi_trace.argtypes = [vp, vp, u32, vp, u64, u32, u64, vp]
+    L.fs_multi_trace_sources.argtypes = [vp, vp, u32, vp, u64, vp]
     L.fs_multi_last_ms.argtypes = [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     L.fs_multi_synchronize.argtypes = [vp]
     for n in ABI_SYMBOLS:
@@ -349,6 +373,45 @@ class Context:
         self._ck(self.L.fs_trace_range_device(self.h, src.ctypes.data, len(src), lis.ctypes.data, n_paths,
                                               g_first, g_count, max_depth, seed, C.c_void_p(d_hist_ptr),
                                               int(zero_first)))
+
+    # -- per-source budgets (fs_trace_sources*): n_paths[S] pairs and depths[S] per source; scalars broadcast --
+    def trace_sources(self, src_pos, n_paths, depths, lis_pos, seed, want_hist=True):
+        d = source_descs(src_pos, n_paths, depths)
+        lis = np.ascontiguousarray(lis_pos, dtype=np.float32).reshape(3)
+        S = len(d)
+        self.n_sources = S
+        hist = np.zeros((S, self.cfg.n_bands, self.cfg.n_bins), dtype=np.uint64) if want_hist else None
+        self._ck(self.L.fs_trace_sources(self.h, C.addressof(d), S, lis.ctypes.data, seed,
+                                         hist.ctypes.data if hist is not None else None))
+        return hist
+
+    def update_sources(self, src_pos, n_paths, depths, lis_pos, seed, hist_out=None, ir_out=None):
+        """fs_update_sources: one trace with per-source budgets + the IR of every source, one synchronisation"""
+        d = source_descs(src_pos, n_paths, depths)
+        lis = np.ascontiguousarray(lis_pos, dtype=np.float32).reshape(3)
+        S = len(d)
+        self.n_sources = S
+        for a, shape, dt in ((hist_out, (S, self.cfg.n_bands, self.cfg.n_bins), np.uint64),
+                             (ir_out, (S, self.cfg.n_channels, self.cfg.sample_rate), np.float32)):
+            if a is not None and (a.shape != shape or a.dtype != dt or not a.flags.c_contiguous):
+                raise ValueError("buffer must be C-contiguous %s of shape %r" % (np.dtype(dt).name, shape))
+        self._ck(self.L.fs_update_sources(self.h, C.addressof(d), S, lis.ctypes.data, seed,
+                                          hist_out.ctypes.data if hist_out is not None else None,
+                                          ir_out.ctypes.data if ir_out is not None else None))
+        return hist_out, ir_out
+
+    def trace_sources_range_device(self, src_pos, n_paths, depths, lis_pos, g_first, g_count, seed, d_hist_ptr,
+                                   zero_first=True):
+        d = source_descs(src_pos, n_paths, depths)
+        lis = np.ascontiguousarray(lis_pos, dtype=np.float32).reshape(3)
+        self.n_sources = len(d)
+        self._ck(self.L.fs_trace_sources_range_device(self.h, C.addressof(d), len(d), lis.ctypes.data, g_first, g_count,
+                                                      seed, C.c_void_p(d_hist_ptr), int(zero_first)))
+
+    def set_histogram_sources_device(self, d_ptr, n_paths):
+        n = np.ascontiguousarray(n_paths, dtype=np.uint64)
+        self.n_sources = len(n)
+        self._ck(self.L.fs_set_histogram_sources_device(self.h, C.c_void_p(d_ptr), len(n), n.ctypes.data))
 
     def trace_debug(self, src_pos, lis_pos, n_paths, g_first, g_count, max_depth, seed):
         src, lis = self._pos(src_pos, lis_pos)
@@ -529,6 +592,14 @@ class MultiContext:
         hist = np.zeros((len(src), self.cfg.n_bands, self.cfg.n_bins), dtype=np.uint64) if want_hist else None
         self._ck(self.L.fs_multi_trace(self.h, src.ctypes.data, len(src), lis.ctypes.data, n_paths, max_depth, seed,
                                        hist.ctypes.data if want_hist else None))
+        return hist
+
+    def trace_sources(self, src_pos, n_paths, depths, lis_pos, seed, want_hist=True):
+        d = source_descs(src_pos, n_paths, depths)
+        lis = np.ascontiguousarray(lis_pos, dtype=np.float32).reshape(3)
+        hist = np.zeros((len(d), self.cfg.n_bands, self.cfg.n_bins), dtype=np.uint64) if want_hist else None
+        self._ck(self.L.fs_multi_trace_sources(self.h, C.addressof(d), len(d), lis.ctypes.data, seed,
+                                               hist.ctypes.data if want_hist else None))
         return hist
 
     def last_ms(self):

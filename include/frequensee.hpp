@@ -204,6 +204,34 @@ public:
         Src.bUseDeviceHistogram = true;
     }
     void ForceUpdateSources() { for (auto* s : ActiveSources) UpdateSource(*s); }                              // SUB.cpp:883-886
+    // Every active source in ONE trace, each with its own RaycastsPerTick and RaycastBounces (COMP.h:35-66): histogram slot
+    // s belongs to ActiveSources[s] until the next update, and each IR is published to its component's own convolver slot.
+    // The random streams differ from UpdateSource's (one flat work range over all sources, fs_trace_sources), so this is
+    // a separate entry point; ForceUpdateSources keeps the reference's one-update-per-source sequence.
+    void UpdateSources()
+    {
+        if (ActiveSources.empty() || !Commit()) return;
+        const float lis[3] = {PawnLocation.X, PawnLocation.Y, PawnLocation.Z};
+        std::vector<fs_source_desc> desc(ActiveSources.size());
+        for (size_t s = 0; s < ActiveSources.size(); ++s) {
+            const UFrequenSeeAudioComponent& c = *ActiveSources[s];
+            const FVector3f L = c.GetActorLocation();
+            desc[s].pos[0] = L.X; desc[s].pos[1] = L.Y; desc[s].pos[2] = L.Z;
+            desc[s].max_depth = (uint32_t)c.RaycastBounces;
+            desc[s].n_paths = (uint64_t)c.RaycastsPerTick;
+        }
+        if (Ctx->Check(fs_trace_sources(Ctx->Get(), desc.data(), (uint32_t)desc.size(), lis, Seed++, nullptr)) != FS_OK) return;
+        fs_stats st;
+        if (fs_get_stats(Ctx->Get(), &st) == FS_OK) LastConnected = st.connected;
+        for (size_t s = 0; s < ActiveSources.size(); ++s) {
+            UFrequenSeeAudioComponent& c = *ActiveSources[s];
+            std::vector<float> flat((size_t)c.NumChannels * c.SampleRate);
+            if (Ctx->Check(fs_build_ir_to(Ctx->Get(), (uint32_t)s, c.GetSourceId(), flat.data())) != FS_OK) return;
+            for (int ch = 0; ch < c.NumChannels; ++ch)
+                std::memcpy(c.ImpulseBuffer[ch].data(), flat.data() + (size_t)ch * c.SampleRate, sizeof(float) * c.SampleRate);
+            c.bUseDeviceHistogram = true;
+        }
+    }
     uint64_t LastConnected = 0;
 
 private:
