@@ -3,6 +3,8 @@
 #include "fs_internal.h"
 
 #include <nvtx3/nvToolsExt.h>          // header-only NVTX 3: named ranges per stage for nsys / ncu --nvtx (SURVEY section 5)
+#include <algorithm>
+#include <climits>
 #include <stdio.h>
 #include <utility>
 #include <stdlib.h>
@@ -44,6 +46,36 @@ struct dev_guard {
     explicit dev_guard(int dev) : prev(-1), ok(false) { if (cudaGetDevice(&prev) == cudaSuccess) ok = (cudaSetDevice(dev) == cudaSuccess); }
     ~dev_guard() { if (prev >= 0) cudaSetDevice(prev); }
 };
+
+// the experiment knobs of a new context (defaults: fs_tune)
+static fs_tune read_tune()
+{
+    fs_tune t;
+    // the knob's value, if the variable is set and its value is within [lo, hi]
+    auto env = [](const char* name, uint32_t& v, int lo = INT_MIN, int hi = INT_MAX) {
+        if (const char* e = getenv(name)) { const int x = atoi(e); if (x >= lo && x <= hi) v = (uint32_t)x; }
+    };
+    env("FS_TUNE_REFILL", t.refill, 1, 32);
+    env("FS_TUNE_LEAF_MAX", t.leaf_max, 1, 8);
+    env("FS_TUNE_TEX", t.tex);
+    env("FS_TUNE_BUILDER", t.builder);
+    env("FS_TUNE_WIDE", t.wide);
+    env("FS_TUNE_W8", t.w8);
+    env("FS_TUNE_NODE_MIN", t.node_min);
+    env("FS_TUNE_TRI_MIN", t.tri_min);
+    env("FS_TUNE_COLLAPSE", t.collapse);
+    env("FS_TUNE_L2PIN", t.l2pin_mb);
+    env("FS_TUNE_TQ", t.tq);
+    env("FS_TUNE_TQ_NODE_MIN", t.tq_node_min);
+    env("FS_TUNE_TQ_FLUSH", t.tq_flush);
+    t.tq_flush = std::min(std::max(t.tq_flush, 1u), 32u);
+    env("FS_TUNE_MEGA", t.mega);
+    env("FS_TUNE_MEGA_FROM", t.mega_from);
+    env("FS_TUNE_MEGA_LANES", t.mega_lanes, 1, FS_MAX_LANES);
+    env("FS_TUNE_STREAMS", t.streams, 1, FS_MAX_LANES);
+    if (const char* e = getenv("FS_TUNE_CARVEOUT")) t.carveout = atoi(e);
+    return t;
+}
 
 extern "C" {
 
@@ -103,31 +135,7 @@ int fs_create(const fs_config* cfg, fs_ctx** out)
     ctx->device = dev;
     ctx->ir_window = ir_window;
     ctx->launches.store(0); ctx->conv_active.store(0);
-    ctx->tune_refill = 4; ctx->tune_leaf_max = FS_LEAF_MAX; ctx->tune_tex = 2; ctx->tune_builder = 1; ctx->tune_wide = 1; ctx->tune_node_min = 14; ctx->tune_tri_min = 4; ctx->tune_collapse = 17 /* bit 4: optimal (dynamic-programme) collapse of the BVH2 into 4-wide nodes: -22 % nodes, -4 % node steps */; ctx->tune_l2pin_mb = 0xffffffffu /* automatic */; ctx->tune_streams = 2;
-    if (const char* e14 = getenv("FS_TUNE_STREAMS")) { int v = atoi(e14); if (v >= 1 && v <= FS_MAX_LANES) ctx->tune_streams = (uint32_t)v; } ctx->tune_tq = 2;      // 0: phased kernels, 1: queue kernel for extension rays only, 2: also for connection rays
-    ctx->tune_tq_node_min = 10; ctx->tune_tq_flush = 24;
-    if (const char* e11 = getenv("FS_TUNE_TQ")) ctx->tune_tq = (uint32_t)atoi(e11);
-    ctx->tune_mega = 2;          // one persistent launch per batch for the extension stage (k_path_q): 0 never, 1 always, 2 when it pays
-    if (const char* e15 = getenv("FS_TUNE_MEGA")) ctx->tune_mega = (uint32_t)atoi(e15);
-    ctx->tune_mega_from = 0; ctx->tune_mega_lanes = 2;   // first bounce inside the persistent kernel; batch lanes with it (2: each lane's
-                                                         // persistent grid on half of the SMs -- one batch's connect / evaluate stage and tail overlap the other's walk: room -2.5 %)
-    if (const char* e16 = getenv("FS_TUNE_MEGA_FROM")) ctx->tune_mega_from = (uint32_t)atoi(e16);
-    if (const char* e17 = getenv("FS_TUNE_MEGA_LANES")) { int v = atoi(e17); if (v >= 1 && v <= FS_MAX_LANES) ctx->tune_mega_lanes = (uint32_t)v; }
-    if (const char* e12 = getenv("FS_TUNE_TQ_NODE_MIN")) ctx->tune_tq_node_min = (uint32_t)atoi(e12);
-    if (const char* e13 = getenv("FS_TUNE_TQ_FLUSH")) ctx->tune_tq_flush = (uint32_t)atoi(e13);
-    if (ctx->tune_tq_flush < 1) ctx->tune_tq_flush = 1;
-    if (ctx->tune_tq_flush > 32) ctx->tune_tq_flush = 32;       // FS_TQ_CAP assumes <= 31 entries carried into a node step
-    if (const char* e10 = getenv("FS_TUNE_L2PIN")) ctx->tune_l2pin_mb = (uint32_t)atoi(e10);
-    if (const char* e9 = getenv("FS_TUNE_COLLAPSE")) ctx->tune_collapse = (uint32_t)atoi(e9);
-    if (const char* e7 = getenv("FS_TUNE_TRI_MIN")) ctx->tune_tri_min = (uint32_t)atoi(e7);
-    if (const char* e6 = getenv("FS_TUNE_NODE_MIN")) ctx->tune_node_min = (uint32_t)atoi(e6);
-    if (const char* e5 = getenv("FS_TUNE_WIDE")) ctx->tune_wide = (uint32_t)atoi(e5);
-    ctx->tune_w8 = 0;            // 1: 8-wide compressed nodes (experimental: measured 5-10 % slower than the 4-wide nodes, profiles/r2_experiments.md)
-    if (const char* e18 = getenv("FS_TUNE_W8")) ctx->tune_w8 = (uint32_t)atoi(e18);
-    if (const char* e4 = getenv("FS_TUNE_BUILDER")) ctx->tune_builder = (uint32_t)atoi(e4);
-    if (const char* e3 = getenv("FS_TUNE_TEX")) ctx->tune_tex = (uint32_t)atoi(e3);
-    if (const char* e1 = getenv("FS_TUNE_REFILL")) { int v = atoi(e1); if (v >= 1 && v <= 32) ctx->tune_refill = (uint32_t)v; }
-    if (const char* e2 = getenv("FS_TUNE_LEAF_MAX")) { int v = atoi(e2); if (v >= 1 && v <= 8) ctx->tune_leaf_max = (uint32_t)v; }
+    ctx->tune = read_tune();
     dev_guard g(dev);
     int rc = FS_OK;
     do {
@@ -286,19 +294,19 @@ int fs_scene_set_materials(fs_ctx* ctx, const float* absorption, uint32_t n_mate
 static void apply_l2_policy(fs_ctx* ctx)
 {
     if (!ctx->bvh.wnodes) return;
-    if (ctx->tune_l2pin_mb == 0xffffffffu) {
+    if (ctx->tune.l2pin_mb == 0xffffffffu) {
         // automatic (default): only for scenes whose nodes + triangles do not fit the L2 anyway -- there a 48 MB window over
         // the top of the tree is worth 2 % (concert hall, profiles/r2_experiments.md); scenes that fit need no help
         int l2 = 0;
         cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, ctx->device);
         const size_t bvh_bytes = (size_t)ctx->bvh.n_wide * 64u + (size_t)ctx->bvh.n_tris * 64u;
-        ctx->tune_l2pin_mb = (l2 > 0 && bvh_bytes > (size_t)l2) ? 48u : 0u;
+        ctx->tune.l2pin_mb = (l2 > 0 && bvh_bytes > (size_t)l2) ? 48u : 0u;
     }
-    if (!ctx->tune_l2pin_mb) return;
+    if (!ctx->tune.l2pin_mb) return;
     int max_persist = 0, max_window = 0;
     cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, ctx->device);
     cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, ctx->device);
-    size_t want = (size_t)ctx->tune_l2pin_mb << 20;
+    size_t want = (size_t)ctx->tune.l2pin_mb << 20;
     const size_t have = (size_t)ctx->bvh.n_wide * 64u;
     if (want > have) want = have;
     if (want > (size_t)max_persist) want = (size_t)max_persist;
@@ -405,7 +413,7 @@ int fs_scene_commit(fs_ctx* ctx)
     }
     uint64_t bvh_launches = 0;
     CK(fs_bvh_build(ctx->stream, ctx->d_verts, ctx->d_tri_mat, ctx->n_tris, &ctx->bvh, &bvh_launches,
-                    ctx->tune_leaf_max, ctx->tune_builder, ctx->tune_collapse | (ctx->tune_w8 ? 4u : 0u)));
+                    ctx->tune.leaf_max, ctx->tune.builder, ctx->tune.collapse | (ctx->tune.w8 ? 4u : 0u)));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->launches.fetch_add(bvh_launches);
     ctx->stats.bvh_nodes = ctx->bvh.n_inner;
@@ -413,6 +421,7 @@ int fs_scene_commit(fs_ctx* ctx)
                                       ctx->bvh.n_tris, ctx->bvh.n_inner, ctx->bvh.n_wide, ctx->bvh.n_wide * 64.0 / 1e6);
     if (getenv("FS_VERBOSE") && ctx->bvh.w8nodes) fprintf(stderr, "[frequensee] BVH: %u 8-wide compressed nodes (%.1f MB)\n", ctx->bvh.n_w8, ctx->bvh.n_w8 * 80.0 / 1e6);
     ctx->stats.bvh_max_leaf = ctx->bvh.max_leaf;
+    ctx->trav = fs_choose_traversal(ctx->tune, ctx->bvh);
     apply_l2_policy(ctx);
     ctx->committed = true;
     ctx->verts_dirty = false;
@@ -446,7 +455,7 @@ int fs_scene_refit(fs_ctx* ctx, float* cost_ratio_out)
     if (!ctx) return FS_ERR_INVALID;
     if (!ctx->committed) return fail(ctx, FS_ERR_STATE, "fs_scene_refit: call fs_scene_commit first");
     nvtx_range nv("fs_scene_refit");
-    if (ctx->tune_w8) {                 // the 8-wide nodes (experiment knob FS_TUNE_W8) are rebuilt, not refitted
+    if (ctx->tune.w8) {                 // the 8-wide nodes (experiment knob FS_TUNE_W8) are rebuilt, not refitted
         int rc = fs_scene_commit(ctx);
         if (rc == FS_OK && cost_ratio_out) *cost_ratio_out = 1.0f;
         return rc;
@@ -456,6 +465,7 @@ int fs_scene_refit(fs_ctx* ctx, float* cost_ratio_out)
     float ratio = 1.0f;
     CK(fs_bvh_refit(ctx->stream, ctx->d_verts, &ctx->bvh, &launches, &ratio));
     ctx->launches.fetch_add(launches);
+    ctx->trav = fs_choose_traversal(ctx->tune, ctx->bvh);
     ctx->verts_dirty = false;
     if (cost_ratio_out) *cost_ratio_out = ratio;
     return FS_OK;
@@ -467,11 +477,12 @@ static void fill_params(fs_ctx* ctx, fs_trace_params* tp, const float lis[3], ui
 {
     const fs_config& c = ctx->cfg;
     memset(tp, 0, sizeof(*tp));
-    tp->bv.nodes_tex = (ctx->tune_tex && ctx->bvh.nodes_tex) ? (unsigned long long)ctx->bvh.nodes_tex : 0ull;
-    tp->bv.tris_tex = (ctx->tune_tex && ctx->bvh.tris_tex) ? (unsigned long long)ctx->bvh.tris_tex : 0ull;
-    tp->bv.wnodes = ctx->tune_wide ? ctx->bvh.wnodes : nullptr;
-    tp->bv.wnodes_tex = (ctx->tune_tex && ctx->bvh.wnodes_tex) ? (unsigned long long)ctx->bvh.wnodes_tex : 0ull;
-    const bool w8 = ctx->tune_w8 && ctx->tune_wide && ctx->bvh.w8nodes;
+    const fs_traversal& tr = ctx->trav;
+    tp->bv.nodes_tex = tr.tex ? (unsigned long long)ctx->bvh.nodes_tex : 0ull;
+    tp->bv.tris_tex = tr.tex ? (unsigned long long)ctx->bvh.tris_tex : 0ull;
+    tp->bv.wnodes = tr.nodes != FS_NODES_BVH2 ? ctx->bvh.wnodes : nullptr;
+    tp->bv.wnodes_tex = tr.tex ? (unsigned long long)ctx->bvh.wnodes_tex : 0ull;
+    const bool w8 = tr.nodes == FS_NODES_W8;
     tp->bv.w8nodes = w8 ? ctx->bvh.w8nodes : nullptr; tp->bv.tris8 = w8 ? ctx->bvh.tris8 : nullptr; tp->bv.tri8_map = w8 ? ctx->bvh.tri8_map : nullptr;
     tp->bv.w8_magic = 0x47000000u;
     for (int a = 0; a < 3; ++a) { tp->bv.qbase[a] = ctx->bvh.qbase[a]; tp->bv.qscale[a] = ctx->bvh.qscale[a]; }
@@ -608,12 +619,12 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
     }
     // equal batches: every bounce of a batch is a pair of launches whose cost has a fixed part (launch + the tail of the
     // slowest rays), so 1.25 M pairs run as 1 x 1.25 M or 2 x 0.63 M, never as 1 M + a 0.25 M remainder.
-    // Batches alternate between up to tune_streams lanes (own stream + own wavefront buffers): a traversal launch ends
+    // Batches alternate between up to tune.streams lanes (own stream + own wavefront buffers): a traversal launch ends
     // with a tail of a few long rays on an almost empty GPU, and the other lane's kernels fill it.  Histogram sums are
     // integer atomics, so the result does not depend on how batches interleave.  Per-kernel timing (FS_FLAG_TIME_KERNELS)
     // and the debug record path run on one lane so that every kernel is timed alone.
     uint32_t cap_cfg = ctx->cfg.max_batch_paths;
-    uint32_t n_lanes = ctx->tune_streams;
+    uint32_t n_lanes = ctx->tune.streams;
     if ((ctx->cfg.flags & FS_FLAG_TIME_KERNELS) || d_dbg) n_lanes = 1;
     if ((ctx->cfg.flags & FS_FLAG_SHARE_LISTENER) && (ctx->cfg.flags & (FS_FLAG_FUSED_EXTEND | FS_FLAG_BRUTE_FORCE)))
         return fail(ctx, FS_ERR_INVALID, "FS_FLAG_SHARE_LISTENER needs the wavefront path");
@@ -635,17 +646,17 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
         if (cap_cfg > lim) cap_cfg = lim;
         n_lanes = 1;
     }
-    // a job that will use the persistent per-batch kernel runs on at most tune_mega_lanes lanes (same rule as in
+    // a job that will use the persistent per-batch kernel runs on at most tune.mega_lanes lanes (same rule as in
     // launch_batch_split: batches of >= FS_MEGA_MIN_BATCH = 2^17 pairs on a scene of >= 4096 triangles, or FS_TUNE_MEGA=1)
     {
         const uint64_t nb1 = g_count ? (g_count + cap_cfg - 1) / cap_cfg : 1;
         const uint64_t cap1 = g_count ? (g_count + nb1 - 1) / nb1 : 1;
         const bool mega_job = !(ctx->cfg.flags & (FS_FLAG_COUNT_VISITS | FS_FLAG_CONNECT_ALL | FS_FLAG_MIS)) && max_depth >= 1 &&
-                              (ctx->tune_mega == 1u || (ctx->tune_mega == 2u && cap1 >= FS_MEGA_MIN_BATCH && ctx->bvh.n_tris >= 4096u &&
+                              (ctx->tune.mega == 1u || (ctx->tune.mega == 2u && cap1 >= FS_MEGA_MIN_BATCH && ctx->bvh.n_tris >= 4096u &&
                                                         ctx->conv_active.load() == 0));
-        if (mega_job && n_lanes > ctx->tune_mega_lanes) n_lanes = ctx->tune_mega_lanes;
+        if (mega_job && n_lanes > ctx->tune.mega_lanes) n_lanes = ctx->tune.mega_lanes;
         // ... and on one lane when half of it would fall below the size from which the persistent kernel pays
-        while (mega_job && ctx->tune_mega == 2u && n_lanes > 1 && g_count / n_lanes < FS_MEGA_MIN_BATCH) --n_lanes;
+        while (mega_job && ctx->tune.mega == 2u && n_lanes > 1 && g_count / n_lanes < FS_MEGA_MIN_BATCH) --n_lanes;
     }
     while (n_lanes > 1 && g_count / n_lanes < (1u << 17)) --n_lanes;            // small jobs: not worth a second set of launches
     uint64_t n_batches = g_count ? (g_count + cap_cfg - 1) / cap_cfg : 1;

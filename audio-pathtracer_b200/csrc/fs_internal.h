@@ -7,6 +7,7 @@
 #include <string>
 #include <atomic>
 #include <mutex>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/frequensee.h"
@@ -143,6 +144,41 @@ struct fs_ptr_table { void* p[FS_PTR_TABLE]; void* q[FS_PTR_TABLE]; };   // per-
 // one batch lane: a stream and its own wavefront buffers.  Lane 0 runs on the context stream itself.
 struct fs_lane { cudaStream_t stream; fs_wave_buffers wb; cudaEvent_t done; };
 
+// Experiment knobs: the FS_TUNE_* environment variables, read once by fs_create (DESIGN.md appendix).  Out-of-range values
+// of refill, leaf_max, streams and mega_lanes are ignored; tq_flush is clamped to 1..32.
+struct fs_tune {
+    uint32_t refill = 4;            // refill a warp once this many lanes are idle, 1..32
+    uint32_t leaf_max = FS_LEAF_MAX;   // LBVH leaf size, 1..8
+    uint32_t tex = 2;               // node fetches through the texture pipe: 0 none, 1 any-hit kernels, 2 every 4-wide / BVH2 kernel
+    uint32_t builder = 1;           // 0 LBVH, 1 PLOC
+    uint32_t wide = 1;              // 0: BVH2 float nodes
+    uint32_t w8 = 0;                // 1: 8-wide compressed nodes (measured 5-10 % slower than the 4-wide nodes, profiles/r2_experiments.md)
+    uint32_t node_min = 14, tri_min = 4;   // thresholds of the phased kernels
+    uint32_t collapse = 17;         // bit 4: optimal (dynamic-programme) collapse of the BVH2 into 4-wide nodes: -22 % nodes, -4 % node steps
+    uint32_t l2pin_mb = 0xffffffffu;   // MB of wide nodes in the persisting L2 window; 0xffffffff automatic (resolved at the first commit)
+    uint32_t tq = 2;                // 0 phased kernels, 1 queue kernel for extension rays only, 2 also for connection rays
+    uint32_t tq_node_min = 10;
+    uint32_t tq_flush = 24;         // FS_TQ_CAP assumes <= 31 entries carried into a node step
+    uint32_t mega = 2;              // one persistent launch per batch for the extension stage (k_path_q): 0 never, 1 always, 2 when it pays
+    uint32_t mega_from = 0;         // first bounce inside the persistent kernel
+    uint32_t mega_lanes = 2;        // batch lanes with it (2: each lane's persistent grid on half of the SMs -- one batch's connect /
+                                    // evaluate stage and tail overlap the other's walk: room -2.5 %), 1..FS_MAX_LANES
+    uint32_t streams = 2;           // batch lanes of the per-bounce pipeline, 1..FS_MAX_LANES
+    int carveout = -1;              // shared-memory carve-out of the traversal kernels in percent (-1: the driver's choice)
+};
+
+// Node format and traversal kernels of the split wavefront and of the debug rays, chosen by fs_choose_traversal from the
+// knobs and the built tree after every fs_scene_commit and fs_scene_refit
+enum fs_node_format : uint8_t { FS_NODES_BVH2, FS_NODES_W4, FS_NODES_W8 };
+struct fs_traversal {
+    fs_node_format nodes;           // node arrays fs_bvh_view exposes: `nodes`, + `wnodes` (W4), + `w8nodes` (W8)
+    bool tex;                       // fs_bvh_view carries the texture handles
+    bool closest_q;                 // closest-hit rays: queue kernel k_trace_q and, per batch, k_path_q (else k_trace_closest)
+    bool any_q;                     // any-hit rays: k_trace_q<ANY> (else k_trace_any)
+    uint8_t closest_tex, any_tex;   // TEX of each instantiation: 2 node fetches through the texture pipe, 0 none
+};
+fs_traversal fs_choose_traversal(const fs_tune& t, const fs_bvh_device& b);
+
 struct fs_ctx {
     fs_config cfg;
     int device;
@@ -160,7 +196,7 @@ struct fs_ctx {
     // trace: batches alternate between lanes -- while one batch's traversal launch drains its slowest rays, the other
     // lane's kernels fill the SMs
     fs_lane lanes[FS_MAX_LANES];
-    cudaEvent_t ev_fork; uint32_t tune_streams;
+    cudaEvent_t ev_fork;
     float4 *lis_rec, *lis_end; uint64_t lis_cache_n; uint32_t lis_cache_depth;   // FS_FLAG_SHARE_LISTENER cache
     unsigned long long* d_hist; uint32_t hist_sources;   // [S][B][K]; hist_sources = allocated, hist_cur_sources = valid
     uint32_t hist_cur_sources;
@@ -180,8 +216,10 @@ struct fs_ctx {
     std::vector<cudaEvent_t> kev; size_t kev_used;   // FS_FLAG_TIME_KERNELS: 4 events per batch
     std::vector<cudaEvent_t> tev; size_t tev_used;   //   + one (begin, end) pair per k_trace_closest launch
     int sm_count;
-    int occ[16];                         // resident CTAs per SM of the persistent kernels (per context = per device)
-    uint32_t tune_refill, tune_leaf_max, tune_tex, tune_builder, tune_wide, tune_node_min, tune_tri_min, tune_collapse, tune_l2pin_mb, tune_tq, tune_tq_node_min, tune_tq_flush, tune_mega, tune_mega_from, tune_mega_lanes, cur_lanes, tune_w8;      // experiment knobs (env FS_TUNE_REFILL / FS_TUNE_LEAF_MAX)
+    std::unordered_map<const void*, int> resident;   // resident CTAs per SM of every traversal kernel launched (per context = per device)
+    fs_tune tune;
+    fs_traversal trav;
+    uint32_t cur_lanes;                  // batch lanes of the running trace call
     // IR / conv
     float* d_energy;            // [K] scratch
     float* d_amp;               // [K]

@@ -2281,14 +2281,83 @@ __global__ void k_dbg_unpack_any(const uint32_t* __restrict__ conn, const uint32
 }
 
 template <typename K>
-int resident_ctas(K kernel, int threads, size_t smem)
+int resident_ctas(const fs_ctx* ctx, K kernel, int threads, size_t smem)
 {
     int n = 0;
     if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     // experiment knob: shared-memory carve-out in percent of the 228 KB (the rest is L1); default = the driver's choice
-    if (const char* e = getenv("FS_TUNE_CARVEOUT")) cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(e));
+    if (ctx->tune.carveout != -1) cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, ctx->tune.carveout);
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, threads, smem) != cudaSuccess || n < 1) n = 1;
     return n;
+}
+
+// Grid of a persistent traversal launch: `kernel`'s resident CTAs on every SM (shared by `lanes` batch lanes that run at
+// the same time), at most `max_ctas`, at least one.  Each instantiation's occupancy is looked up once per context.
+template <typename K>
+uint32_t tr_grid(fs_ctx* ctx, K kernel, size_t smem, uint32_t max_ctas, uint32_t lanes = 1)
+{
+    int& occ = ctx->resident[reinterpret_cast<const void*>(kernel)];
+    if (!occ) occ = resident_ctas(ctx, kernel, TR_THREADS, smem);
+    const uint32_t grid = (uint32_t)(ctx->sm_count * occ) / lanes;
+    return grid > max_ctas ? (max_ctas ? max_ctas : 1) : grid;
+}
+
+// FS_FLAG_TIME_KERNELS: the next n events of one of a context's event pools, which grows as needed
+cudaEvent_t* take_events(std::vector<cudaEvent_t>& pool, size_t& used, size_t n)
+{
+    if (pool.size() < used + n) {
+        const size_t old = pool.size();
+        pool.resize(used + n);
+        for (size_t i = old; i < pool.size(); ++i) cudaEventCreate(&pool[i]);
+    }
+    cudaEvent_t* ev = &pool[used];
+    used += n;
+    return ev;
+}
+
+// Closest-hit rays (origin, direction + tmax; ray count and work cursor on the device) through the kernel `tr` names;
+// (t, triangle) records to `hit`
+template <bool COUNT>
+void launch_closest(fs_ctx* ctx, const fs_traversal& tr, uint32_t max_ctas, cudaStream_t st, const fs_bvh_view& bv,
+                    const float4* ro, const float4* rd, const uint32_t* count, uint32_t* cursor, float2* hit)
+{
+    const fs_tune& t = ctx->tune;
+    auto queue = [&](auto kernel, size_t smem) {
+        kernel<<<tr_grid(ctx, kernel, smem, max_ctas), TR_THREADS, smem, st>>>(bv, ro, rd, count, cursor, hit, nullptr, nullptr, nullptr,
+                                                                             ctx->d_counters, t.refill, t.tq_node_min, t.tq_flush);
+    };
+    auto phased = [&](auto kernel) {
+        kernel<<<tr_grid(ctx, kernel, TR_SMEM_CLOSEST, max_ctas), TR_THREADS, TR_SMEM_CLOSEST, st>>>(bv, ro, rd, count, cursor, hit,
+                                                                             ctx->d_counters, t.refill, t.node_min, t.tri_min);
+    };
+    const bool tex = tr.closest_tex == 2;
+    if (tr.closest_q && tr.nodes == FS_NODES_W8) queue(k_trace_q<COUNT, 0, false, true>, TR_SMEM_TQ8);
+    else if (tr.closest_q) tex ? queue(k_trace_q<COUNT, 2, false, false>, TR_SMEM_TQ) : queue(k_trace_q<COUNT, 0, false, false>, TR_SMEM_TQ);
+    else if (tr.nodes != FS_NODES_BVH2) tex ? phased(k_trace_closest<COUNT, 2, true>) : phased(k_trace_closest<COUNT, 0, true>);
+    else tex ? phased(k_trace_closest<COUNT, 2, false>) : phased(k_trace_closest<COUNT, 0, false>);
+}
+
+// Any-hit rays (origin, direction + tmax; ray count and work cursor on the device) through the kernel `tr` names; the ids of
+// the unoccluded rays are appended to conn[], counted by *conn_count
+template <bool COUNT>
+void launch_any(fs_ctx* ctx, const fs_traversal& tr, uint32_t max_ctas, cudaStream_t st, const fs_bvh_view& bv,
+                const float4* ro, const float4* rd, const uint32_t* count, uint32_t* cursor, uint32_t* conn, uint32_t* conn_count,
+                fs_path_dbg* dbg)
+{
+    const fs_tune& t = ctx->tune;
+    auto queue = [&](auto kernel, size_t smem) {
+        kernel<<<tr_grid(ctx, kernel, smem, max_ctas), TR_THREADS, smem, st>>>(bv, ro, rd, count, cursor, nullptr, conn, conn_count, dbg,
+                                                                             ctx->d_counters, t.refill, t.tq_node_min, t.tq_flush);
+    };
+    auto phased = [&](auto kernel) {
+        kernel<<<tr_grid(ctx, kernel, TR_SMEM_ANY, max_ctas), TR_THREADS, TR_SMEM_ANY, st>>>(bv, ro, rd, count, cursor, conn, conn_count,
+                                                                             ctx->d_counters, dbg, t.refill, t.node_min);
+    };
+    const bool tex = tr.any_tex == 2;
+    if (tr.any_q && tr.nodes == FS_NODES_W8) queue(k_trace_q<COUNT, 0, true, true>, TR_SMEM_TQ8);
+    else if (tr.any_q) tex ? queue(k_trace_q<COUNT, 2, true, false>, TR_SMEM_TQ) : queue(k_trace_q<COUNT, 0, true, false>, TR_SMEM_TQ);
+    else if (tr.nodes != FS_NODES_BVH2) tex ? phased(k_trace_any<COUNT, 2, true>) : phased(k_trace_any<COUNT, 0, true>);
+    else tex ? phased(k_trace_any<COUNT, 2, false>) : phased(k_trace_any<COUNT, 0, false>);
 }
 
 int pick_mode(const fs_trace_params& tp)
@@ -2299,6 +2368,22 @@ int pick_mode(const fs_trace_params& tp)
 }
 
 }  // namespace
+
+fs_traversal fs_choose_traversal(const fs_tune& t, const fs_bvh_device& b)
+{
+    fs_traversal c = {};
+    c.tex = t.tex != 0;
+    c.nodes = !(t.wide && b.wnodes) ? FS_NODES_BVH2 : (t.w8 && b.w8nodes) ? FS_NODES_W8 : FS_NODES_W4;
+    // queue entries are single triangles: 4-wide nodes with single-triangle leaves, or the 8-wide nodes (such leaves by construction)
+    c.closest_q = t.tq && (c.nodes == FS_NODES_W8 || (c.nodes == FS_NODES_W4 && b.max_leaf == 1));
+    c.any_q = c.closest_q && t.tq >= 2;
+    // TEX 2 needs the texture handle of the node array the kernel walks; the 8-wide kernels have no texture path
+    const bool w8q = c.closest_q && c.nodes == FS_NODES_W8;
+    const bool has_tex = (c.nodes == FS_NODES_BVH2 ? b.nodes_tex : b.wnodes_tex) != 0;
+    c.closest_tex = (has_tex && !w8q && t.tex >= 2) ? 2 : 0;
+    c.any_tex = (has_tex && !(w8q && c.any_q) && t.tex != 0) ? 2 : 0;
+    return c;
+}
 
 cudaError_t fs_wave_alloc(fs_ctx* ctx, fs_lane* lane, uint32_t cap, uint32_t max_depth)
 {
@@ -2330,7 +2415,7 @@ cudaError_t fs_wave_alloc(fs_ctx* ctx, fs_lane* lane, uint32_t cap, uint32_t max
         if ((e = cudaMalloc(&wb->all_d, sizeof(float4) * wb->all_cap)) != cudaSuccess) return e;
         if ((e = cudaMalloc(&wb->all_conn, 4ull * wb->all_cap)) != cudaSuccess) return e;
     }
-    const bool mega_alloc = ctx->tune_mega == 1u || (ctx->tune_mega == 2u && cap >= FS_MEGA_MIN_BATCH && ctx->bvh.n_tris >= 4096u);
+    const bool mega_alloc = ctx->tune.mega == 1u || (ctx->tune.mega == 2u && cap >= FS_MEGA_MIN_BATCH && ctx->bvh.n_tris >= 4096u);
     if (mega_alloc && max_depth >= 1 && cap <= (1u << 21) && !(ctx->cfg.flags & (FS_FLAG_CONNECT_ALL | FS_FLAG_MIS | FS_FLAG_COUNT_VISITS))) {
         const uint64_t lc = (uint64_t)n2 * max_depth;                  // every subpath traces at most max_depth rays
         if (lc < 0xffffffffull) {
@@ -2366,23 +2451,14 @@ static cudaError_t launch_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_param
     const fs_wave_buffers& wb = lane->wb;
     const size_t smem = (MODE == MODE_TOP) ? (size_t)tp.n_top * 64 : 0;
     // occupancy depends on the instantiation (COUNT, MODE) and on the treelet size: queried per call, it is a host-only lookup
-    const int occ_ext = resident_ctas(k_extend<COUNT, MODE>, WF_THREADS, smem);
-    const int occ_con = resident_ctas(k_connect<COUNT, MODE>, WF_THREADS, smem);
+    const int occ_ext = resident_ctas(ctx, k_extend<COUNT, MODE>, WF_THREADS, smem);
+    const int occ_con = resident_ctas(ctx, k_connect<COUNT, MODE>, WF_THREADS, smem);
     if (smem > 48 * 1024) {
         cudaFuncSetAttribute(k_extend<COUNT, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         cudaFuncSetAttribute(k_connect<COUNT, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     }
     const bool timing = (tp.flags & FS_FLAG_TIME_KERNELS) != 0;
-    cudaEvent_t* ev = nullptr;
-    if (timing) {
-        if (ctx->kev.size() < ctx->kev_used + 4) {
-            size_t old = ctx->kev.size();
-            ctx->kev.resize(ctx->kev_used + 4);
-            for (size_t i = old; i < ctx->kev.size(); ++i) cudaEventCreate(&ctx->kev[i]);
-        }
-        ev = &ctx->kev[ctx->kev_used];
-        ctx->kev_used += 4;
-    }
+    cudaEvent_t* ev = timing ? take_events(ctx->kev, ctx->kev_used, 4) : nullptr;
     const uint32_t nq = tp.max_depth + 4;
     k_reset_queues<<<(nq + 63) / 64, 64, 0, st>>>(wb.q_count, wb.q_cursor, nq, ctx->d_counters, 0);
     ctx->launches.fetch_add(1);
@@ -2428,25 +2504,10 @@ static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace
 {
     cudaStream_t st = lane->stream;
     fs_wave_buffers& wb = lane->wb;
-    // resident CTAs per SM of the persistent kernels: cached per context (= per device) and per instantiation
-    int* occ = ctx->occ + (COUNT ? 4 : 0);
-    if (!occ[0]) occ[0] = resident_ctas(k_trace_closest<COUNT, 2, true>, TR_THREADS, TR_SMEM_CLOSEST);
-    if (!occ[1]) occ[1] = resident_ctas(k_trace_q<COUNT, 2, false, false>, TR_THREADS, TR_SMEM_TQ);
-    if (!occ[3]) occ[3] = resident_ctas(k_trace_q<COUNT, 0, false, true>, TR_THREADS, TR_SMEM_TQ8);
-    if (!occ[2]) occ[2] = resident_ctas(k_trace_any<COUNT, 2, true>, TR_THREADS, TR_SMEM_ANY);
-    const bool use_w8 = ctx->tune_tq && tp.bv.w8nodes != nullptr;               // 8-wide compressed nodes (single-triangle leaves by construction)
-    const int occ_tr = occ[0], occ_tq = use_w8 ? occ[3] : occ[1], occ_any = occ[2];
+    const fs_traversal& tr = ctx->trav;
+    const fs_tune& t = ctx->tune;
     const bool timing = (tp.flags & FS_FLAG_TIME_KERNELS) != 0;
-    cudaEvent_t* ev = nullptr;
-    if (timing) {
-        if (ctx->kev.size() < ctx->kev_used + 4) {
-            size_t old = ctx->kev.size();
-            ctx->kev.resize(ctx->kev_used + 4);
-            for (size_t i = old; i < ctx->kev.size(); ++i) cudaEventCreate(&ctx->kev[i]);
-        }
-        ev = &ctx->kev[ctx->kev_used];
-        ctx->kev_used += 4;
-    }
+    cudaEvent_t* ev = timing ? take_events(ctx->kev, ctx->kev_used, 4) : nullptr;
     const uint32_t nq = tp.max_depth + 4;
     k_reset_queues<<<(nq + 63) / 64, 64, 0, st>>>(wb.q_count, wb.q_cursor, nq, ctx->d_counters, 0);
     ctx->launches.fetch_add(1);
@@ -2454,10 +2515,7 @@ static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace
     const uint32_t n_sub = 2u * tp.batch;
     uint32_t grid_sh = (n_sub + FS_SG_THREADS - 1) / FS_SG_THREADS;
     if (grid_sh > (uint32_t)ctx->sm_count * (2048u / FS_SG_THREADS)) grid_sh = (uint32_t)ctx->sm_count * (2048u / FS_SG_THREADS);
-    const bool use_tq = (ctx->tune_tq && tp.bv.wnodes != nullptr && ctx->bvh.max_leaf == 1) || use_w8;    // queue entries are single triangles
-    uint32_t grid_tr = (uint32_t)(ctx->sm_count * (use_tq ? occ_tq : occ_tr));
     const uint32_t ctas_needed = (n_sub + TR_THREADS - 1) / TR_THREADS;
-    if (grid_tr > ctas_needed) grid_tr = ctas_needed ? ctas_needed : 1;
     if (timing) cudaEventRecord(ev[0], st);
     if (D == 0) {
         k_init_ends<<<(n_sub + 255u) / 256u, 256, 0, st>>>(tp, wb);
@@ -2472,43 +2530,29 @@ static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace
         // shoebox +16 ... +32 %: one long persistent launch has a longer tail than it saves, in-kernel shading at partial warps)
         // ... and only while no convolver source is active: a persistent grid holds every SM for the whole batch (4-5 ms), an
         // audio callback issued meanwhile would wait for it (measured p99 3.6 ms); between per-bounce kernels it waits 0.3 ms
-        const bool mega_ok = ctx->tune_mega == 1u || (ctx->tune_mega == 2u && tp.batch >= FS_MEGA_MIN_BATCH && tp.bv.n_tris >= 4096u &&
-                                                      ctx->conv_active.load() == 0);
-        const bool mega = !COUNT && use_tq && wb.log_o && mega_ok && (uint64_t)n_sub * D <= wb.log_cap;
-        const uint32_t k0 = mega ? (ctx->tune_mega_from < D ? ctx->tune_mega_from : D) : D;
+        const bool mega_ok = t.mega == 1u || (t.mega == 2u && tp.batch >= FS_MEGA_MIN_BATCH && tp.bv.n_tris >= 4096u &&
+                                              ctx->conv_active.load() == 0);
+        const bool mega = !COUNT && tr.closest_q && wb.log_o && mega_ok && (uint64_t)n_sub * D <= wb.log_cap;
+        const uint32_t k0 = mega ? (t.mega_from < D ? t.mega_from : D) : D;
         for (uint32_t k = 0; k <= D; ++k) {
             k_shade_gen<<<grid_sh, FS_SG_THREADS, 0, st>>>(tp, wb, k, ctx->d_counters);
             ctx->launches.fetch_add(1);
             if (k == D) break;
             if (k == k0) {
-                // the flag / ticket protocol does not need the whole grid resident (any resident warp can take any ray);
-                // with several batch lanes each lane's persistent grid gets its share of the SMs
-                const bool texq = tp.bv.wnodes_tex && ctx->tune_tex >= 2;
-                int& occ_pq = ctx->occ[use_w8 ? 10 : (texq ? 8 : 9)];
-                if (!occ_pq) occ_pq = use_w8 ? resident_ctas(k_path_q<0, true>, TR_THREADS, PQ_SMEM8)
-                                             : (texq ? resident_ctas(k_path_q<2, false>, TR_THREADS, PQ_SMEM) : resident_ctas(k_path_q<0, false>, TR_THREADS, PQ_SMEM));
                 const uint32_t epoch = ++wb.pq_epoch;
                 pq_globals* g = (pq_globals*)wb.pq;
                 k_pq_seed<<<ctx->sm_count * 4, 256, 0, st>>>(wb, wb.log_o, wb.log_d, wb.log_flag, epoch, g, k0);
-                uint32_t grid_pq = (uint32_t)(ctx->sm_count * occ_pq) / (ctx->cur_lanes ? ctx->cur_lanes : 1u);
-                if (grid_pq > ctas_needed) grid_pq = ctas_needed ? ctas_needed : 1;
-                cudaEvent_t* te = nullptr;
-                if (timing) {                              // the persistent launch is the "traversal launch" of this batch
-                    if (ctx->tev.size() < ctx->tev_used + 2) {
-                        size_t old = ctx->tev.size();
-                        ctx->tev.resize(ctx->tev_used + 2);
-                        for (size_t i = old; i < ctx->tev.size(); ++i) cudaEventCreate(&ctx->tev[i]);
-                    }
-                    te = &ctx->tev[ctx->tev_used];
-                    ctx->tev_used += 2;
-                    cudaEventRecord(te[0], st);
-                }
-                if (use_w8) k_path_q<0, true><<<grid_pq, TR_THREADS, PQ_SMEM8, st>>>(tp, wb, wb.log_o, wb.log_d, wb.log_flag, epoch, wb.log_cap, g,
-                                                                                   ctx->tune_refill, ctx->tune_tq_node_min, ctx->tune_tq_flush);
-                else if (texq) k_path_q<2, false><<<grid_pq, TR_THREADS, PQ_SMEM, st>>>(tp, wb, wb.log_o, wb.log_d, wb.log_flag, epoch, wb.log_cap, g,
-                                                                          ctx->tune_refill, ctx->tune_tq_node_min, ctx->tune_tq_flush);
-                else k_path_q<0, false><<<grid_pq, TR_THREADS, PQ_SMEM, st>>>(tp, wb, wb.log_o, wb.log_d, wb.log_flag, epoch, wb.log_cap, g,
-                                                                     ctx->tune_refill, ctx->tune_tq_node_min, ctx->tune_tq_flush);
+                cudaEvent_t* te = timing ? take_events(ctx->tev, ctx->tev_used, 2) : nullptr;
+                if (timing) cudaEventRecord(te[0], st);   // the persistent launch is the "traversal launch" of this batch
+                // the flag / ticket protocol does not need the whole grid resident (any resident warp can take any ray);
+                // with several batch lanes each lane's persistent grid gets its share of the SMs
+                auto path_q = [&](auto kernel, size_t smem) {
+                    const uint32_t grid = tr_grid(ctx, kernel, smem, ctas_needed, ctx->cur_lanes ? ctx->cur_lanes : 1u);
+                    kernel<<<grid, TR_THREADS, smem, st>>>(tp, wb, wb.log_o, wb.log_d, wb.log_flag, epoch, wb.log_cap, g,
+                                                           t.refill, t.tq_node_min, t.tq_flush);
+                };
+                if (tr.nodes == FS_NODES_W8) path_q(k_path_q<0, true>, PQ_SMEM8);
+                else tr.closest_tex == 2 ? path_q(k_path_q<2, false>, PQ_SMEM) : path_q(k_path_q<0, false>, PQ_SMEM);
                 if (timing) cudaEventRecord(te[1], st);
                 ctx->stats.persistent_launches += 1;
                 k_pq_finish<<<1, 1, 0, st>>>(wb, g, D, ctx->d_counters, k0);
@@ -2516,32 +2560,10 @@ static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace
                 ctx->stats.extend_launches += 1;
                 break;
             }
-            const bool wide = tp.bv.wnodes != nullptr;
-            const int texm = (wide ? tp.bv.wnodes_tex : tp.bv.nodes_tex) ? (int)ctx->tune_tex : 0;
-            cudaEvent_t* te = nullptr;
-            if (timing) {
-                if (ctx->tev.size() < ctx->tev_used + 2) {
-                    size_t old = ctx->tev.size();
-                    ctx->tev.resize(ctx->tev_used + 2);
-                    for (size_t i = old; i < ctx->tev.size(); ++i) cudaEventCreate(&ctx->tev[i]);
-                }
-                te = &ctx->tev[ctx->tev_used];
-                ctx->tev_used += 2;
-                cudaEventRecord(te[0], st);
-            }
-#define FS_LAUNCH_TRACE(TEXV, WIDEV)                                                                                   \
-            k_trace_closest<COUNT, TEXV, WIDEV><<<grid_tr, TR_THREADS, TR_SMEM_CLOSEST, st>>>(tp.bv, wb.st_pos[k & 1u], wb.st_nrm[k & 1u], \
-                wb.q_count + k, wb.q_cursor + k, wb.hit, ctx->d_counters, ctx->tune_refill, ctx->tune_node_min, ctx->tune_tri_min)
-#define FS_LAUNCH_TQ(TEXV, W8V)                                                                                        \
-            k_trace_q<COUNT, TEXV, false, W8V><<<grid_tr, TR_THREADS, W8V ? TR_SMEM_TQ8 : TR_SMEM_TQ, st>>>(tp.bv, wb.st_pos[k & 1u], \
-                wb.st_nrm[k & 1u], wb.q_count + k, wb.q_cursor + k, wb.hit, nullptr, nullptr, nullptr, ctx->d_counters, ctx->tune_refill, \
-                ctx->tune_tq_node_min, ctx->tune_tq_flush)
-            if (use_w8) FS_LAUNCH_TQ(0, true);
-            else if (use_tq) { if (texm >= 2) FS_LAUNCH_TQ(2, false); else FS_LAUNCH_TQ(0, false); }
-            else if (wide) { if (texm >= 2) FS_LAUNCH_TRACE(2, true); else FS_LAUNCH_TRACE(0, true); }
-            else { if (texm >= 2) FS_LAUNCH_TRACE(2, false); else FS_LAUNCH_TRACE(0, false); }
-#undef FS_LAUNCH_TQ
-#undef FS_LAUNCH_TRACE
+            cudaEvent_t* te = timing ? take_events(ctx->tev, ctx->tev_used, 2) : nullptr;
+            if (timing) cudaEventRecord(te[0], st);
+            launch_closest<COUNT>(ctx, tr, ctas_needed, st, tp.bv, wb.st_pos[k & 1u], wb.st_nrm[k & 1u], wb.q_count + k,
+                                  wb.q_cursor + k, wb.hit);
             if (timing) cudaEventRecord(te[1], st);
             ctx->launches.fetch_add(1);
             ++ctx->stats.extend_launches;
@@ -2565,29 +2587,12 @@ static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace
         k_connect_all_gen<<<grid_ca ? grid_ca : 1, WF_THREADS, 0, st>>>(tp, wb, ctx->d_counters);
     }
     else k_connect_gen<<<grid_cg, WF_THREADS, 0, st>>>(tp, wb, ctx->d_counters, d_dbg);
-    uint32_t grid_any = (uint32_t)(ctx->sm_count * ((use_tq && ctx->tune_tq >= 2) ? occ_tq : occ_any));
-    const uint32_t ctas_any = (tp.batch + TR_THREADS - 1) / TR_THREADS;
-    if (!all && grid_any > ctas_any) grid_any = ctas_any ? ctas_any : 1;
+    const uint32_t ctas_any = all ? ~0u : (tp.batch + TR_THREADS - 1) / TR_THREADS;   // `all`: the ray count is known on the device only
     const float4* any_o = all ? wb.all_o : wb.st_pos[0];
     const float4* any_d = all ? wb.all_d : wb.st_nrm[0];
     uint32_t* any_conn = all ? wb.all_conn : wb.conn_queue;
-    {
-        const bool wide = tp.bv.wnodes != nullptr;
-        const bool tex = (wide ? tp.bv.wnodes_tex : tp.bv.nodes_tex) && ctx->tune_tex;
-#define FS_LAUNCH_ANY(TEXV, WIDEV)                                                                                     \
-        k_trace_any<COUNT, TEXV, WIDEV><<<grid_any, TR_THREADS, TR_SMEM_ANY, st>>>(tp.bv, any_o, any_d, wb.q_count + (D + 2), \
-            wb.q_cursor + (D + 2), any_conn, wb.q_count + (D + 1), ctx->d_counters, all ? nullptr : d_dbg, ctx->tune_refill, ctx->tune_node_min)
-#define FS_LAUNCH_ANYQ(TEXV, W8V)                                                                                      \
-        k_trace_q<COUNT, TEXV, true, W8V><<<grid_any, TR_THREADS, W8V ? TR_SMEM_TQ8 : TR_SMEM_TQ, st>>>(tp.bv, any_o, any_d,       \
-            wb.q_count + (D + 2), wb.q_cursor + (D + 2), nullptr, any_conn, wb.q_count + (D + 1), all ? nullptr : d_dbg, ctx->d_counters, \
-            ctx->tune_refill, ctx->tune_tq_node_min, ctx->tune_tq_flush)
-        if (use_w8 && ctx->tune_tq >= 2) FS_LAUNCH_ANYQ(0, true);
-        else if (use_tq && ctx->tune_tq >= 2) { if (tex) FS_LAUNCH_ANYQ(2, false); else FS_LAUNCH_ANYQ(0, false); }
-        else if (wide) { if (tex) FS_LAUNCH_ANY(2, true); else FS_LAUNCH_ANY(0, true); }
-        else { if (tex) FS_LAUNCH_ANY(2, false); else FS_LAUNCH_ANY(0, false); }
-#undef FS_LAUNCH_ANYQ
-#undef FS_LAUNCH_ANY
-    }
+    launch_any<COUNT>(ctx, tr, ctas_any, st, tp.bv, any_o, any_d, wb.q_count + (D + 2), wb.q_cursor + (D + 2), any_conn,
+                      wb.q_count + (D + 1), all ? nullptr : d_dbg);
     ctx->launches.fetch_add(2);
     if (timing) cudaEventRecord(ev[2], st);
     uint32_t grid_ev = (uint32_t)ctx->sm_count * 8u;
@@ -2636,7 +2641,7 @@ cudaError_t fs_wave_debug_rays(fs_ctx* ctx, const fs_trace_params& tp, const flo
     cudaStream_t st = ctx->stream;
     const int mode = pick_mode(tp);
     if (!(tp.flags & (FS_FLAG_FUSED_EXTEND | FS_FLAG_BRUTE_FORCE)) && n < 0xffffffffull) {
-        // default: the same k_trace_closest / k_trace_any the BDPT update runs (4-wide nodes, smem stack, ...)
+        // default: the traversal kernels the trace chose for this tree and these knobs (ctx->trav)
         float4 *ro = nullptr, *rd = nullptr; float2* hits = nullptr; uint32_t *misc = nullptr, *conn = nullptr;
         cudaError_t e;
         if ((e = cudaMalloc(&ro, sizeof(float4) * n)) != cudaSuccess) return e;
@@ -2647,27 +2652,12 @@ cudaError_t fs_wave_debug_rays(fs_ctx* ctx, const fs_trace_params& tp, const flo
         cudaMemsetAsync(misc, 0, 16, st);            // [0] ray count, [1] cursor, [2] connected count
         const uint32_t g = (uint32_t)((n + 255) / 256);
         k_dbg_pack<<<g, 256, 0, st>>>(d_rays, d_hit ? d_tmax : nullptr, n, ro, rd, misc, d_hit);
-        const bool wide = tp.bv.wnodes != nullptr;
-        const bool tex = (wide ? tp.bv.wnodes_tex : tp.bv.nodes_tex) && ctx->tune_tex;
-        uint32_t grid = (uint32_t)((n + TR_THREADS - 1) / TR_THREADS);
-        if (grid > (uint32_t)ctx->sm_count * 5u) grid = (uint32_t)ctx->sm_count * 5u;
+        const uint32_t ctas = (uint32_t)((n + TR_THREADS - 1) / TR_THREADS);
         if (d_hit) {
-#define FS_DBG_ANY(TEXV, WIDEV) k_trace_any<false, TEXV, WIDEV><<<grid, TR_THREADS, TR_SMEM_ANY, st>>>(tp.bv, ro, rd, misc, misc + 1, conn, misc + 2, ctx->d_counters, nullptr, ctx->tune_refill, ctx->tune_node_min)
-#define FS_DBG_ANYQ(TEXV, W8V) k_trace_q<false, TEXV, true, W8V><<<grid, TR_THREADS, W8V ? TR_SMEM_TQ8 : TR_SMEM_TQ, st>>>(tp.bv, ro, rd, misc, misc + 1, nullptr, conn, misc + 2, nullptr, ctx->d_counters, ctx->tune_refill, ctx->tune_tq_node_min, ctx->tune_tq_flush)
-            if (tp.bv.w8nodes && ctx->tune_tq >= 2) FS_DBG_ANYQ(0, true);
-            else if (wide && ctx->tune_tq >= 2 && ctx->bvh.max_leaf == 1) { if (tex) FS_DBG_ANYQ(2, false); else FS_DBG_ANYQ(0, false); }
-            else if (wide) { if (tex) FS_DBG_ANY(2, true); else FS_DBG_ANY(0, true); } else { if (tex) FS_DBG_ANY(2, false); else FS_DBG_ANY(0, false); }
-#undef FS_DBG_ANYQ
-#undef FS_DBG_ANY
+            launch_any<false>(ctx, ctx->trav, ctas, st, tp.bv, ro, rd, misc, misc + 1, conn, misc + 2, nullptr);
             k_dbg_unpack_any<<<g, 256, 0, st>>>(conn, misc + 2, d_hit);
         } else {
-#define FS_DBG_CL(TEXV, WIDEV) k_trace_closest<false, TEXV, WIDEV><<<grid, TR_THREADS, TR_SMEM_CLOSEST, st>>>(tp.bv, ro, rd, misc, misc + 1, hits, ctx->d_counters, ctx->tune_refill, ctx->tune_node_min, ctx->tune_tri_min)
-#define FS_DBG_TQ(TEXV, W8V) k_trace_q<false, TEXV, false, W8V><<<grid, TR_THREADS, W8V ? TR_SMEM_TQ8 : TR_SMEM_TQ, st>>>(tp.bv, ro, rd, misc, misc + 1, hits, nullptr, nullptr, nullptr, ctx->d_counters, ctx->tune_refill, ctx->tune_tq_node_min, ctx->tune_tq_flush)
-            if (tp.bv.w8nodes && ctx->tune_tq) FS_DBG_TQ(0, true);
-            else if (wide && ctx->tune_tq && ctx->bvh.max_leaf == 1) { if (tex) FS_DBG_TQ(2, false); else FS_DBG_TQ(0, false); }
-            else if (wide) { if (tex) FS_DBG_CL(2, true); else FS_DBG_CL(0, true); } else { if (tex) FS_DBG_CL(2, false); else FS_DBG_CL(0, false); }
-#undef FS_DBG_TQ
-#undef FS_DBG_CL
+            launch_closest<false>(ctx, ctx->trav, ctas, st, tp.bv, ro, rd, misc, misc + 1, hits);
             k_dbg_unpack_closest<<<g, 256, 0, st>>>(tp.bv, hits, n, d_t, d_tri);
         }
         ctx->launches.fetch_add(3);
