@@ -122,14 +122,18 @@ struct fs_wave_buffers {
 struct fs_conv_source {
     bool active;
     float2* fdl;                // [P][C][NF] input spectra ring
-    float2* H[2];               // double-buffered IR partition spectra [P][C][NF]
+    float2* H[3];               // IR partition spectra [P][C][NF]: two buffers, a third (H[2]) only with FS_FLAG_CONV_CROSSFADE
     float* prev;                // [C][Bk] previous input block
     float* ir;                  // [C][sample_rate] device IR of this source
     // IR hand-off (game thread -> audio thread), all under fs_ctx::conv_mu: `pub` is the buffer the convolver reads;
     // `pending` (or -1) was written by the last IR update and becomes `pub` at the first callback that finds its
-    // h_ready event complete -- the audio thread never waits for a trace that is still running
-    int pub, pending;
-    cudaEvent_t h_ready[2];
+    // h_ready event complete -- the audio thread never waits for a trace that is still running.
+    // With FS_FLAG_CONV_CROSSFADE, `heard` (or -1 after fs_conv_init_source) is the buffer the last callback ended with;
+    // a callback whose `pub` differs from it fades from H[heard] to H[pub] over its first block and then sets heard = pub.
+    // Invariant: an IR update writes neither `pub` nor `heard` (pending is always a third buffer), and the callback
+    // reads both only under conv_mu, which it holds until the stream has synchronised.  Without the flag heard stays -1.
+    int pub, pending, heard;
+    cudaEvent_t h_ready[3];
     uint32_t head;              // FDL head slot
 };
 
@@ -226,6 +230,7 @@ struct fs_ctx {
     float* d_amp_all; uint32_t amp_all_cap;   // [FS_PTR_TABLE][K]: multi-source IR build
     float* d_carriers; float* d_amp_bands; uint64_t carrier_seed;   // per-band IR synthesis: [C][B][fs] noise carriers, [B][K]
     float2* d_twiddle;          // [conv fft size / 2]
+    float* d_xfade;             // FS_FLAG_CONV_CROSSFADE: [Bk] fade-in window w[i] = 0.5 - 0.5 cos(pi (i+1) / Bk)
     uint32_t fft_n, n_part, n_freq, ir_window;
     // per-source convolver state: FS_MAX_SOURCES stable slots (never reallocated: the audio thread may hold one while the
     // game thread creates another); creation, release and the IR hand-off fields are guarded by conv_mu

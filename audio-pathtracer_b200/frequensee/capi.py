@@ -21,6 +21,7 @@ FLAG_SHARE_LISTENER = 128
 FLAG_MATERIAL_MODEL = 256
 FLAG_MIS = 512
 FLAG_IR_NORMALIZE = 1024
+FLAG_CONV_CROSSFADE = 2048
 
 # every symbol include/frequensee.h declares (tests/test_abi.py checks the library exports them all)
 ABI_SYMBOLS = [
