@@ -109,6 +109,9 @@ int fs_create(const fs_config* cfg, fs_ctx** out)
     if ((uint32_t)((double)cfg->bin_ms * 1e-3 * cfg->sample_rate + 0.5) < 1u)
         return fail(nullptr, FS_ERR_INVALID, "bin_ms * sample_rate / 1000 must be at least one sample");
     if (!(cfg->ir_lowpass > 0.0f) || cfg->ir_lowpass > 1.0f) return fail(nullptr, FS_ERR_INVALID, "ir_lowpass must be in (0,1]");
+    if ((cfg->flags & FS_FLAG_NOISE_STATS) && (cfg->flags & (FS_FLAG_CONNECT_ALL | FS_FLAG_MIS)))
+        return fail(nullptr, FS_ERR_INVALID, "FS_FLAG_NOISE_STATS needs the endpoint connection (not with FS_FLAG_CONNECT_ALL / "
+                                             "FS_FLAG_MIS: a pair adds to several bins there)");
     // warm-up window of the per-sample low-pass evaluation: (1 - a)^W <= 1e-12, a multiple of 32 taps
     uint32_t ir_window = 32;
     if (cfg->ir_lowpass < 1.0f) {
@@ -194,7 +197,7 @@ void fs_destroy(fs_ctx* ctx)
     cudaFree(ctx->d_bsdf_tab); cudaFree(ctx->d_lobes);
     fs_bvh_free(&ctx->bvh);
     cudaFree(ctx->d_verts); cudaFree(ctx->d_tri_mat); cudaFree(ctx->d_refl_over_pi);
-    cudaFree(ctx->d_hist); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
+    cudaFree(ctx->d_hist); cudaFree(ctx->d_m2); cudaFree(ctx->d_noise); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
     cudaFree(ctx->d_amp); cudaFree(ctx->d_energy);
     for (cudaEvent_t e : ctx->kev) cudaEventDestroy(e);
     for (cudaEvent_t e : ctx->tev) cudaEventDestroy(e);
@@ -514,6 +517,23 @@ static int ensure_hist(fs_ctx* ctx, uint32_t n_sources)
     return FS_OK;
 }
 
+// FS_FLAG_NOISE_STATS: the second-moment buffer for n_sources, zeroed on the context stream like the histogram; null
+// without the flag
+static int prepare_m2(fs_ctx* ctx, uint32_t n_sources, ulonglong2** out)
+{
+    *out = nullptr;
+    if (!(ctx->cfg.flags & FS_FLAG_NOISE_STATS)) return FS_OK;
+    const size_t n = (size_t)n_sources * (ctx->cfg.n_bands + 1u) * ctx->cfg.n_bins;
+    if (!ctx->d_m2 || ctx->m2_sources < n_sources) {
+        cudaFree(ctx->d_m2); ctx->d_m2 = nullptr; ctx->m2_sources = 0;
+        CK(cudaMalloc(&ctx->d_m2, sizeof(ulonglong2) * n));
+        ctx->m2_sources = n_sources;
+    }
+    CK(cudaMemsetAsync(ctx->d_m2, 0, sizeof(ulonglong2) * n, ctx->stream));
+    *out = ctx->d_m2;
+    return FS_OK;
+}
+
 // bookkeeping of the histogram that fs_build_ir* read: its source count and the path count of every source (per_source:
 // host [n_sources] after fs_trace_sources*, null = n_paths for all)
 static void set_hist_counts(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, const uint64_t* per_source)
@@ -585,7 +605,8 @@ static bool lis_cache_fits(fs_ctx* ctx, uint64_t n_paths, uint32_t max_depth)
 // the work range is [0, G) with G = tab->off[S]; null = uniform budgets, G = n_sources * n_paths
 static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3],
                         uint64_t n_paths, uint64_t g_first, uint64_t g_count, uint32_t max_depth, uint64_t seed,
-                        unsigned long long* d_hist, fs_path_dbg* d_dbg, const fs_src_table* tab = nullptr)
+                        unsigned long long* d_hist, fs_path_dbg* d_dbg, const fs_src_table* tab = nullptr,
+                        ulonglong2* d_m2 = nullptr)
 {
     nvtx_range nv("fs_trace");
     if (!ctx->committed) return fail(ctx, FS_ERR_STATE, "fs_trace: call fs_scene_commit first");
@@ -601,6 +622,7 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
     int rc_ovf = check_overflow(ctx, false);
     if (rc_ovf) return rc_ovf;
     const int reset_ovf = ctx->overflow_pending ? 0 : 1;
+    ctx->m2_valid = false;                    // the callers that pass d_m2 set it again once the trace is enqueued
     if (ctx->src_cap < n_sources) {
         cudaFree(ctx->d_src_pos); ctx->d_src_pos = nullptr;
         CK(cudaMalloc(&ctx->d_src_pos, sizeof(float) * 3 * n_sources));
@@ -688,7 +710,7 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
         for (uint64_t i0 = 0; i0 < n_paths; i0 += cap) {
             tp.g_first = i0;
             tp.batch = (uint32_t)(n_paths - i0 < cap ? n_paths - i0 : cap);
-            CK(fs_wave_trace_batch(ctx, &ctx->lanes[0], tp, d_hist, nullptr));
+            CK(fs_wave_trace_batch(ctx, &ctx->lanes[0], tp, d_hist, nullptr, nullptr));
         }
         tp.lis_mode = 2;
     }
@@ -708,7 +730,7 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
         tp.g_first = g_first + done;
         tp.batch = (uint32_t)nb;
         const uint32_t l = b % n_lanes;
-        CK(fs_wave_trace_batch(ctx, &ctx->lanes[l], tp, d_hist, (d_dbg && l == 0) ? d_dbg + done : nullptr));
+        CK(fs_wave_trace_batch(ctx, &ctx->lanes[l], tp, d_hist, (d_dbg && l == 0) ? d_dbg + done : nullptr, d_m2));
         done += nb;
     }
     for (uint32_t l = 1; l < n_lanes; ++l) {
@@ -781,10 +803,13 @@ int fs_trace(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float 
     if (rc) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemsetAsync(ctx->d_hist, 0, 8 * hn, ctx->stream));            // FlushEnergyBuffer, COMP.h:76-79
+    ulonglong2* d_m2 = nullptr;
+    if ((rc = prepare_m2(ctx, n_sources, &d_m2))) return rc;
     rc = trace_common(ctx, src_pos, n_sources, lis_pos, n_paths, 0, (uint64_t)n_sources * n_paths, max_depth, seed,
-                      ctx->d_hist, nullptr);
+                      ctx->d_hist, nullptr, nullptr, d_m2);
     if (rc) return rc;
     set_hist_counts(ctx, n_sources, n_paths, nullptr);
+    ctx->m2_valid = d_m2 != nullptr;
     if (hist_out) {
         CK(cudaMemcpyAsync(hist_out, ctx->d_hist, 8 * hn, cudaMemcpyDeviceToHost, ctx->stream));
         return finish_stats(ctx);
@@ -792,17 +817,27 @@ int fs_trace(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float 
     return FS_OK;
 }
 
-int fs_trace_range_device(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3],
-                          uint64_t n_paths, uint64_t g_first, uint64_t g_count, uint32_t max_depth, uint64_t seed,
-                          void* d_hist, int zero_first)
+// shard forms; d_m2 (device [S][B+1][K], null = none) accumulates the second moments like d_hist (fs_multi)
+static int trace_range_device(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3],
+                              uint64_t n_paths, uint64_t g_first, uint64_t g_count, uint32_t max_depth, uint64_t seed,
+                              void* d_hist, ulonglong2* d_m2, int zero_first)
 {
     if (!ctx) return FS_ERR_INVALID;
     if (!d_hist) return fail(ctx, FS_ERR_INVALID, "fs_trace_range_device: null histogram");
     dev_guard g(ctx->device);
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     if (zero_first) CK(cudaMemsetAsync(d_hist, 0, 8 * hn, ctx->stream));
+    if (zero_first && d_m2) CK(cudaMemsetAsync(d_m2, 0, sizeof(ulonglong2) * (size_t)n_sources * (ctx->cfg.n_bands + 1u) * ctx->cfg.n_bins, ctx->stream));
     return trace_common(ctx, src_pos, n_sources, lis_pos, n_paths, g_first, g_count, max_depth, seed,
-                        (unsigned long long*)d_hist, nullptr);
+                        (unsigned long long*)d_hist, nullptr, nullptr, d_m2);
+}
+
+int fs_trace_range_device(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3],
+                          uint64_t n_paths, uint64_t g_first, uint64_t g_count, uint32_t max_depth, uint64_t seed,
+                          void* d_hist, int zero_first)
+{
+    return trace_range_device(ctx, src_pos, n_sources, lis_pos, n_paths, g_first, g_count, max_depth, seed, d_hist, nullptr,
+                              zero_first);
 }
 
 int fs_trace_range(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3], uint64_t n_paths,
@@ -907,6 +942,7 @@ int fs_set_histogram(fs_ctx* ctx, const uint64_t* hist, uint32_t n_sources, uint
     CK(cudaMemcpyAsync(ctx->d_hist, hist, 8 * hn, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     set_hist_counts(ctx, n_sources, n_paths, nullptr);
+    ctx->m2_valid = false;
     return FS_OK;
 }
 
@@ -920,6 +956,7 @@ int fs_set_histogram_device(fs_ctx* ctx, const void* d_hist, uint32_t n_sources,
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemcpyAsync(ctx->d_hist, d_hist, 8 * hn, cudaMemcpyDeviceToDevice, ctx->stream));
     set_hist_counts(ctx, n_sources, n_paths, nullptr);
+    ctx->m2_valid = false;
     return FS_OK;
 }
 
@@ -938,6 +975,7 @@ int fs_set_histogram_sources_device(fs_ctx* ctx, const void* d_hist, uint32_t n_
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemcpyAsync(ctx->d_hist, d_hist, 8 * hn, cudaMemcpyDeviceToDevice, ctx->stream));
     set_hist_counts(ctx, n_sources, n_max, n_paths);
+    ctx->m2_valid = false;
     return FS_OK;
 }
 
@@ -1128,9 +1166,13 @@ int fs_trace_sources(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources,
     if ((rc = ensure_hist(ctx, n_sources))) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemsetAsync(ctx->d_hist, 0, 8 * hn, ctx->stream));            // FlushEnergyBuffer, COMP.h:76-79
-    rc = trace_common(ctx, t.pos.data(), n_sources, lis_pos, t.n_max, 0, t.off[n_sources], t.d_max, seed, ctx->d_hist, nullptr, &t);
+    ulonglong2* d_m2 = nullptr;
+    if ((rc = prepare_m2(ctx, n_sources, &d_m2))) return rc;
+    rc = trace_common(ctx, t.pos.data(), n_sources, lis_pos, t.n_max, 0, t.off[n_sources], t.d_max, seed, ctx->d_hist, nullptr, &t,
+                      d_m2);
     if (rc) return rc;
     set_hist_counts(ctx, n_sources, t.n_max, t.n_paths.data());
+    ctx->m2_valid = d_m2 != nullptr;
     if (hist_out) {
         CK(cudaMemcpyAsync(hist_out, ctx->d_hist, 8 * hn, cudaMemcpyDeviceToHost, ctx->stream));
         return finish_stats(ctx);
@@ -1157,8 +1199,9 @@ int fs_update_sources(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources
     return FS_OK;
 }
 
-int fs_trace_sources_range_device(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3],
-                                  uint64_t g_first, uint64_t g_count, uint64_t seed, void* d_hist, int zero_first)
+static int trace_sources_range_device(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3],
+                                      uint64_t g_first, uint64_t g_count, uint64_t seed, void* d_hist, ulonglong2* d_m2,
+                                      int zero_first)
 {
     if (!ctx) return FS_ERR_INVALID;
     if (!d_hist) return fail(ctx, FS_ERR_INVALID, "fs_trace_sources_range_device: null histogram");
@@ -1170,8 +1213,15 @@ int fs_trace_sources_range_device(fs_ctx* ctx, const fs_source_desc* src, uint32
     dev_guard g(ctx->device);
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     if (zero_first) CK(cudaMemsetAsync(d_hist, 0, 8 * hn, ctx->stream));
+    if (zero_first && d_m2) CK(cudaMemsetAsync(d_m2, 0, sizeof(ulonglong2) * (size_t)n_sources * (ctx->cfg.n_bands + 1u) * ctx->cfg.n_bins, ctx->stream));
     return trace_common(ctx, t.pos.data(), n_sources, lis_pos, t.n_max, g_first, g_count, t.d_max, seed,
-                        (unsigned long long*)d_hist, nullptr, &t);
+                        (unsigned long long*)d_hist, nullptr, &t, d_m2);
+}
+
+int fs_trace_sources_range_device(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3],
+                                  uint64_t g_first, uint64_t g_count, uint64_t seed, void* d_hist, int zero_first)
+{
+    return trace_sources_range_device(ctx, src, n_sources, lis_pos, g_first, g_count, seed, d_hist, nullptr, zero_first);
 }
 
 int fs_build_ir_bands(fs_ctx* ctx, uint32_t hist_source, uint32_t conv_source, uint64_t noise_seed, float* ir_out)
@@ -1303,6 +1353,77 @@ int fs_debug_rfft(fs_ctx* ctx, const float* in, uint32_t n, float* out_ri)
     return FS_OK;
 }
 
+// the state rules of fs_get_noise / fs_get_histogram_m2
+static int noise_state(fs_ctx* ctx, const char* who)
+{
+    std::string w(who);
+    if (!(ctx->cfg.flags & FS_FLAG_NOISE_STATS)) return fail(ctx, FS_ERR_STATE, (w + ": the context was created without FS_FLAG_NOISE_STATS").c_str());
+    if (!ctx->m2_valid || !ctx->d_hist || ctx->hist_cur_sources == 0)
+        return fail(ctx, FS_ERR_STATE, (w + ": no second moments for the current histogram (trace with fs_trace / fs_trace_sources / "
+                                            "fs_update* / fs_multi_trace* first)").c_str());
+    return FS_OK;
+}
+
+static double snr_db(double signal, double variance)
+{
+    if (!(signal > 0.0)) return -INFINITY;
+    if (!(variance > 0.0)) return INFINITY;
+    return 10.0 * log10(signal / variance);
+}
+
+int fs_get_noise(fs_ctx* ctx, fs_noise_stats* out, uint32_t n_sources)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!out) return fail(ctx, FS_ERR_INVALID, "fs_get_noise: null output");
+    int rc = noise_state(ctx, "fs_get_noise");
+    if (rc) return rc;
+    const uint32_t S = ctx->hist_cur_sources, B = ctx->cfg.n_bands;
+    if (n_sources != S) return fail(ctx, FS_ERR_INVALID, "fs_get_noise: n_sources differs from fs_get_histogram_sources");
+    dev_guard g(ctx->device);
+    const size_t n_out = (size_t)S * (B + 1u) * 2u;
+    if (ctx->noise_cap < S) {
+        cudaFree(ctx->d_noise); ctx->d_noise = nullptr; ctx->noise_cap = 0;
+        CK(cudaMalloc(&ctx->d_noise, sizeof(double) * ((size_t)S + n_out)));
+        ctx->noise_cap = S;
+    }
+    std::vector<uint64_t> n(S);
+    for (uint32_t s = 0; s < S; ++s) n[s] = hist_paths(ctx, s);
+    std::vector<double> h(n_out);
+    uint64_t* d_n = (uint64_t*)ctx->d_noise;
+    double* d_out = ctx->d_noise + S;
+    CK(cudaMemcpyAsync(d_n, n.data(), 8ull * S, cudaMemcpyHostToDevice, ctx->stream));
+    CK(fs_noise_reduce(ctx->d_hist, ctx->d_m2, d_n, S, B, ctx->cfg.n_bins, d_out, ctx->stream));
+    ctx->launches.fetch_add(1);
+    CK(cudaMemcpyAsync(h.data(), d_out, sizeof(double) * n_out, cudaMemcpyDeviceToHost, ctx->stream));
+    if ((rc = finish_stats(ctx))) return rc;
+    for (uint32_t s = 0; s < S; ++s) {
+        fs_noise_stats& o = out[s];
+        memset(&o, 0, sizeof(o));
+        o.n_paths = n[s];
+        const double* r = h.data() + (size_t)s * (B + 1u) * 2u;
+        for (uint32_t b = 0; b < B; ++b) {
+            o.band_signal[b] = r[2 * b]; o.band_variance[b] = r[2 * b + 1];
+            o.band_snr_db[b] = snr_db(r[2 * b], r[2 * b + 1]);
+        }
+        o.signal = r[2 * B]; o.variance = r[2 * B + 1];
+        o.snr_db = snr_db(o.signal, o.variance);
+        o.no_energy = o.signal > 0.0 ? 0u : 1u;
+    }
+    return FS_OK;
+}
+
+int fs_get_histogram_m2(fs_ctx* ctx, uint64_t* out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!out) return fail(ctx, FS_ERR_INVALID, "fs_get_histogram_m2: null output");
+    int rc = noise_state(ctx, "fs_get_histogram_m2");
+    if (rc) return rc;
+    dev_guard g(ctx->device);
+    const size_t n = (size_t)ctx->hist_cur_sources * (ctx->cfg.n_bands + 1u) * ctx->cfg.n_bins;
+    CK(cudaMemcpyAsync(out, ctx->d_m2, sizeof(ulonglong2) * n, cudaMemcpyDeviceToHost, ctx->stream));
+    return finish_stats(ctx);
+}
+
 int fs_get_stats(fs_ctx* ctx, fs_stats* out)
 {
     if (!ctx || !out) return FS_ERR_INVALID;
@@ -1319,18 +1440,37 @@ int fs_get_stats(fs_ctx* ctx, fs_stats* out)
 // fs_multi.cu: make context 0's histogram the target of a multi-device update (allocated for n_sources, zeroed on the
 // context stream, bookkeeping of fs_trace)
 // per_source: host [n_sources] path counts of a per-source-budget update, or null (n_paths for every source)
+// d_m2_out: context 0's second-moment buffer (zeroed), or null without FS_FLAG_NOISE_STATS
 int fs_internal_hist_prepare(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, const uint64_t* per_source,
-                             unsigned long long** d_hist_out)
+                             unsigned long long** d_hist_out, ulonglong2** d_m2_out)
 {
     dev_guard g(ctx->device);
     int rc = ensure_hist(ctx, n_sources);
     if (rc) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemsetAsync(ctx->d_hist, 0, 8 * hn, ctx->stream));
+    if ((rc = prepare_m2(ctx, n_sources, d_m2_out))) return rc;
     set_hist_counts(ctx, n_sources, n_paths, per_source);
+    ctx->m2_valid = false;
     *d_hist_out = ctx->d_hist;
     return FS_OK;
 }
+// fs_multi.cu: the shard traces with second moments (d_m2 null = fs_trace_range_device / fs_trace_sources_range_device)
+int fs_internal_trace_range(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3], uint64_t n_paths,
+                            uint64_t g_first, uint64_t g_count, uint32_t max_depth, uint64_t seed, void* d_hist,
+                            ulonglong2* d_m2, int zero_first)
+{
+    return trace_range_device(ctx, src_pos, n_sources, lis_pos, n_paths, g_first, g_count, max_depth, seed, d_hist, d_m2,
+                              zero_first);
+}
+int fs_internal_trace_sources_range(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3],
+                                    uint64_t g_first, uint64_t g_count, uint64_t seed, void* d_hist, ulonglong2* d_m2,
+                                    int zero_first)
+{
+    return trace_sources_range_device(ctx, src, n_sources, lis_pos, g_first, g_count, seed, d_hist, d_m2, zero_first);
+}
+// fs_multi.cu: the reduced second moments of context 0 belong to its histogram
+void fs_internal_m2_valid(fs_ctx* ctx, bool valid) { ctx->m2_valid = valid; }
 
 // ---- text float arrays (saved_ir.txt: one float per line, COMP.cpp:454-505); host only
 int fs_load_float_array(const char* path, float* out, uint64_t cap, uint64_t* n_out)

@@ -206,6 +206,11 @@ struct fs_ctx {
     uint32_t hist_cur_sources;
     uint64_t hist_n_paths;
     std::vector<uint64_t> hist_src_paths;   // per-source path counts after fs_trace_sources* (empty: every source has hist_n_paths)
+    // FS_FLAG_NOISE_STATS: exact second moments of the per-pair Q32.32 contributions, [S][B+1][K] (lo, hi) mod 2^128, slot B
+    // broadband.  Allocated at the first trace with the flag; m2_valid = they belong to the histogram in d_hist (set by
+    // fs_trace / fs_trace_sources / fs_update* / fs_multi_trace*, cleared by every other call that writes d_hist)
+    ulonglong2* d_m2; uint32_t m2_sources; bool m2_valid;
+    double* d_noise; uint32_t noise_cap;    // fs_get_noise scratch: [S] path counts (u64), then [S][B+1] (signal, variance)
     void* d_src_tab; uint32_t src_tab_cap;  // per-source budgets on the device: [S+1] u64 offsets, then [S] u32 depths
     fs_dev_counters* d_counters;
     // traversal-stack overflow of the last trace: one 4-byte async copy into pinned memory after every fs_trace*, looked at
@@ -245,8 +250,9 @@ struct fs_ctx {
 // fs_wavefront.cu
 cudaError_t fs_wave_alloc(fs_ctx* ctx, fs_lane* lane, uint32_t cap, uint32_t max_depth);
 void fs_wave_free(fs_wave_buffers* wb);
+// d_m2: FS_FLAG_NOISE_STATS second moments [S][B+1][K] (lo, hi), accumulated by k_eval<false, true>; null = none
 cudaError_t fs_wave_trace_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_params& tp, unsigned long long* d_hist,
-                                fs_path_dbg* d_dbg);
+                                fs_path_dbg* d_dbg, ulonglong2* d_m2);
 cudaError_t fs_wave_reset_counters(fs_ctx* ctx, int reset_overflow);
 cudaError_t fs_wave_debug_rays(fs_ctx* ctx, const fs_trace_params& tp, const float* d_rays, const float* d_tmax,
                                uint64_t n, float* d_t, uint32_t* d_tri, uint8_t* d_hit);
@@ -260,6 +266,11 @@ cudaError_t fs_ir_build_bands(fs_ctx* ctx, const unsigned long long* d_hist_src,
                               float* d_ir_out);
 cudaError_t fs_ir_build(fs_ctx* ctx, const unsigned long long* d_hist_src, uint64_t n_paths,
                         const float* d_energy_in, float* d_ir_out);
+
+// fs_noise.cu: per (source, band or broadband) sum over bins of mu^2 and of Var(mu_hat) from the histogram, the second
+// moments and the per-source pair counts d_n [S]; out [S][B+1][2] (signal, variance), energy units.  Fixed-order double sums.
+cudaError_t fs_noise_reduce(const unsigned long long* d_hist, const ulonglong2* d_m2, const uint64_t* d_n, uint32_t n_sources,
+                            uint32_t n_bands, uint32_t n_bins, double* d_out, cudaStream_t st);
 
 // fs_conv.cu
 cudaError_t fs_conv_setup(fs_ctx* ctx);

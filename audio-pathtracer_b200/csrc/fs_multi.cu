@@ -20,8 +20,16 @@
 #include <new>
 #include <thread>
 
+// fs_api.cu
 int fs_internal_hist_prepare(fs_ctx* ctx, uint32_t n_sources, uint64_t n_paths, const uint64_t* per_source,
-                             unsigned long long** d_hist_out);   // fs_api.cu
+                             unsigned long long** d_hist_out, ulonglong2** d_m2_out);
+int fs_internal_trace_range(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3], uint64_t n_paths,
+                            uint64_t g_first, uint64_t g_count, uint32_t max_depth, uint64_t seed, void* d_hist,
+                            ulonglong2* d_m2, int zero_first);
+int fs_internal_trace_sources_range(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3],
+                                    uint64_t g_first, uint64_t g_count, uint64_t seed, void* d_hist, ulonglong2* d_m2,
+                                    int zero_first);
+void fs_internal_m2_valid(fs_ctx* ctx, bool valid);
 
 namespace {
 
@@ -38,6 +46,21 @@ __global__ void k_hist_sum(unsigned long long* __restrict__ hist, const unsigned
         unsigned long long s = hist[i];
         for (uint32_t k = 0; k < n_slots; ++k) s += staging[(size_t)k * slot_stride + i];
         hist[i] = s;
+    }
+}
+
+// FS_FLAG_NOISE_STATS: m2[j] += sum_i staging[i][j] mod 2^128 (carry from the low word into the high word)
+__global__ void k_m2_sum(ulonglong2* __restrict__ m2, const ulonglong2* __restrict__ staging, size_t n, uint32_t n_slots,
+                         size_t slot_stride)
+{
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        ulonglong2 s = m2[i];
+        for (uint32_t k = 0; k < n_slots; ++k) {
+            const ulonglong2 v = staging[(size_t)k * slot_stride + i];
+            s.x += v.x;
+            s.y += v.y + (s.x < v.x ? 1ull : 0ull);
+        }
+        m2[i] = s;
     }
 }
 
@@ -89,6 +112,10 @@ struct fs_multi {
     std::vector<cudaEvent_t> ev_pushed;            // [i] recorded on device i's stream after its peer store
     unsigned long long* d_staging = nullptr;       // on device 0: [n - 1][cap] slots
     size_t cap = 0;                                // u64 elements per slot
+    // FS_FLAG_NOISE_STATS: the same for the second moments, [S][B+1][K] (lo, hi) per slot
+    std::vector<ulonglong2*> d_local_m2;
+    ulonglong2* d_staging_m2 = nullptr;
+    size_t cap_m2 = 0;                             // ulonglong2 elements per slot
     cudaEvent_t ev_ready = nullptr, ev_t0 = nullptr, ev_t1 = nullptr, ev_t2 = nullptr;
     float last_total_ms = 0.f, last_reduce_ms = 0.f;
     std::string err;
@@ -142,7 +169,7 @@ int fs_multi_create(const fs_config* cfg, const int* devices, uint32_t n_devices
         if (cudaEventCreateWithFlags(&m->ev_ready, cudaEventDisableTiming) != cudaSuccess || cudaEventCreate(&m->ev_t0) != cudaSuccess ||
             cudaEventCreate(&m->ev_t1) != cudaSuccess || cudaEventCreate(&m->ev_t2) != cudaSuccess)
             rc = mfail(FS_ERR_CUDA, "cudaEventCreate");
-        m->d_local.assign(m->n, nullptr); m->ev_pushed.assign(m->n, nullptr);
+        m->d_local.assign(m->n, nullptr); m->d_local_m2.assign(m->n, nullptr); m->ev_pushed.assign(m->n, nullptr);
         for (uint32_t i = 1; i < m->n && rc == FS_OK; ++i) {
             cudaSetDevice(m->dev[i]);
             if (cudaEventCreateWithFlags(&m->ev_pushed[i], cudaEventDisableTiming) != cudaSuccess) rc = mfail(FS_ERR_CUDA, "cudaEventCreate");
@@ -171,11 +198,12 @@ void fs_multi_destroy(fs_multi* m)
         cudaSetDevice(m->dev[i]);
         cudaDeviceSynchronize();
         if (i < m->d_local.size()) cudaFree(m->d_local[i]);
+        if (i < m->d_local_m2.size()) cudaFree(m->d_local_m2[i]);
         if (i < m->ev_pushed.size() && m->ev_pushed[i]) cudaEventDestroy(m->ev_pushed[i]);
     }
     if (!m->dev.empty()) {
         cudaSetDevice(m->dev[0]);
-        cudaFree(m->d_staging);
+        cudaFree(m->d_staging); cudaFree(m->d_staging_m2);
         for (cudaEvent_t e : {m->ev_ready, m->ev_t0, m->ev_t1, m->ev_t2}) if (e) cudaEventDestroy(e);
     }
     for (fs_ctx* x : m->ctx) fs_destroy(x);
@@ -256,8 +284,11 @@ int fs_multi_scene_refit(fs_multi* m, float* cost_ratio_out)
 // follows without a host synchronisation).  hist_out (host [S][B][K]) may be NULL; non-NULL synchronises.
 // G: the flat work range [0, G); trace(ctx, first, count, d_hist, zero_first) traces one shard; n_paths / per_source: the
 // path counts context 0 records for its IR builders
+// With FS_FLAG_NOISE_STATS the second moments travel the same way (trace's ulonglong2* argument: the shard's buffer) and are
+// summed into context 0's with the carry.
 static int multi_trace_common(fs_multi* m, uint32_t n_sources, uint64_t G, uint64_t n_paths, const uint64_t* per_source,
-                              uint64_t* hist_out, const std::function<int(fs_ctx*, uint64_t, uint64_t, void*, int)>& trace)
+                              uint64_t* hist_out,
+                              const std::function<int(fs_ctx*, uint64_t, uint64_t, void*, ulonglong2*, int)>& trace)
 {
     cur_dev_guard guard;
     fs_ctx* c0 = m->ctx[0];
@@ -277,11 +308,28 @@ static int multi_trace_common(fs_multi* m, uint32_t n_sources, uint64_t G, uint6
         }
         m->cap = cap;
     }
+    const bool noise = (c0->cfg.flags & FS_FLAG_NOISE_STATS) != 0;
+    const size_t mn = noise ? (size_t)n_sources * (c0->cfg.n_bands + 1u) * c0->cfg.n_bins : 0;
+    if (m->cap_m2 < mn) {
+        cudaSetDevice(m->dev[0]);
+        cudaDeviceSynchronize();
+        cudaFree(m->d_staging_m2); m->d_staging_m2 = nullptr;
+        if (m->n > 1 && cudaMalloc(&m->d_staging_m2, sizeof(ulonglong2) * mn * (m->n - 1)) != cudaSuccess)
+            return mfail(FS_ERR_NOMEM, "fs_multi_trace: staging");
+        for (uint32_t i = 1; i < m->n; ++i) {
+            cudaSetDevice(m->dev[i]);
+            cudaDeviceSynchronize();
+            cudaFree(m->d_local_m2[i]); m->d_local_m2[i] = nullptr;
+            if (cudaMalloc(&m->d_local_m2[i], sizeof(ulonglong2) * mn) != cudaSuccess) return mfail(FS_ERR_NOMEM, "fs_multi_trace: shard moments");
+        }
+        m->cap_m2 = mn;
+    }
     unsigned long long* d_hist0 = nullptr;
+    ulonglong2* d_m20 = nullptr;
     {   // device 0: histogram of context 0, zeroed ("Flush", COMP.h:76-79)
         cudaSetDevice(m->dev[0]);
         if (cudaEventRecord(m->ev_t0, c0->stream) != cudaSuccess) return mfail(FS_ERR_CUDA, "cudaEventRecord");
-        int rc = fs_internal_hist_prepare(c0, n_sources, n_paths, per_source, &d_hist0);
+        int rc = fs_internal_hist_prepare(c0, n_sources, n_paths, per_source, &d_hist0, &d_m20);
         if (rc) return mfail(rc, fs_last_error(c0));
     }
     std::vector<std::string> errs(m->n);
@@ -290,7 +338,8 @@ static int multi_trace_common(fs_multi* m, uint32_t n_sources, uint64_t G, uint6
         const uint64_t first = i * base + (i < rem ? i : rem), count = base + (i < rem ? 1 : 0);
         fs_ctx* c = m->ctx[i];
         cudaSetDevice(m->dev[i]);
-        int r = trace(c, first, count, i == 0 ? (void*)d_hist0 : (void*)m->d_local[i], i == 0 ? 0 : 1);
+        int r = trace(c, first, count, i == 0 ? (void*)d_hist0 : (void*)m->d_local[i], i == 0 ? d_m20 : (noise ? m->d_local_m2[i] : nullptr),
+                      i == 0 ? 0 : 1);
         if (r) { errs[i] = fs_last_error(c); return r; }
         if (i > 0) {
             // hand-written peer store: this device's shard histogram -> its slot of the staging buffer on device 0
@@ -302,6 +351,12 @@ static int multi_trace_common(fs_multi* m, uint32_t n_sources, uint64_t G, uint6
             if (grid > 4u * (uint32_t)c->sm_count) grid = 4u * (uint32_t)c->sm_count;
             k_hist_peer_store<<<grid, 256, 0, c->stream>>>(reinterpret_cast<const ulonglong2*>(m->d_local[i]), remote, n2);
             c->launches.fetch_add(1);
+            if (noise) {
+                uint32_t grid2 = (uint32_t)((mn + 255) / 256);
+                if (grid2 > 4u * (uint32_t)c->sm_count) grid2 = 4u * (uint32_t)c->sm_count;
+                k_hist_peer_store<<<grid2, 256, 0, c->stream>>>(m->d_local_m2[i], m->d_staging_m2 + (size_t)(i - 1) * m->cap_m2, mn);
+                c->launches.fetch_add(1);
+            }
             cudaError_t e = cudaGetLastError();
             if (e == cudaSuccess) e = cudaEventRecord(m->ev_pushed[i], c->stream);
             if (e != cudaSuccess) { errs[i] = std::string("peer store: ") + cudaGetErrorString(e); return (int)FS_ERR_CUDA; }
@@ -318,7 +373,15 @@ static int multi_trace_common(fs_multi* m, uint32_t n_sources, uint64_t G, uint6
         k_hist_sum<<<grid, 256, 0, c0->stream>>>(d_hist0, m->d_staging, hn, m->n - 1, m->cap);
         c0->launches.fetch_add(1);
         if (cudaGetLastError() != cudaSuccess) return mfail(FS_ERR_CUDA, "k_hist_sum");
+        if (noise) {
+            uint32_t grid2 = (uint32_t)((mn + 255) / 256);
+            if (grid2 > 4u * (uint32_t)c0->sm_count) grid2 = 4u * (uint32_t)c0->sm_count;
+            k_m2_sum<<<grid2, 256, 0, c0->stream>>>(d_m20, m->d_staging_m2, mn, m->n - 1, m->cap_m2);
+            c0->launches.fetch_add(1);
+            if (cudaGetLastError() != cudaSuccess) return mfail(FS_ERR_CUDA, "k_m2_sum");
+        }
     }
+    if (noise) fs_internal_m2_valid(c0, true);
     cudaEventRecord(m->ev_t2, c0->stream);
     cudaEventRecord(m->ev_ready, c0->stream);                 // the staging slots may be overwritten by the next update
     if (hist_out) {
@@ -338,9 +401,9 @@ int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const 
     if (!m) return FS_ERR_INVALID;
     if (!src_pos || !lis_pos || n_sources == 0 || n_paths == 0) return mfail(FS_ERR_INVALID, "fs_multi_trace: bad argument");
     return multi_trace_common(m, n_sources, (uint64_t)n_sources * n_paths, n_paths, nullptr, hist_out,
-                              [&](fs_ctx* c, uint64_t first, uint64_t count, void* d_hist, int zero_first) {
-                                  return fs_trace_range_device(c, src_pos, n_sources, lis_pos, n_paths, first, count, max_depth,
-                                                               seed, d_hist, zero_first); });
+                              [&](fs_ctx* c, uint64_t first, uint64_t count, void* d_hist, ulonglong2* d_m2, int zero_first) {
+                                  return fs_internal_trace_range(c, src_pos, n_sources, lis_pos, n_paths, first, count, max_depth,
+                                                                 seed, d_hist, d_m2, zero_first); });
 }
 
 // fs_trace_sources over all devices: the flat range [0, sum n_s) is sharded like fs_multi_trace's
@@ -358,9 +421,9 @@ int fs_multi_trace_sources(fs_multi* m, const fs_source_desc* src, uint32_t n_so
         if (src[s].n_paths > n_max) n_max = src[s].n_paths;
     }
     return multi_trace_common(m, n_sources, G, n_max, counts.data(), hist_out,
-                              [&](fs_ctx* c, uint64_t first, uint64_t count, void* d_hist, int zero_first) {
-                                  return fs_trace_sources_range_device(c, src, n_sources, lis_pos, first, count, seed, d_hist,
-                                                                       zero_first); });
+                              [&](fs_ctx* c, uint64_t first, uint64_t count, void* d_hist, ulonglong2* d_m2, int zero_first) {
+                                  return fs_internal_trace_sources_range(c, src, n_sources, lis_pos, first, count, seed, d_hist,
+                                                                         d_m2, zero_first); });
 }
 
 // device time of the last fs_multi_trace on device 0's stream: the whole update (it ends when the slowest device has

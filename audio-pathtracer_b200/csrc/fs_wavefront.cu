@@ -344,6 +344,34 @@ __device__ __forceinline__ unsigned long long reduce_peers(uint32_t peers, unsig
     return v;
 }
 
+// reduce_peers for a 128-bit value (lo, hi): the second moment of FS_FLAG_NOISE_STATS.  Sums are taken mod 2^128.
+__device__ __forceinline__ void reduce_peers_u128(uint32_t peers, unsigned long long& lo, unsigned long long& hi)
+{
+    const uint32_t group = peers;
+    const uint32_t lane = lane_id();
+    uint32_t rel = __popc(peers & ((1u << lane) - 1u));
+    peers &= (0xfffffffeu << lane);
+    while (__any_sync(group, peers)) {
+        const int next = __ffs(peers);
+        const int src = next ? next - 1 : (int)lane;
+        const unsigned long long tl = __shfl_sync(group, lo, src), th = __shfl_sync(group, hi, src);
+        if (next) { lo += tl; hi += th + (lo < tl ? 1ull : 0ull); }
+        const bool done = rel & 1u;
+        if (done) peers = 0;
+        peers &= __ballot_sync(group, !done);
+        rel >>= 1;
+    }
+}
+
+// *p += (lo, hi) mod 2^128: one atomic on the low word, one on the high word with the carry of the first.  Every add is
+// exact mod 2^128, so the sum does not depend on the order of the adds.
+__device__ __forceinline__ void atomic_add_u128(ulonglong2* p, unsigned long long lo, unsigned long long hi)
+{
+    const unsigned long long old = atomicAdd(&p->x, lo);
+    if (old + lo < old) ++hi;
+    if (hi) atomicAdd(&p->y, hi);
+}
+
 // one band of one segment of EvaluatePath (SUB.cpp:368-399); P = prob^pdf_exponent comes from the node record
 __device__ __forceinline__ void eval_seg_band(const fs_eval_params& ep, float bs, float P, float d, float air_b, float& E)
 {
@@ -371,10 +399,12 @@ __device__ __forceinline__ fs_vec3 node_pos(const fs_trace_params& tp, const fs_
     return fs_mk(v.x, v.y, v.z);
 }
 
-template <bool ALL>
+// M2 (FS_FLAG_NOISE_STATS, endpoint connection only): also splats the exact square of every Q32.32 value into
+// m2 [S][B+1][K] (lo, hi): q_b^2 into slot b, and (sum_b q_b)^2 of the path into slot B (broadband)
+template <bool ALL, bool M2 = false>
 __global__ void __launch_bounds__(WF_THREADS)
 k_eval(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long long* __restrict__ hist,
-       fs_dev_counters* __restrict__ dc, fs_path_dbg* __restrict__ dbg)
+       fs_dev_counters* __restrict__ dc, fs_path_dbg* __restrict__ dbg, ulonglong2* __restrict__ m2)
 {
     const uint32_t lane = lane_id();
     const uint32_t sub = lane >> 3, b = lane & 7u;
@@ -392,7 +422,7 @@ k_eval(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long long* _
         const bool valid = (j < count) && band_on;
         unsigned long long q = 0ull;
         uint32_t key = 0xffffffffu;
-        size_t hidx = 0;
+        size_t hidx = 0, midx = 0;
         if (valid) {
             // ALL: the queue entry names a prefix pair (pair << 12 | (s-1) << 6 | (t-1)); the path is F[0..s) ++ reverse(B[0..t)),
             // its connecting segment is recomputed from the node positions, its weight is 1 / (s + t - 1)
@@ -459,20 +489,50 @@ k_eval(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long long* _
             q = (unsigned long long)(e * 4294967296.0f);                          // Q32.32
             hidx = ((size_t)s * NBr + b) * tp.n_bins + bin;
             key = (s * tp.n_bins + bin) * 8u + b;
+            if (M2) midx = ((size_t)s * (NBr + 1u) + b) * tp.n_bins + bin;
             if (dbg) {
                 dbg[p].energy[b] = e;
                 if (b == 0) { dbg[p].bin = (int32_t)bin; dbg[p].delay_s = delay; dbg[p].total_dist = total; }
             }
+        }
+        // broadband value of the path: its 8 lanes sum their q_b (lanes past n_bands and past the queue hold 0);
+        // q_b <= clamp * gain * 2^32, so the sum fits 64 bits for clamp * gain < 2^29
+        unsigned long long qs = 0ull;
+        if (M2) {
+            qs = q;
+            qs += __shfl_xor_sync(0xffffffffu, qs, 4);
+            qs += __shfl_xor_sync(0xffffffffu, qs, 2);
+            qs += __shfl_xor_sync(0xffffffffu, qs, 1);
         }
         // splat: lanes with the same (source, band, bin) combine first, one RED.64 per group
         const uint32_t active = __ballot_sync(0xffffffffu, valid);
         if (valid) {
             if (tp.flags & FS_FLAG_NO_SPLAT_AGG) {
                 atomicAdd(hist + hidx, q);
+                if (M2) {
+                    atomic_add_u128(m2 + midx, q * q, __umul64hi(q, q));
+                    if (b == 0) atomic_add_u128(m2 + midx + (size_t)NBr * tp.n_bins, qs * qs, __umul64hi(qs, qs));
+                }
             } else {
                 const uint32_t peers = __match_any_sync(active, key);
+                const bool leader = (uint32_t)(__ffs(peers) - 1) == lane;
+                if (M2) {
+                    unsigned long long lo = q * q, hi = __umul64hi(q, q);
+                    if (peers != (1u << lane)) reduce_peers_u128(peers, lo, hi);
+                    if (leader) atomic_add_u128(m2 + midx, lo, hi);
+                }
                 if (peers != (1u << lane)) q = reduce_peers(peers, q);
-                if ((uint32_t)(__ffs(peers) - 1) == lane) atomicAdd(hist + hidx, q);
+                if (leader) atomicAdd(hist + hidx, q);
+                if (M2) {
+                    // broadband: one lane per path (band 0), grouped by (source, bin)
+                    const uint32_t bb_active = __ballot_sync(active, b == 0);
+                    if (b == 0) {
+                        const uint32_t bpeers = __match_any_sync(bb_active, key >> 3);
+                        unsigned long long lo = qs * qs, hi = __umul64hi(qs, qs);
+                        if (bpeers != (1u << lane)) reduce_peers_u128(bpeers, lo, hi);
+                        if ((uint32_t)(__ffs(bpeers) - 1) == lane) atomic_add_u128(m2 + midx + (size_t)NBr * tp.n_bins, lo, hi);
+                    }
+                }
             }
         }
     }
@@ -2445,7 +2505,7 @@ void fs_wave_free(fs_wave_buffers* wb)
 
 template <bool COUNT, int MODE>
 static cudaError_t launch_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_params& tp, unsigned long long* d_hist,
-                                fs_path_dbg* d_dbg)
+                                fs_path_dbg* d_dbg, ulonglong2* d_m2)
 {
     cudaStream_t st = lane->stream;
     const fs_wave_buffers& wb = lane->wb;
@@ -2487,7 +2547,8 @@ static cudaError_t launch_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_param
     uint32_t grid_ev = (uint32_t)ctx->sm_count * 8u;
     const uint32_t ctas_ev = (tp.batch / 4u + WF_THREADS / 32 - 1) / (WF_THREADS / 32) + 1;
     if (grid_ev > ctas_ev) grid_ev = ctas_ev;
-    k_eval<false><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg);
+    if (d_m2) k_eval<false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, d_m2);
+    else k_eval<false><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, nullptr);
     ctx->launches.fetch_add(1);
     if (timing) cudaEventRecord(ev[3], st);
     return cudaGetLastError();
@@ -2500,7 +2561,7 @@ static cudaError_t launch_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_param
 // ---------------------------------------------------------------------------------------------
 template <bool COUNT>
 static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace_params& tp, unsigned long long* d_hist,
-                                      fs_path_dbg* d_dbg)
+                                      fs_path_dbg* d_dbg, ulonglong2* d_m2)
 {
     cudaStream_t st = lane->stream;
     fs_wave_buffers& wb = lane->wb;
@@ -2599,15 +2660,16 @@ static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace
     const uint32_t ctas_ev = (tp.batch / 4u + WF_THREADS / 32 - 1) / (WF_THREADS / 32) + 1;   // 4 paths per warp
     if (!all && grid_ev > ctas_ev) grid_ev = ctas_ev;
     if (tp.flags & FS_FLAG_MIS) k_eval_mis<<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters);
-    else if (all) k_eval<true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, nullptr);
-    else k_eval<false><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg);
+    else if (all) k_eval<true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, nullptr, nullptr);
+    else if (d_m2) k_eval<false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, d_m2);
+    else k_eval<false><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, nullptr);
     ctx->launches.fetch_add(1);
     if (timing) cudaEventRecord(ev[3], st);
     return cudaGetLastError();
 }
 
 cudaError_t fs_wave_trace_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_params& tp, unsigned long long* d_hist,
-                                fs_path_dbg* d_dbg)
+                                fs_path_dbg* d_dbg, ulonglong2* d_m2)
 {
     const bool count = (tp.flags & FS_FLAG_COUNT_VISITS) != 0;
     if (tp.src_off) {
@@ -2615,15 +2677,16 @@ cudaError_t fs_wave_trace_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_param
         ctx->launches.fetch_add(1);
     }
     if (!(tp.flags & (FS_FLAG_FUSED_EXTEND | FS_FLAG_BRUTE_FORCE)))
-        return count ? launch_batch_split<true>(ctx, lane, tp, d_hist, d_dbg) : launch_batch_split<false>(ctx, lane, tp, d_hist, d_dbg);
+        return count ? launch_batch_split<true>(ctx, lane, tp, d_hist, d_dbg, d_m2)
+                     : launch_batch_split<false>(ctx, lane, tp, d_hist, d_dbg, d_m2);
     switch (pick_mode(tp)) {
-    case MODE_BRUTE: return launch_batch<false, MODE_BRUTE>(ctx, lane, tp, d_hist, d_dbg);
+    case MODE_BRUTE: return launch_batch<false, MODE_BRUTE>(ctx, lane, tp, d_hist, d_dbg, d_m2);
     case MODE_TOP:
-        return count ? launch_batch<true, MODE_TOP>(ctx, lane, tp, d_hist, d_dbg)
-                     : launch_batch<false, MODE_TOP>(ctx, lane, tp, d_hist, d_dbg);
+        return count ? launch_batch<true, MODE_TOP>(ctx, lane, tp, d_hist, d_dbg, d_m2)
+                     : launch_batch<false, MODE_TOP>(ctx, lane, tp, d_hist, d_dbg, d_m2);
     default:
-        return count ? launch_batch<true, MODE_BVH>(ctx, lane, tp, d_hist, d_dbg)
-                     : launch_batch<false, MODE_BVH>(ctx, lane, tp, d_hist, d_dbg);
+        return count ? launch_batch<true, MODE_BVH>(ctx, lane, tp, d_hist, d_dbg, d_m2)
+                     : launch_batch<false, MODE_BVH>(ctx, lane, tp, d_hist, d_dbg, d_m2);
     }
 }
 

@@ -6,4 +6,4 @@ torch.distributed ranks.  The C++ mirror of the reference's UFrequenSeeAudioComp
 UAudioRayTracingSubsystem / FFrequenSeeAudioReverbPlugin interface is include/frequensee.hpp.
 """
 from . import capi, scenes  # noqa: F401
-from .capi import Context, MultiContext, FrequenSeeError, default_config, load_float_array, save_float_array  # noqa: F401
+from .capi import Context, MultiContext, FrequenSeeError, default_config, load_float_array, save_float_array, allocate_paths  # noqa: F401

@@ -22,6 +22,7 @@ FLAG_MATERIAL_MODEL = 256
 FLAG_MIS = 512
 FLAG_IR_NORMALIZE = 1024
 FLAG_CONV_CROSSFADE = 2048
+FLAG_NOISE_STATS = 4096
 
 # every symbol include/frequensee.h declares (tests/test_abi.py checks the library exports them all)
 ABI_SYMBOLS = [
@@ -30,6 +31,7 @@ ABI_SYMBOLS = [
     "fs_scene_update_vertices", "fs_scene_refit",
     "fs_trace", "fs_update", "fs_trace_range_device", "fs_trace_range", "fs_trace_debug",
     "fs_trace_sources", "fs_update_sources", "fs_trace_sources_range_device", "fs_set_histogram_sources_device",
+    "fs_get_noise", "fs_get_histogram_m2", "fs_allocate_paths",
     "fs_debug_closest_hits", "fs_debug_any_hits",
     "fs_build_ir", "fs_build_ir_to", "fs_build_ir_all", "fs_build_ir_bands", "fs_build_ir_from_energy", "fs_set_histogram", "fs_set_histogram_device",
     "fs_get_histogram", "fs_get_histogram_sources", "fs_set_ir", "fs_load_float_array", "fs_save_float_array",
@@ -137,6 +139,28 @@ def source_descs(src_pos, n_paths, depths):
     return arr
 
 
+class NoiseStats(C.Structure):
+    """fs_noise_stats: Monte Carlo noise of one source in the last update (FS_FLAG_NOISE_STATS)"""
+    _fields_ = [("n_paths", C.c_uint64), ("no_energy", C.c_uint32), ("reserved", C.c_uint32),
+                ("signal", C.c_double), ("variance", C.c_double), ("snr_db", C.c_double),
+                ("band_signal", C.c_double * MAX_BANDS), ("band_variance", C.c_double * MAX_BANDS),
+                ("band_snr_db", C.c_double * MAX_BANDS)]
+
+
+def noise_stats_array(d):
+    """fs_noise_stats[S] from the dict Context.noise_stats() returns (keys n_paths, no_energy, signal, variance, band_signal,
+    band_variance; snr values are not read by fs_allocate_paths)"""
+    S = len(d["n_paths"])
+    arr = (NoiseStats * S)()
+    for s in range(S):
+        arr[s].n_paths = int(d["n_paths"][s])
+        arr[s].no_energy = int(d["no_energy"][s])
+        arr[s].signal = float(d["signal"][s])
+        arr[s].variance = float(d["variance"][s])
+        arr[s].snr_db = float(d["snr_db"][s]) if "snr_db" in d else 0.0
+    return arr
+
+
 class FrequenSeeError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__("frequensee error %d: %s" % (code, msg))
@@ -180,6 +204,9 @@ def load():
     L.fs_update_sources.argtypes = [vp, vp, u32, vp, u64, vp, vp]
     L.fs_trace_sources_range_device.argtypes = [vp, vp, u32, vp, u64, u64, u64, vp, i32]
     L.fs_set_histogram_sources_device.argtypes = [vp, vp, u32, vp]
+    L.fs_get_noise.argtypes = [vp, vp, u32]
+    L.fs_get_histogram_m2.argtypes = [vp, vp]
+    L.fs_allocate_paths.argtypes = [vp, u32, u64, u64, u64, vp, vp]
     L.fs_debug_closest_hits.argtypes = [vp, vp, u64, vp, vp]
     L.fs_debug_any_hits.argtypes = [vp, vp, vp, u64, vp]
     L.fs_build_ir.argtypes = [vp, u32, vp]
@@ -454,6 +481,33 @@ class Context:
         self._ck(self.L.fs_get_histogram(self.h, hist.ctypes.data))
         return hist
 
+    def noise_stats(self):
+        """fs_get_noise: per-source noise of the last update as a dict of numpy arrays -- n_paths [S], no_energy [S] bool,
+        signal / variance / snr_db [S] (broadband) and band_signal / band_variance / band_snr_db [S][B]"""
+        n = C.c_uint32(0)
+        self._ck(self.L.fs_get_histogram_sources(self.h, C.byref(n)))
+        S, B = n.value, self.cfg.n_bands
+        arr = (NoiseStats * max(S, 1))()
+        self._ck(self.L.fs_get_noise(self.h, arr, S))
+        return {
+            "n_paths": np.array([arr[s].n_paths for s in range(S)], np.uint64),
+            "no_energy": np.array([bool(arr[s].no_energy) for s in range(S)]),
+            "signal": np.array([arr[s].signal for s in range(S)]),
+            "variance": np.array([arr[s].variance for s in range(S)]),
+            "snr_db": np.array([arr[s].snr_db for s in range(S)]),
+            "band_signal": np.array([list(arr[s].band_signal)[:B] for s in range(S)]).reshape(S, B),
+            "band_variance": np.array([list(arr[s].band_variance)[:B] for s in range(S)]).reshape(S, B),
+            "band_snr_db": np.array([list(arr[s].band_snr_db)[:B] for s in range(S)]).reshape(S, B),
+        }
+
+    def histogram_m2(self):
+        """fs_get_histogram_m2: second moments of the last update, uint64 [S][B+1][K][2] (lo, hi); slot B is broadband"""
+        n = C.c_uint32(0)
+        self._ck(self.L.fs_get_histogram_sources(self.h, C.byref(n)))
+        out = np.zeros((n.value, self.cfg.n_bands + 1, self.cfg.n_bins, 2), dtype=np.uint64)
+        self._ck(self.L.fs_get_histogram_m2(self.h, out.ctypes.data))
+        return out
+
     def build_ir(self, source=0, want_ir=True, out=None):
         shape = (self.cfg.n_channels, self.cfg.sample_rate)
         if out is not None:
@@ -621,6 +675,21 @@ class MultiContext:
 
     def __exit__(self, *a):
         self.close()
+
+
+def allocate_paths(stats, total, min_paths, max_paths, weight=None):
+    """fs_allocate_paths: ray budgets [S] (uint64, sum == total) for the next update from Context.noise_stats() of the last
+    one (a dict, or a NoiseStats array); host only, no context"""
+    L = load()
+    arr = stats if isinstance(stats, C.Array) else noise_stats_array(stats)
+    S = len(arr)
+    w = None if weight is None else np.ascontiguousarray(np.broadcast_to(np.asarray(weight, np.float32), (S,)))
+    out = np.zeros(S, np.uint64)
+    rc = L.fs_allocate_paths(arr, S, int(total), int(min_paths), int(max_paths), w.ctypes.data if w is not None else None,
+                             out.ctypes.data)
+    if rc != FS_OK:
+        raise FrequenSeeError(rc, "fs_allocate_paths: invalid argument")
+    return out
 
 
 def load_float_array(path):

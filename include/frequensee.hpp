@@ -74,6 +74,11 @@ public:
     bool bApplyReverb = true;
     int RaycastsPerTick = 1 << 20;     // path pairs per update (reference USED_RAY_COUNT = 1000, SUB.h:176)
     int RaycastBounces = 16;           // max depth (reference RaycastBounces = 10 / unbounded RR)
+    // weight of this emitter when UAudioRayTracingSubsystem::TotalRaysPerTick is split (fs_allocate_paths): a source of
+    // weight 2 is given twice the SNR of one of weight 1; 0 = as few rays as the bounds allow
+    float NoiseWeight = 1.0f;
+    // FS_FLAG_NOISE_STATS: the noise of this source in the last UpdateSources() (fs_get_noise; n_paths = the budget it had)
+    fs_noise_stats LastNoise{};
 
     std::vector<float> EnergyBuffer;   // COMP.h:70
     void FlushEnergyBuffer() { EnergyBuffer.assign(NumBins, 0.0f); bUseDeviceHistogram = false; }          // COMP.h:76-79
@@ -208,21 +213,43 @@ public:
     // s belongs to ActiveSources[s] until the next update, and each IR is published to its component's own convolver slot.
     // The random streams differ from UpdateSource's (one flat work range over all sources, fs_trace_sources), so this is
     // a separate entry point; ForceUpdateSources keeps the reference's one-update-per-source sequence.
+    //
+    // Automatic budgets (the allocateSamples the reference declares, SUB.h:136, and never defines): with TotalRaysPerTick > 0
+    // on a context created with FS_FLAG_NOISE_STATS, the components' RaycastsPerTick are ignored and TotalRaysPerTick is
+    // split over the active sources, each between MinRaysPerSource and MaxRaysPerSource (0 = TotalRaysPerTick).  The first
+    // update, and the first after the set of active sources has changed, splits it equally; every later one splits it with
+    // fs_allocate_paths from the noise of the previous update (each component's LastNoise) and its NoiseWeight.
+    // RaycastBounces stays per component.  A split the bounds make impossible fails the update (FS_ERR_INVALID in
+    // Ctx->LastStatus).
+    uint64_t TotalRaysPerTick = 0;     // 0: every source traces its own RaycastsPerTick
+    uint64_t MinRaysPerSource = 1024, MaxRaysPerSource = 0;
     void UpdateSources()
     {
         if (ActiveSources.empty() || !Commit()) return;
         const float lis[3] = {PawnLocation.X, PawnLocation.Y, PawnLocation.Z};
-        std::vector<fs_source_desc> desc(ActiveSources.size());
-        for (size_t s = 0; s < ActiveSources.size(); ++s) {
+        const uint32_t S = (uint32_t)ActiveSources.size();
+        const bool noise = (Ctx->Config().flags & FS_FLAG_NOISE_STATS) != 0;
+        std::vector<uint64_t> budget(S);
+        for (uint32_t s = 0; s < S; ++s) budget[s] = (uint64_t)ActiveSources[s]->RaycastsPerTick;
+        if (noise && TotalRaysPerTick > 0 && !SplitTotal(budget)) return;
+        std::vector<fs_source_desc> desc(S);
+        for (uint32_t s = 0; s < S; ++s) {
             const UFrequenSeeAudioComponent& c = *ActiveSources[s];
             const FVector3f L = c.GetActorLocation();
             desc[s].pos[0] = L.X; desc[s].pos[1] = L.Y; desc[s].pos[2] = L.Z;
             desc[s].max_depth = (uint32_t)c.RaycastBounces;
-            desc[s].n_paths = (uint64_t)c.RaycastsPerTick;
+            desc[s].n_paths = budget[s];
         }
-        if (Ctx->Check(fs_trace_sources(Ctx->Get(), desc.data(), (uint32_t)desc.size(), lis, Seed++, nullptr)) != FS_OK) return;
+        NoiseSources.clear();
+        if (Ctx->Check(fs_trace_sources(Ctx->Get(), desc.data(), S, lis, Seed++, nullptr)) != FS_OK) return;
         fs_stats st;
         if (fs_get_stats(Ctx->Get(), &st) == FS_OK) LastConnected = st.connected;
+        if (noise) {
+            std::vector<fs_noise_stats> ns(S);
+            if (Ctx->Check(fs_get_noise(Ctx->Get(), ns.data(), S)) != FS_OK) return;
+            for (uint32_t s = 0; s < S; ++s) ActiveSources[s]->LastNoise = ns[s];
+            NoiseSources = ActiveSources;
+        }
         for (size_t s = 0; s < ActiveSources.size(); ++s) {
             UFrequenSeeAudioComponent& c = *ActiveSources[s];
             std::vector<float> flat((size_t)c.NumChannels * c.SampleRate);
@@ -235,6 +262,24 @@ public:
     uint64_t LastConnected = 0;
 
 private:
+    // TotalRaysPerTick over the active sources: equally, or by fs_allocate_paths from the last update's noise when it
+    // belongs to the same sources
+    bool SplitTotal(std::vector<uint64_t>& budget)
+    {
+        const uint32_t S = (uint32_t)budget.size();
+        const uint64_t lo = MinRaysPerSource, hi = MaxRaysPerSource ? MaxRaysPerSource : TotalRaysPerTick;
+        if (NoiseSources == ActiveSources) {
+            std::vector<fs_noise_stats> ns(S);
+            std::vector<float> w(S);
+            for (uint32_t s = 0; s < S; ++s) { ns[s] = ActiveSources[s]->LastNoise; w[s] = ActiveSources[s]->NoiseWeight; }
+            return Ctx->Check(fs_allocate_paths(ns.data(), S, TotalRaysPerTick, lo, hi, w.data(), budget.data())) == FS_OK;
+        }
+        // equal split: fs_allocate_paths with the same demand everywhere
+        std::vector<fs_noise_stats> eq(S);
+        for (uint32_t s = 0; s < S; ++s) { eq[s] = fs_noise_stats{}; eq[s].n_paths = 1; eq[s].signal = 1.0; eq[s].variance = 1.0; }
+        return Ctx->Check(fs_allocate_paths(eq.data(), S, TotalRaysPerTick, lo, hi, nullptr, budget.data())) == FS_OK;
+    }
+    std::vector<UFrequenSeeAudioComponent*> NoiseSources;   // the sources whose LastNoise the last update filled
     bool Commit()
     {
         if (!bDirty) return CommitMoves();
