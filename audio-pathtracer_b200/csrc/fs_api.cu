@@ -5,6 +5,7 @@
 #include <nvtx3/nvToolsExt.h>          // header-only NVTX 3: named ranges per stage for nsys / ncu --nvtx (SURVEY section 5)
 #include <algorithm>
 #include <climits>
+#include <cmath>
 #include <stdio.h>
 #include <utility>
 #include <stdlib.h>
@@ -198,6 +199,7 @@ void fs_destroy(fs_ctx* ctx)
     fs_bvh_free(&ctx->bvh);
     cudaFree(ctx->d_verts); cudaFree(ctx->d_tri_mat); cudaFree(ctx->d_refl_over_pi);
     cudaFree(ctx->d_hist); cudaFree(ctx->d_m2); cudaFree(ctx->d_noise); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
+    cudaFree(ctx->d_dir_gain); cudaFree(ctx->d_dir_orient);
     cudaFree(ctx->d_amp); cudaFree(ctx->d_energy);
     for (cudaEvent_t e : ctx->kev) cudaEventDestroy(e);
     for (cudaEvent_t e : ctx->tev) cudaEventDestroy(e);
@@ -505,6 +507,16 @@ static void fill_params(fs_ctx* ctx, fs_trace_params* tp, const float lis[3], ui
     tp->src_pos = ctx->d_src_pos;
     if (lis) { tp->lis[0] = lis[0]; tp->lis[1] = lis[1]; tp->lis[2] = lis[2]; }
     tp->flags = c.flags;
+    tp->dir_orient = ctx->dir_sources ? ctx->d_dir_orient : nullptr;
+    tp->dir_gain = ctx->d_dir_gain; tp->n_dir_patterns = ctx->dir_patterns;
+}
+
+// with source orientations installed, a trace must name exactly that many sources; checked before anything is enqueued
+static int check_dir_sources(fs_ctx* ctx, uint32_t n_sources, const char* who)
+{
+    if (!ctx->dir_sources || n_sources == ctx->dir_sources) return FS_OK;
+    return fail(ctx, FS_ERR_INVALID, (std::string(who) + ": n_sources (" + std::to_string(n_sources) + ") differs from the " +
+                                      std::to_string(ctx->dir_sources) + " source orientations installed by fs_set_source_directivity").c_str());
 }
 
 static int ensure_hist(fs_ctx* ctx, uint32_t n_sources)
@@ -617,6 +629,7 @@ static int trace_common(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, c
     const uint64_t G = tab ? tab->off[n_sources] : (uint64_t)n_sources * n_paths;
     if (g_first + g_count > G || g_first + g_count < g_first) return fail(ctx, FS_ERR_INVALID, "fs_trace: work range exceeds the sources' paths");
     if ((uint64_t)n_sources * ctx->cfg.n_bins >= 0xffffffffull) return fail(ctx, FS_ERR_INVALID, "fs_trace: n_sources * n_bins too large");
+    if (int rc = check_dir_sources(ctx, n_sources, "fs_trace")) return rc;
     // an overflow of the PREVIOUS trace that nobody has looked at yet: report it now if its flag has landed; if it is
     // still in flight the device flag is left set (reset_ovf = 0) so that this call's copy carries it
     int rc_ovf = check_overflow(ctx, false);
@@ -799,7 +812,9 @@ int fs_trace(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float 
     if (!ctx) return FS_ERR_INVALID;
     dev_guard g(ctx->device);
     if (n_sources == 0) return fail(ctx, FS_ERR_INVALID, "fs_trace: no source");
-    int rc = ensure_hist(ctx, n_sources);
+    int rc = check_dir_sources(ctx, n_sources, "fs_trace");
+    if (rc) return rc;
+    rc = ensure_hist(ctx, n_sources);
     if (rc) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemsetAsync(ctx->d_hist, 0, 8 * hn, ctx->stream));            // FlushEnergyBuffer, COMP.h:76-79
@@ -824,6 +839,7 @@ static int trace_range_device(fs_ctx* ctx, const float* src_pos, uint32_t n_sour
 {
     if (!ctx) return FS_ERR_INVALID;
     if (!d_hist) return fail(ctx, FS_ERR_INVALID, "fs_trace_range_device: null histogram");
+    if (int rc = check_dir_sources(ctx, n_sources, "fs_trace_range_device")) return rc;
     dev_guard g(ctx->device);
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     if (zero_first) CK(cudaMemsetAsync(d_hist, 0, 8 * hn, ctx->stream));
@@ -846,7 +862,9 @@ int fs_trace_range(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const 
     if (!ctx) return FS_ERR_INVALID;
     if (!hist_inout) return fail(ctx, FS_ERR_INVALID, "fs_trace_range: null histogram");
     dev_guard g(ctx->device);
-    int rc = ensure_hist(ctx, n_sources);
+    int rc = check_dir_sources(ctx, n_sources, "fs_trace_range");
+    if (rc) return rc;
+    rc = ensure_hist(ctx, n_sources);
     if (rc) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
     CK(cudaMemcpyAsync(ctx->d_hist, hist_inout, 8 * hn, cudaMemcpyHostToDevice, ctx->stream));
@@ -863,7 +881,9 @@ int fs_trace_debug(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const 
     if (!ctx) return FS_ERR_INVALID;
     if (!dbg_out) return fail(ctx, FS_ERR_INVALID, "fs_trace_debug: null output");
     dev_guard g(ctx->device);
-    int rc = ensure_hist(ctx, n_sources);
+    int rc = check_dir_sources(ctx, n_sources, "fs_trace_debug");
+    if (rc) return rc;
+    rc = ensure_hist(ctx, n_sources);
     if (rc) return rc;
     if (ctx->dbg_cap < g_count) {
         cudaFree(ctx->d_dbg); ctx->d_dbg = nullptr; ctx->dbg_cap = 0;
@@ -1161,7 +1181,7 @@ int fs_trace_sources(fs_ctx* ctx, const fs_source_desc* src, uint32_t n_sources,
     nvtx_range nv("fs_trace_sources");
     fs_src_table t;
     int rc = prepare_sources(ctx, "fs_trace_sources", src, n_sources, lis_pos, &t);
-    if (rc) return rc;
+    if (rc || (rc = check_dir_sources(ctx, n_sources, "fs_trace_sources"))) return rc;
     dev_guard g(ctx->device);
     if ((rc = ensure_hist(ctx, n_sources))) return rc;
     const size_t hn = (size_t)n_sources * ctx->cfg.n_bands * ctx->cfg.n_bins;
@@ -1207,7 +1227,7 @@ static int trace_sources_range_device(fs_ctx* ctx, const fs_source_desc* src, ui
     if (!d_hist) return fail(ctx, FS_ERR_INVALID, "fs_trace_sources_range_device: null histogram");
     fs_src_table t;
     int rc = prepare_sources(ctx, "fs_trace_sources_range_device", src, n_sources, lis_pos, &t);
-    if (rc) return rc;
+    if (rc || (rc = check_dir_sources(ctx, n_sources, "fs_trace_sources_range_device"))) return rc;
     if (g_first + g_count > t.off[n_sources] || g_first + g_count < g_first)
         return fail(ctx, FS_ERR_INVALID, "fs_trace_sources_range_device: work range exceeds the sum of the path counts");
     dev_guard g(ctx->device);
@@ -1424,6 +1444,86 @@ int fs_get_histogram_m2(fs_ctx* ctx, uint64_t* out)
     return finish_stats(ctx);
 }
 
+// ---- directional sources ------------------------------------------------------------------------
+// The tables live on the device and are replaced by stream-ordered copies on the context stream: a trace enqueued before a
+// set call reads the old contents, one enqueued after it the new.  The host data is copied into a pageable vector first, so
+// the caller's buffer is free when the call returns whatever memory it is.
+int fs_set_directivity_patterns(fs_ctx* ctx, const fs_directivity* patterns, uint32_t n_patterns)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!patterns || n_patterns < 1 || n_patterns > 256)
+        return fail(ctx, FS_ERR_INVALID, "fs_set_directivity_patterns: 1..256 patterns needed");
+    for (uint32_t p = 0; p < n_patterns; ++p)
+        for (uint32_t b = 0; b < ctx->cfg.n_bands; ++b)
+            for (int i = 0; i < FS_DIR_POINTS; ++i) {
+                const float v = patterns[p].gain[b][i];
+                if (!(v >= 0.0f) || !std::isfinite(v))
+                    return fail(ctx, FS_ERR_INVALID, ("fs_set_directivity_patterns: gain of pattern " + std::to_string(p) + ", band " +
+                                                      std::to_string(b) + " is negative or not finite").c_str());
+            }
+    dev_guard g(ctx->device);
+    const size_t n = (size_t)n_patterns * FS_MAX_BANDS * FS_DIR_POINTS;
+    std::vector<float> h(n);
+    memcpy(h.data(), patterns, sizeof(float) * n);
+    if (!ctx->d_dir_gain) CK(cudaMalloc(&ctx->d_dir_gain, sizeof(float) * FS_MAX_BANDS * FS_DIR_POINTS * 256));   // 270 KB, the largest table
+    CK(cudaMemcpyAsync(ctx->d_dir_gain, h.data(), sizeof(float) * n, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->dir_patterns = n_patterns;
+    ctx->dir_sources = 0;                        // the orientations named indices of the old table
+    return FS_OK;
+}
+
+int fs_set_source_directivity(fs_ctx* ctx, const fs_source_orient* o, uint32_t n_sources)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (n_sources == 0) { ctx->dir_sources = 0; return FS_OK; }
+    if (!o) return fail(ctx, FS_ERR_INVALID, "fs_set_source_directivity: null orientations");
+    std::vector<float4> h(n_sources);
+    for (uint32_t s = 0; s < n_sources; ++s) {
+        const std::string who = "fs_set_source_directivity: source " + std::to_string(s);
+        const uint32_t pat = o[s].pattern;
+        if (pat != FS_OMNI && !ctx->dir_patterns)
+            return fail(ctx, FS_ERR_INVALID, (who + ": pattern index without an installed pattern table (fs_set_directivity_patterns)").c_str());
+        if (pat != FS_OMNI && pat >= ctx->dir_patterns)
+            return fail(ctx, FS_ERR_INVALID, (who + ": pattern index " + std::to_string(pat) + " >= the " +
+                                              std::to_string(ctx->dir_patterns) + " installed patterns").c_str());
+        const double x = o[s].forward[0], y = o[s].forward[1], z = o[s].forward[2];
+        const double len = sqrt(x * x + y * y + z * z);
+        if (!std::isfinite(x) || !std::isfinite(y) || !std::isfinite(z) || !(len > 0.0))
+            return fail(ctx, FS_ERR_INVALID, (who + ": forward must be a non-zero finite vector").c_str());
+        h[s] = make_float4((float)(x / len), (float)(y / len), (float)(z / len), 0.0f);
+        uint32_t bits = pat;
+        memcpy(&h[s].w, &bits, 4);
+    }
+    dev_guard g(ctx->device);
+    if (ctx->dir_orient_cap < n_sources) {
+        cudaFree(ctx->d_dir_orient); ctx->d_dir_orient = nullptr; ctx->dir_orient_cap = 0; ctx->dir_sources = 0;
+        CK(cudaMalloc(&ctx->d_dir_orient, sizeof(float4) * n_sources));
+        ctx->dir_orient_cap = n_sources;
+    }
+    CK(cudaMemcpyAsync(ctx->d_dir_orient, h.data(), sizeof(float4) * n_sources, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->dir_sources = n_sources;
+    return FS_OK;
+}
+
+int fs_directivity_polar(const float* dipole_weight, const float* power, uint32_t n_bands, fs_directivity* out)
+{
+    if (!dipole_weight || !power || !out || n_bands < 1 || n_bands > FS_MAX_BANDS)
+        return fail(nullptr, FS_ERR_INVALID, "fs_directivity_polar: null argument or n_bands outside 1..8");
+    for (uint32_t b = 0; b < n_bands; ++b) {
+        if (!(dipole_weight[b] >= 0.0f && dipole_weight[b] <= 1.0f))
+            return fail(nullptr, FS_ERR_INVALID, "fs_directivity_polar: dipole weight outside [0, 1]");
+        if (!(power[b] >= 0.0f && power[b] <= 64.0f))
+            return fail(nullptr, FS_ERR_INVALID, "fs_directivity_polar: power outside [0, 64]");
+    }
+    memset(out, 0, sizeof(*out));
+    for (uint32_t b = 0; b < n_bands; ++b)
+        for (int i = 0; i < FS_DIR_POINTS; ++i) {
+            const double c = -1.0 + i / 16.0, w = dipole_weight[b];
+            out->gain[b][i] = (float)pow(fabs((1.0 - w) + w * c), (double)power[b]);
+        }
+    return FS_OK;
+}
+
 int fs_get_stats(fs_ctx* ctx, fs_stats* out)
 {
     if (!ctx || !out) return FS_ERR_INVALID;
@@ -1471,6 +1571,7 @@ int fs_internal_trace_sources_range(fs_ctx* ctx, const fs_source_desc* src, uint
 }
 // fs_multi.cu: the reduced second moments of context 0 belong to its histogram
 void fs_internal_m2_valid(fs_ctx* ctx, bool valid) { ctx->m2_valid = valid; }
+int fs_internal_check_dir_sources(fs_ctx* ctx, uint32_t n_sources, const char* who) { return check_dir_sources(ctx, n_sources, who); }
 
 // ---- text float arrays (saved_ir.txt: one float per line, COMP.cpp:454-505); host only
 int fs_load_float_array(const char* path, float* out, uint64_t cap, uint64_t* n_out)

@@ -13,6 +13,7 @@
 #include "../../include/frequensee.h"
 #include "fs_math.cuh"
 #include "fs_bvh.cuh"
+#include "fs_directivity.h"
 
 #define FS_TOP_CAP 1024          // nodes of the shared-memory treelet (64 KB)
 
@@ -95,6 +96,11 @@ struct fs_trace_params {
     uint32_t lis_mode;
     float4* lis_rec;            // cache [max_depth+1][n_paths]: node records of listener subpath i
     float4* lis_end;            // cache [n_paths]: (end.xyz, bits(n_nodes))
+    // directional sources (fs_set_source_directivity): null = none (k_eval<..., false>).  dir_orient [S]: (unit forward.xyz,
+    // bits(pattern index or FS_OMNI)); dir_gain [P][FS_MAX_BANDS][FS_DIR_POINTS] energy gains (fs_directivity.h)
+    const float4* dir_orient;
+    const float* dir_gain;
+    uint32_t n_dir_patterns;
 };
 
 struct fs_wave_buffers {
@@ -212,6 +218,10 @@ struct fs_ctx {
     ulonglong2* d_m2; uint32_t m2_sources; bool m2_valid;
     double* d_noise; uint32_t noise_cap;    // fs_get_noise scratch: [S] path counts (u64), then [S][B+1] (signal, variance)
     void* d_src_tab; uint32_t src_tab_cap;  // per-source budgets on the device: [S+1] u64 offsets, then [S] u32 depths
+    // directional sources: the installed pattern table [P][FS_MAX_BANDS][FS_DIR_POINTS] and orientations [dir_sources]
+    // (float4: unit forward, bits(pattern)); dir_sources = 0: none installed, every source omni
+    float* d_dir_gain; uint32_t dir_patterns;
+    float4* d_dir_orient; uint32_t dir_sources, dir_orient_cap;
     fs_dev_counters* d_counters;
     // traversal-stack overflow of the last trace: one 4-byte async copy into pinned memory after every fs_trace*, looked at
     // by the next call that can (sticky until reported)

@@ -30,6 +30,7 @@ int fs_internal_trace_sources_range(fs_ctx* ctx, const fs_source_desc* src, uint
                                     uint64_t g_first, uint64_t g_count, uint64_t seed, void* d_hist, ulonglong2* d_m2,
                                     int zero_first);
 void fs_internal_m2_valid(fs_ctx* ctx, bool valid);
+int fs_internal_check_dir_sources(fs_ctx* ctx, uint32_t n_sources, const char* who);
 
 namespace {
 
@@ -291,6 +292,8 @@ static int multi_trace_common(fs_multi* m, uint32_t n_sources, uint64_t G, uint6
                               const std::function<int(fs_ctx*, uint64_t, uint64_t, void*, ulonglong2*, int)>& trace)
 {
     cur_dev_guard guard;
+    for (fs_ctx* c : m->ctx)                                  // before anything is enqueued on any device
+        if (int r = fs_internal_check_dir_sources(c, n_sources, "fs_multi_trace")) return mfail(r, fs_last_error(c));
     fs_ctx* c0 = m->ctx[0];
     const size_t hn = (size_t)n_sources * c0->cfg.n_bands * c0->cfg.n_bins;
     const size_t cap = (hn + 1) & ~(size_t)1;                 // 16-byte vector stores
@@ -424,6 +427,24 @@ int fs_multi_trace_sources(fs_multi* m, const fs_source_desc* src, uint32_t n_so
                               [&](fs_ctx* c, uint64_t first, uint64_t count, void* d_hist, ulonglong2* d_m2, int zero_first) {
                                   return fs_internal_trace_sources_range(c, src, n_sources, lis_pos, first, count, seed, d_hist,
                                                                          d_m2, zero_first); });
+}
+
+// directional sources: every device weights its shard's paths with the same tables
+int fs_multi_set_directivity_patterns(fs_multi* m, const fs_directivity* patterns, uint32_t n_patterns)
+{
+    if (!m) return FS_ERR_INVALID;
+    std::vector<std::string> errs(m->n);
+    int rc = on_all(m, [&](uint32_t i) { int r = fs_set_directivity_patterns(m->ctx[i], patterns, n_patterns); if (r) errs[i] = fs_last_error(m->ctx[i]); return r; });
+    if (rc) for (auto& e : errs) if (!e.empty()) { mfail(rc, e); break; }
+    return rc;
+}
+int fs_multi_set_source_directivity(fs_multi* m, const fs_source_orient* o, uint32_t n_sources)
+{
+    if (!m) return FS_ERR_INVALID;
+    std::vector<std::string> errs(m->n);
+    int rc = on_all(m, [&](uint32_t i) { int r = fs_set_source_directivity(m->ctx[i], o, n_sources); if (r) errs[i] = fs_last_error(m->ctx[i]); return r; });
+    if (rc) for (auto& e : errs) if (!e.empty()) { mfail(rc, e); break; }
+    return rc;
 }
 
 // device time of the last fs_multi_trace on device 0's stream: the whole update (it ends when the slowest device has

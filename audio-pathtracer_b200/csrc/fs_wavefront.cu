@@ -399,9 +399,33 @@ __device__ __forceinline__ fs_vec3 node_pos(const fs_trace_params& tp, const fs_
     return fs_mk(v.x, v.y, v.z);
 }
 
+// Directional sources: energy gain of band b for a path of source s that leaves it along the unit direction (dx, dy, dz);
+// 1 for an omni source (fs_directivity.h has the interpolation rule)
+__device__ __forceinline__ float dir_gain(const fs_trace_params& tp, uint32_t s, uint32_t b, float dx, float dy, float dz)
+{
+    const float4 o = __ldg(tp.dir_orient + s);
+    const uint32_t pat = __float_as_uint(o.w);
+    if (pat == FS_OMNI) return 1.0f;
+    float t;
+    const uint32_t i = fs_dir_index(fs_dir_cos(dx, dy, dz, o.x, o.y, o.z), &t);
+    const float* T = tp.dir_gain + ((size_t)pat * FS_MAX_BANDS + b) * FS_DIR_POINTS + i;
+    return fs_dir_lerp(__ldg(T), __ldg(T + 1), t);
+}
+
+// bounce-0 direction of the source subpath of work index g: what choose_direction / k_extend drew at node 0
+__device__ __forceinline__ fs_vec3 source_bounce0(const fs_trace_params& tp, uint64_t g)
+{
+    uint32_t r[4];
+    fs_philox4x32_10((uint32_t)g, (uint32_t)(g >> 32), 0u, 0u, tp.seed_lo, tp.seed_hi, r);
+    return fs_sample_sphere(fs_u01(r[1]), fs_u01(r[2]));
+}
+
 // M2 (FS_FLAG_NOISE_STATS, endpoint connection only): also splats the exact square of every Q32.32 value into
 // m2 [S][B+1][K] (lo, hi): q_b^2 into slot b, and (sum_b q_b)^2 of the path into slot B (broadband)
-template <bool ALL, bool M2 = false>
+// DIR (directional sources, tp.dir_orient set): every band starts at the gain of its source's pattern at the path's emission
+// direction instead of 1.  The 8 lanes of a path compute that direction redundantly: they run in lockstep, so one lane
+// doing it alone would cost the warp the same issue slots and add shuffles to hand the result out.
+template <bool ALL, bool M2 = false, bool DIR = false>
 __global__ void __launch_bounds__(WF_THREADS)
 k_eval(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long long* __restrict__ hist,
        fs_dev_counters* __restrict__ dc, fs_path_dbg* __restrict__ dbg, ulonglong2* __restrict__ m2)
@@ -432,11 +456,26 @@ k_eval(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long long* _
             const uint32_t nf = ALL ? ((id >> 6) & 63u) + 1u : __float_as_uint(wb.end_pos[sf].w);
             const uint32_t nb = ALL ? (id & 63u) + 1u : __float_as_uint(wb.end_pos[sb].w);
             float len;
+            fs_vec3 dl;
             if (ALL) {
-                const fs_vec3 dl = fs_sub(node_pos(tp, wb, sb, nb - 1u, stride), node_pos(tp, wb, sf, nf - 1u, stride));
+                dl = fs_sub(node_pos(tp, wb, sb, nb - 1u, stride), node_pos(tp, wb, sf, nf - 1u, stride));
                 len = sqrtf(fs_dot(dl, dl));
             } else len = wb.conn_len[p];
             float E = 1.0f, total = 0.0f;
+            if (DIR) {
+                // emission direction: the bounce-0 sample if the source prefix left node 0, else the connection ray's
+                fs_vec3 d;
+                if (nf >= 2u) d = source_bounce0(tp, tp.g_first + p);
+                else {
+                    if (!ALL) {
+                        const float4 fe = wb.end_pos[sf], be = wb.end_pos[sb];
+                        dl = fs_sub(fs_mk(be.x, be.y, be.z), fs_mk(fe.x, fe.y, fe.z));
+                    }
+                    const float inv = 1.0f / len;
+                    d = fs_mk(dl.x * inv, dl.y * inv, dl.z * inv);
+                }
+                E = dir_gain(tp, pair_source(tp, wb, p), b, d.x, d.y, d.z);
+            }
             float bs = 1.0f, P = 1.0f;                    // node 0 of the source subpath: no material, probability 1
             const float4* __restrict__ rf = wb.rec + sf;
             const float4* __restrict__ rb = wb.rec + sb;
@@ -560,6 +599,8 @@ __device__ __forceinline__ void mis_vertex(const fs_trace_params& tp, const fs_w
     N = fs_mk(nv.x, nv.y, nv.z);
 }
 
+// DIR: f starts at the gain of the source's pattern at normalize(x1 - x0), the direction of the path's first edge
+template <bool DIR = false>
 __global__ void __launch_bounds__(WF_THREADS)
 k_eval_mis(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long long* __restrict__ hist, fs_dev_counters* __restrict__ dc)
 {
@@ -589,7 +630,7 @@ k_eval_mis(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long lon
             const uint32_t k = s + t;
             float total = 0.0f;
             bool ok = k <= (uint32_t)FS_MIS_MAXV;
-            fs_vec3 Pa, Na;
+            fs_vec3 Pa, Na, d0;
             if (ok) mis_vertex(tp, wb, sf, sb, s, k, 0u, stride, Pa, Na);
             for (uint32_t i = 0; ok && i + 1u < k; ++i) {
                 fs_vec3 Pb, Nb;
@@ -601,6 +642,7 @@ k_eval_mis(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long lon
                 if (d < tp.ep.min_seg) { ok = false; break; }
                 const float inv = 1.0f / d;
                 const fs_vec3 dir = fs_mk(dl.x * inv, dl.y * inv, dl.z * inv);
+                if (DIR && i == 0u) d0 = dir;
                 const float cp = (i == 0u) ? 1.0f : fabsf(fs_dot(Na, dir));
                 const float cm = (i + 2u == k) ? 1.0f : fabsf(fs_dot(Nb, dir));
                 const float rd2 = 1.0f / d2;
@@ -618,6 +660,7 @@ k_eval_mis(const fs_trace_params tp, const fs_wave_buffers wb, unsigned long lon
                 r = 1.0f;
                 for (uint32_t sp = s; sp > 1u && k - sp <= depth; --sp) { r = r * (pb[sp - 1u] / pf[sp - 2u]); sum += r; }
                 float val = FS_INV_4PI;
+                if (DIR) val = dir_gain(tp, pair_source(tp, wb, p), b, d0.x, d0.y, d0.z) * FS_INV_4PI;
                 for (uint32_t i = 0; i + 1u < k; ++i) {
                     val = val * gg[i];
                     val = val * fs_exp(-air_b * dlen[i]);
@@ -2547,7 +2590,10 @@ static cudaError_t launch_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_param
     uint32_t grid_ev = (uint32_t)ctx->sm_count * 8u;
     const uint32_t ctas_ev = (tp.batch / 4u + WF_THREADS / 32 - 1) / (WF_THREADS / 32) + 1;
     if (grid_ev > ctas_ev) grid_ev = ctas_ev;
-    if (d_m2) k_eval<false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, d_m2);
+    const bool dir = tp.dir_orient != nullptr;
+    if (dir && d_m2) k_eval<false, true, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, d_m2);
+    else if (dir) k_eval<false, false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, nullptr);
+    else if (d_m2) k_eval<false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, d_m2);
     else k_eval<false><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, nullptr);
     ctx->launches.fetch_add(1);
     if (timing) cudaEventRecord(ev[3], st);
@@ -2659,7 +2705,13 @@ static cudaError_t launch_batch_split(fs_ctx* ctx, fs_lane* lane, const fs_trace
     uint32_t grid_ev = (uint32_t)ctx->sm_count * 8u;
     const uint32_t ctas_ev = (tp.batch / 4u + WF_THREADS / 32 - 1) / (WF_THREADS / 32) + 1;   // 4 paths per warp
     if (!all && grid_ev > ctas_ev) grid_ev = ctas_ev;
-    if (tp.flags & FS_FLAG_MIS) k_eval_mis<<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters);
+    if (tp.dir_orient) {                          // directional sources: the same kernels, each band starting at its gain
+        if (tp.flags & FS_FLAG_MIS) k_eval_mis<true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters);
+        else if (all) k_eval<true, false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, nullptr, nullptr);
+        else if (d_m2) k_eval<false, true, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, d_m2);
+        else k_eval<false, false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, nullptr);
+    }
+    else if (tp.flags & FS_FLAG_MIS) k_eval_mis<false><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters);
     else if (all) k_eval<true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, nullptr, nullptr);
     else if (d_m2) k_eval<false, true><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, d_m2);
     else k_eval<false><<<grid_ev, WF_THREADS, 0, st>>>(tp, wb, d_hist, ctx->d_counters, d_dbg, nullptr);

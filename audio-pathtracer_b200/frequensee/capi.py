@@ -23,6 +23,8 @@ FLAG_MIS = 512
 FLAG_IR_NORMALIZE = 1024
 FLAG_CONV_CROSSFADE = 2048
 FLAG_NOISE_STATS = 4096
+DIR_POINTS = 33          # FS_DIR_POINTS: directivity tables are sampled at cos = -1 + i/16
+OMNI = 0xFFFFFFFF        # FS_OMNI: a source without a pattern
 
 # every symbol include/frequensee.h declares (tests/test_abi.py checks the library exports them all)
 ABI_SYMBOLS = [
@@ -42,6 +44,8 @@ ABI_SYMBOLS = [
     "fs_multi_scene_set_triangles", "fs_multi_scene_set_materials", "fs_multi_scene_set_materials_ex", "fs_multi_scene_commit",
     "fs_multi_scene_update_vertices", "fs_multi_scene_refit",
     "fs_multi_trace", "fs_multi_trace_sources", "fs_multi_last_ms", "fs_multi_synchronize",
+    "fs_set_directivity_patterns", "fs_set_source_directivity", "fs_directivity_polar",
+    "fs_multi_set_directivity_patterns", "fs_multi_set_source_directivity",
 ]
 
 
@@ -137,6 +141,34 @@ def source_descs(src_pos, n_paths, depths):
         arr[s].max_depth = int(d[s])
         arr[s].n_paths = int(n[s])
     return arr
+
+
+class SourceOrient(C.Structure):
+    """fs_source_orient: forward axis and pattern index (or OMNI) of one directional source"""
+    _fields_ = [("forward", C.c_float * 3), ("pattern", C.c_uint32)]
+
+
+def _patterns(gains):
+    """fs_directivity[P] from energy gains [P][B][33] (B <= 8; missing bands are zero and ignored)"""
+    g = np.asarray(gains, dtype=np.float32)
+    if g.ndim == 2:
+        g = g[None]
+    if g.ndim != 3 or g.shape[1] > MAX_BANDS or g.shape[2] != DIR_POINTS:
+        raise ValueError("gains must be [P][B][%d] with B <= %d" % (DIR_POINTS, MAX_BANDS))
+    full = np.zeros((g.shape[0], MAX_BANDS, DIR_POINTS), np.float32)
+    full[:, :g.shape[1]] = g
+    return full
+
+
+def _orients(forward, pattern):
+    """fs_source_orient[S] from forward axes [S][3] and pattern indices [S] (OMNI for an omni source)"""
+    f = np.asarray(forward, dtype=np.float32).reshape(-1, 3)
+    pat = np.broadcast_to(np.asarray(pattern, dtype=np.uint64), (len(f),))
+    arr = (SourceOrient * max(len(f), 1))()
+    for s in range(len(f)):
+        arr[s].forward[:] = [float(v) for v in f[s]]
+        arr[s].pattern = int(pat[s])
+    return arr, len(f)
 
 
 class NoiseStats(C.Structure):
@@ -250,6 +282,11 @@ def load():
     L.fs_multi_trace_sources.argtypes = [vp, vp, u32, vp, u64, vp]
     L.fs_multi_last_ms.argtypes = [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     L.fs_multi_synchronize.argtypes = [vp]
+    L.fs_set_directivity_patterns.argtypes = [vp, vp, u32]
+    L.fs_set_source_directivity.argtypes = [vp, vp, u32]
+    L.fs_directivity_polar.argtypes = [vp, vp, u32, vp]
+    L.fs_multi_set_directivity_patterns.argtypes = [vp, vp, u32]
+    L.fs_multi_set_source_directivity.argtypes = [vp, vp, u32]
     for n in ABI_SYMBOLS:
         if n not in ("fs_default_config", "fs_destroy", "fs_last_error", "fs_multi_destroy", "fs_multi_last_error",
                      "fs_multi_device_count", "fs_multi_context"):
@@ -481,6 +518,18 @@ class Context:
         self._ck(self.L.fs_get_histogram(self.h, hist.ctypes.data))
         return hist
 
+    # -- directional sources --
+    def set_directivity_patterns(self, gains):
+        """fs_set_directivity_patterns: energy gains [P][B][33] at cos = -1 + i/16 (B <= 8); replaces the table and clears the
+        source orientations"""
+        full = _patterns(gains)
+        self._ck(self.L.fs_set_directivity_patterns(self.h, full.ctypes.data, len(full)))
+
+    def set_source_directivity(self, forward, pattern):
+        """fs_set_source_directivity: forward axes [S][3] and pattern indices [S] (OMNI: omni); S = 0 (forward = []) clears"""
+        arr, S = _orients(forward, pattern)
+        self._ck(self.L.fs_set_source_directivity(self.h, arr, S))
+
     def noise_stats(self):
         """fs_get_noise: per-source noise of the last update as a dict of numpy arrays -- n_paths [S], no_energy [S] bool,
         signal / variance / snr_db [S] (broadband) and band_signal / band_variance / band_snr_db [S][B]"""
@@ -657,6 +706,16 @@ class MultiContext:
                                                hist.ctypes.data if want_hist else None))
         return hist
 
+    def set_directivity_patterns(self, gains):
+        """fs_multi_set_directivity_patterns: Context.set_directivity_patterns on every device"""
+        full = _patterns(gains)
+        self._ck(self.L.fs_multi_set_directivity_patterns(self.h, full.ctypes.data, len(full)))
+
+    def set_source_directivity(self, forward, pattern):
+        """fs_multi_set_source_directivity: Context.set_source_directivity on every device"""
+        arr, S = _orients(forward, pattern)
+        self._ck(self.L.fs_multi_set_source_directivity(self.h, arr, S))
+
     def last_ms(self):
         a, b = C.c_float(), C.c_float()
         self._ck(self.L.fs_multi_last_ms(self.h, C.byref(a), C.byref(b)))
@@ -690,6 +749,17 @@ def allocate_paths(stats, total, min_paths, max_paths, weight=None):
     if rc != FS_OK:
         raise FrequenSeeError(rc, "fs_allocate_paths: invalid argument")
     return out
+
+
+def directivity_polar(dipole_weight, power):
+    """fs_directivity_polar: energy gains [B][33] of |(1 - w_b) + w_b c| ^ p_b at c = -1 + i/16 (B = len(w)); host only"""
+    w = np.ascontiguousarray(np.atleast_1d(dipole_weight), dtype=np.float32)
+    p = np.ascontiguousarray(np.broadcast_to(np.asarray(power, np.float32), w.shape))
+    out = np.zeros((MAX_BANDS, DIR_POINTS), np.float32)
+    rc = load().fs_directivity_polar(w.ctypes.data, p.ctypes.data, len(w), out.ctypes.data)
+    if rc != FS_OK:
+        raise FrequenSeeError(rc, "fs_directivity_polar: invalid argument")
+    return out[:len(w)]
 
 
 def load_float_array(path):

@@ -339,6 +339,52 @@ int fs_get_histogram_m2(fs_ctx* ctx, uint64_t* out);
 int fs_allocate_paths(const fs_noise_stats* st, uint32_t n_sources, uint64_t total, uint64_t min_paths, uint64_t max_paths,
                       const float* weight, uint64_t* n_out);
 
+/* ---- directional sources ----------------------------------------------------------------------
+ * EXTENDS the reference: its emitters radiate the same energy in every direction (node 0 of the source subpath samples a
+ * uniform sphere, VRand at SUB.cpp:306-311, and EvaluatePath starts every path at Energy = 1, SUB.cpp:367).  A directional
+ * source weights each connected path by a per-band energy gain of the direction in which the path LEAVES the source; the
+ * walk, its random numbers and the estimator are unchanged (the histogram of an omni source is bit-identical).
+ *
+ * Pattern: gain[b][i] = energy gain of band b at cos = -1 + i/16 between the emission direction d and the source's
+ * forward axis f (finite, >= 0; bands >= n_bands are ignored).  The factor of band b is
+ *     c = clamp(dot(d, f), -1, 1),  x = (c + 1) 16,  i = min(floor(x), 31),  t = x - i,  g_b = T[i] + t (T[i+1] - T[i])
+ * (dot as fmaf(d.z, f.z, fmaf(d.y, f.y, d.x f.x)); a constant table of 1.0 gives exactly 1.0).
+ * Emission direction d of a connected path of source s:
+ *   endpoint mode (default) and FS_FLAG_CONNECT_ALL: the source prefix has >= 2 nodes -> the bounce-0 direction of the source
+ *     subpath (the uniform-sphere sample of Philox block (g, bounce 0, side 0), regenerated, not stored); 1 node -> the
+ *     connection vector times 1 / its length (the direction of the connection ray);
+ *   FS_FLAG_MIS: normalize(x1 - x0) of the path's first two vertices (the contribution f is a function of the vertices, so
+ *     every strategy that builds the same path gets the same factor).
+ * The factor multiplies the band's energy before the clamp and gain (EvaluatePath starts at g_b instead of 1; with
+ * FS_FLAG_MIS the product that forms f starts at g_b); a source with pattern FS_OMNI is not multiplied.  fs_path_dbg.energy
+ * includes it; FS_FLAG_NOISE_STATS moments are those of the weighted values.
+ * State: both set calls copy at call time and retain nothing; the uploads are stream-ordered on the context stream (a trace
+ * already enqueued uses the table installed before it).  fs_set_directivity_patterns (1..256 patterns) replaces the table
+ * and clears the orientations.  fs_set_source_directivity installs one orientation per source (n_sources = 0 clears: all
+ * omni); FS_ERR_INVALID for a pattern index >= n_patterns other than FS_OMNI, a zero or non-finite forward, or
+ * any index other than FS_OMNI when no pattern table is installed (a rejected call changes nothing).  While orientations
+ * are installed every trace entry point (fs_trace, fs_update, fs_trace_range*, fs_trace_debug, fs_trace_sources*,
+ * fs_update_sources, fs_multi_trace*) returns FS_ERR_INVALID, before anything is enqueued, if its n_sources differs from
+ * the installed count. */
+#define FS_DIR_POINTS 33
+typedef struct fs_directivity {
+    float gain[FS_MAX_BANDS][FS_DIR_POINTS];   /* energy gain at cos = -1 + i/16; finite, >= 0; bands >= n_bands ignored */
+} fs_directivity;                               /* 1056 bytes */
+
+#define FS_OMNI 0xffffffffu
+typedef struct fs_source_orient {
+    float    forward[3];   /* any non-zero finite vector; normalised on the host (double, rounded to float) */
+    uint32_t pattern;      /* index into the installed pattern table, or FS_OMNI */
+} fs_source_orient;        /* 16 bytes */
+
+int fs_set_directivity_patterns(fs_ctx* ctx, const fs_directivity* patterns, uint32_t n_patterns);  /* 1..256; replaces the table */
+int fs_set_source_directivity(fs_ctx* ctx, const fs_source_orient* o, uint32_t n_sources);          /* 0 = clear (all omni) */
+/* host only, no context: gain_b(c) = |(1 - w_b) + w_b c| ^ p_b at the 33 points (w = 0: omni, w = 0.5: cardioid, w = 1:
+ * figure of eight; p = 1 for a pressure-squared pattern of that first-order shape), computed in double and rounded to float;
+ * bands >= n_bands are 0.  FS_ERR_INVALID for n_bands outside 1..8, a weight outside [0,1], a power outside [0,64] or a
+ * non-finite input */
+int fs_directivity_polar(const float* dipole_weight, const float* power, uint32_t n_bands, fs_directivity* out);
+
 /* single rays through the device BVH (parity tests of the intersector):
  * rays: [n][6] (origin, direction); out_t [n] (inf on miss), out_tri [n] (0xffffffff on miss) */
 int fs_debug_closest_hits(fs_ctx* ctx, const float* rays, uint64_t n, float* out_t, uint32_t* out_tri);
@@ -444,6 +490,10 @@ int fs_multi_trace(fs_multi* m, const float* src_pos, uint32_t n_sources, const 
  * reduced histogram and the per-source path counts */
 int fs_multi_trace_sources(fs_multi* m, const fs_source_desc* src, uint32_t n_sources, const float lis_pos[3], uint64_t seed,
                            uint64_t* hist_out);
+/* fs_set_directivity_patterns / fs_set_source_directivity on every device (the shards of fs_multi_trace* must weight their
+ * paths alike) */
+int fs_multi_set_directivity_patterns(fs_multi* m, const fs_directivity* patterns, uint32_t n_patterns);
+int fs_multi_set_source_directivity(fs_multi* m, const fs_source_orient* o, uint32_t n_sources);
 /* device time of the last fs_multi_trace (CUDA events on device 0's stream): the whole update, and the part after device
  * 0's own shard was done (waiting for the peers' stores + the sum).  Synchronises. */
 int fs_multi_last_ms(fs_multi* m, float* total_ms, float* reduce_ms);

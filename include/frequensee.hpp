@@ -79,6 +79,10 @@ public:
     float NoiseWeight = 1.0f;
     // FS_FLAG_NOISE_STATS: the noise of this source in the last UpdateSources() (fs_get_noise; n_paths = the budget it had)
     fs_noise_stats LastNoise{};
+    // directional source: the owner's forward axis (GetActorForwardVector(); a direction, so no cm -> m conversion) and an
+    // index into the patterns of UAudioRayTracingSubsystem::SetDirectivityPatterns, or FS_OMNI (radiates alike everywhere)
+    FVector3f Forward{1.f, 0.f, 0.f};
+    uint32_t DirectivityPattern = FS_OMNI;
 
     std::vector<float> EnergyBuffer;   // COMP.h:70
     void FlushEnergyBuffer() { EnergyBuffer.assign(NumBins, 0.0f); bUseDeviceHistogram = false; }          // COMP.h:76-79
@@ -188,6 +192,12 @@ public:
     }
     void SetPlayerPawnLocation(FVector3f L) { PawnLocation = L; }                                              // SUB.cpp:70-80
     uint64_t Seed = 0x5EED;
+    // the polar patterns components name by DirectivityPattern (fs_set_directivity_patterns; replaces the table)
+    bool SetDirectivityPatterns(const std::vector<fs_directivity>& Patterns)
+    {
+        bDirInstalled = false;
+        return Ctx->Check(fs_set_directivity_patterns(Ctx->Get(), Patterns.data(), (uint32_t)Patterns.size())) == FS_OK;
+    }
 
     // UpdateSource (SUB.cpp:128-195): GenerateFullPaths + EvaluatePath + Flush + AddEnergyAtDelay (on the
     // device, integer) + ReconstructImpulseResponse.  FIX: no second flush before the IR (SUB.cpp:191).
@@ -197,6 +207,8 @@ public:
         const FVector3f S = Src.GetActorLocation();
         const float src[3] = {S.X, S.Y, S.Z}, lis[3] = {PawnLocation.X, PawnLocation.Y, PawnLocation.Z};
         // one source per call: the device histogram of source slot 0 belongs to Src until the next update
+        UFrequenSeeAudioComponent* One[1] = {&Src};
+        if (!InstallOrientations(One, 1)) return;
         if (Ctx->Check(fs_trace(Ctx->Get(), src, 1, lis, (uint64_t)Src.RaycastsPerTick, (uint32_t)Src.RaycastBounces,
                                 Seed++, nullptr)) != FS_OK) return;
         fs_stats st;
@@ -241,6 +253,7 @@ public:
             desc[s].n_paths = budget[s];
         }
         NoiseSources.clear();
+        if (!InstallOrientations(ActiveSources.data(), S)) return;
         if (Ctx->Check(fs_trace_sources(Ctx->Get(), desc.data(), S, lis, Seed++, nullptr)) != FS_OK) return;
         fs_stats st;
         if (fs_get_stats(Ctx->Get(), &st) == FS_OK) LastConnected = st.connected;
@@ -262,6 +275,25 @@ public:
     uint64_t LastConnected = 0;
 
 private:
+    // the orientations of the sources a trace is about to trace (slot s = Src[s]), or none when every one is omni
+    bool InstallOrientations(UFrequenSeeAudioComponent* const* Src, uint32_t S)
+    {
+        bool any = false;
+        for (uint32_t s = 0; s < S; ++s) any = any || Src[s]->DirectivityPattern != FS_OMNI;
+        if (!any) {
+            if (bDirInstalled && Ctx->Check(fs_set_source_directivity(Ctx->Get(), nullptr, 0)) != FS_OK) return false;
+            bDirInstalled = false;
+            return true;
+        }
+        std::vector<fs_source_orient> o(S);
+        for (uint32_t s = 0; s < S; ++s) {
+            o[s].forward[0] = Src[s]->Forward.X; o[s].forward[1] = Src[s]->Forward.Y; o[s].forward[2] = Src[s]->Forward.Z;
+            o[s].pattern = Src[s]->DirectivityPattern;
+        }
+        bDirInstalled = Ctx->Check(fs_set_source_directivity(Ctx->Get(), o.data(), S)) == FS_OK;
+        return bDirInstalled;
+    }
+    bool bDirInstalled = false;        // orientations are installed on the context
     // TotalRaysPerTick over the active sources: equally, or by fs_allocate_paths from the last update's noise when it
     // belongs to the same sources
     bool SplitTotal(std::vector<uint64_t>& budget)
