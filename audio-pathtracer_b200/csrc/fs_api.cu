@@ -200,6 +200,7 @@ void fs_destroy(fs_ctx* ctx)
     cudaFree(ctx->d_verts); cudaFree(ctx->d_tri_mat); cudaFree(ctx->d_refl_over_pi);
     cudaFree(ctx->d_hist); cudaFree(ctx->d_m2); cudaFree(ctx->d_noise); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
     cudaFree(ctx->d_dir_gain); cudaFree(ctx->d_dir_orient);
+    cudaFree(ctx->d_occl_tau); cudaFree(ctx->d_occl);
     cudaFree(ctx->d_amp); cudaFree(ctx->d_energy);
     for (cudaEvent_t e : ctx->kev) cudaEventDestroy(e);
     for (cudaEvent_t e : ctx->tev) cudaEventDestroy(e);
@@ -353,6 +354,39 @@ int fs_scene_set_materials_ex(fs_ctx* ctx, const float* absorption, const float*
     return FS_OK;
 }
 
+// Transmitted factor of one (material, band) of the material asset, for the material model and for fs_occlusion: tau is
+// limited so that Refl + tau <= 1 (MaterialAcousticProcessor.cpp:59-60; limited in place, the lobe thresholds use it) and
+// raised to ThicknessCm / 2.5 (ex), a Beer-Lambert layer with the asset's default 2.5 cm as the reference thickness.
+static float transmitted_factor(float absorption, float& tau, float ex)
+{
+    const float refl = 1.0f - absorption;
+    if (refl + tau > 1.0f) tau = 1.0f - refl;
+    if (!(tau > 0.0f)) return 0.0f;
+    return (ex == 1.0f) ? tau : fs_pow(tau, ex);
+}
+
+// fs_occlusion's table tau_eff [M][B], for every context (with or without FS_FLAG_MATERIAL_MODEL); materials set without
+// Transmission have tau = 0: their surfaces block
+static int build_occlusion_table(fs_ctx* ctx)
+{
+    const uint32_t M = ctx->n_mats, B = ctx->cfg.n_bands;
+    std::vector<float> tab((size_t)M * B);
+    const float* tr = ctx->mat_transmission.empty() ? nullptr : ctx->mat_transmission.data();
+    const float* th = ctx->mat_thickness_cm.empty() ? nullptr : ctx->mat_thickness_cm.data();
+    for (uint32_t m = 0; m < M; ++m) {
+        const float ex = (th ? th[m] : 2.5f) / 2.5f;
+        for (uint32_t b = 0; b < B; ++b) {
+            float tau = tr ? tr[(size_t)m * B + b] : 0.0f;
+            tab[(size_t)m * B + b] = transmitted_factor(ctx->mat_absorption[(size_t)m * B + b], tau, ex);
+        }
+    }
+    cudaFree(ctx->d_occl_tau); ctx->d_occl_tau = nullptr;
+    CK(cudaMalloc(&ctx->d_occl_tau, sizeof(float) * tab.size()));
+    CK(cudaMemcpyAsync(ctx->d_occl_tau, tab.data(), sizeof(float) * tab.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return FS_OK;
+}
+
 // FS_FLAG_MATERIAL_MODEL (SURVEY 8f rank 3): per (event, material, band) energy factors and per material lobe thresholds.
 // Plain float arithmetic in a fixed order that the CPU harness restates (the tables must be
 // bit-identical on both sides); fs_pow is the shared polynomial of fs_math.cuh.
@@ -372,10 +406,8 @@ static int build_material_model(fs_ctx* ctx)
             const float a = ctx->mat_absorption[(size_t)m * B + b];
             const float refl = 1.0f - a;
             float tau = tr ? tr[(size_t)m * B + b] : 0.0f;
-            if (refl + tau > 1.0f) tau = 1.0f - refl;                      // MaterialAcousticProcessor.cpp:59-60
+            const float tau_eff = transmitted_factor(a, tau, ex);
             const float sig = sc ? sc[(size_t)m * B + b] : 1.0f;
-            float tau_eff = 0.0f;
-            if (tau > 0.0f) tau_eff = (ex == 1.0f) ? tau : fs_pow(tau, ex);
             tab[((size_t)0 * M + m) * B + b] = (refl * sig) / FS_PI;
             tab[((size_t)1 * M + m) * B + b] = refl * (1.0f - sig);
             tab[((size_t)2 * M + m) * B + b] = tau_eff;
@@ -416,6 +448,7 @@ int fs_scene_commit(fs_ctx* ctx)
         int rc = build_material_model(ctx);
         if (rc) return rc;
     }
+    if (int rc = build_occlusion_table(ctx)) return rc;
     uint64_t bvh_launches = 0;
     CK(fs_bvh_build(ctx->stream, ctx->d_verts, ctx->d_tri_mat, ctx->n_tris, &ctx->bvh, &bvh_launches,
                     ctx->tune.leaf_max, ctx->tune.builder, ctx->tune.collapse | (ctx->tune.w8 ? 4u : 0u)));
@@ -1521,6 +1554,74 @@ int fs_directivity_polar(const float* dipole_weight, const float* power, uint32_
             const double c = -1.0 + i / 16.0, w = dipole_weight[b];
             out->gain[b][i] = (float)pow(fabs((1.0 - w) + w * c), (double)power[b]);
         }
+    return FS_OK;
+}
+
+// ---- direct-path occlusion ------------------------------------------------------------------------
+int fs_occlusion(fs_ctx* ctx, const fs_occlusion_source* src, uint32_t n_sources, const float lis_pos[3], uint32_t max_crossings,
+                 uint64_t seed, fs_occlusion_result* out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!ctx->committed) return fail(ctx, FS_ERR_STATE, "fs_occlusion: call fs_scene_commit first");
+    if (ctx->verts_dirty) return fail(ctx, FS_ERR_STATE, "fs_occlusion: triangles were moved; call fs_scene_refit (or fs_scene_commit) first");
+    if (!src || !lis_pos || !out) return fail(ctx, FS_ERR_INVALID, "fs_occlusion: null argument");
+    if (n_sources == 0 || n_sources > FS_MAX_SOURCES) return fail(ctx, FS_ERR_INVALID, "fs_occlusion: n_sources must be 1..4096");
+    if (max_crossings > 16) return fail(ctx, FS_ERR_INVALID, "fs_occlusion: max_crossings must be 0..16");
+    auto bad_pos = [](const float* p) {
+        for (int a = 0; a < 3; ++a) if (!std::isfinite(p[a]) || fabsf(p[a]) > 1e18f) return true;
+        return false;
+    };
+    if (bad_pos(lis_pos)) return fail(ctx, FS_ERR_INVALID, "fs_occlusion: non-finite or > 1e18 listener position");
+    const uint32_t S = n_sources, B = ctx->cfg.n_bands, W = B + 1u;
+    // host staging of the upload: [S] float4 (centre, radius), then [S+1] u32 ray offsets
+    std::vector<float4> hsrc(S + (S + 1u + 3u) / 4u);
+    uint32_t* off = (uint32_t*)(hsrc.data() + S);
+    uint32_t n_rays = 0;
+    for (uint32_t s = 0; s < S; ++s) {
+        const fs_occlusion_source& d = src[s];
+        const std::string who = "fs_occlusion: source " + std::to_string(s);
+        if (bad_pos(d.pos)) return fail(ctx, FS_ERR_INVALID, (who + ": non-finite or > 1e18 position").c_str());
+        if (!(d.radius >= 0.0f) || !std::isfinite(d.radius)) return fail(ctx, FS_ERR_INVALID, (who + ": radius must be finite and >= 0").c_str());
+        if (d.radius > 0.0f && (d.n_rays == 0 || d.n_rays > 65536u)) return fail(ctx, FS_ERR_INVALID, (who + ": n_rays must be 1..65536").c_str());
+        if (d.reserved) return fail(ctx, FS_ERR_INVALID, (who + ": reserved field must be 0").c_str());
+        hsrc[s] = make_float4(d.pos[0], d.pos[1], d.pos[2], d.radius);
+        off[s] = n_rays;
+        n_rays += d.radius > 0.0f ? d.n_rays : 1u;
+    }
+    off[S] = n_rays;
+    dev_guard g(ctx->device);
+    // device scratch: [S][B+1] u64 sums, one u64 slot for the overflow flag, then the staged sources and offsets
+    const size_t acc_bytes = (8ull * S * W + 8ull + 15ull) & ~15ull, up_bytes = sizeof(float4) * hsrc.size();
+    if (ctx->occl_cap < acc_bytes + up_bytes) {
+        cudaFree(ctx->d_occl); ctx->d_occl = nullptr; ctx->occl_cap = 0;
+        const size_t cap = 8ull * FS_MAX_SOURCES * (FS_MAX_BANDS + 1) + 16ull + sizeof(float4) * (FS_MAX_SOURCES + 1026);   // 0.35 MB: the largest call
+        CK(cudaMalloc(&ctx->d_occl, cap));
+        ctx->occl_cap = (uint32_t)cap;
+    }
+    unsigned long long* d_acc = (unsigned long long*)ctx->d_occl;
+    uint32_t* d_overflow = (uint32_t*)(d_acc + (size_t)S * W);
+    float4* d_src = (float4*)((char*)ctx->d_occl + acc_bytes);
+    fs_trace_params tp;
+    fill_params(ctx, &tp, nullptr, 1, 1, 0);
+    std::vector<unsigned long long> h(acc_bytes / 8u);
+    CK(cudaMemcpyAsync(d_src, hsrc.data(), up_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(d_acc, 0, acc_bytes, ctx->stream));
+    CK(fs_occlusion_run(tp.bv, d_src, (const uint32_t*)(d_src + S), S, n_rays, lis_pos, ctx->d_occl_tau, B, max_crossings,
+                        ctx->cfg.eps_connect, ctx->cfg.eps_offset, seed, d_acc, d_overflow, ctx->stream));
+    ctx->launches.fetch_add(1);
+    CK(cudaMemcpyAsync(h.data(), d_acc, acc_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    for (uint32_t s = 0; s < S; ++s) {
+        const double n = (double)(off[s + 1] - off[s]);
+        const unsigned long long* r = h.data() + (size_t)s * W;
+        fs_occlusion_result& o = out[s];
+        memset(&o, 0, sizeof(o));
+        o.visible = (float)((double)r[B] / n);
+        for (uint32_t b = 0; b < B; ++b) o.transmission[b] = (float)((double)r[b] * 0x1p-32 / n);
+        o.n_rays = off[s + 1] - off[s];
+    }
+    if ((uint32_t)h[(size_t)S * W])
+        return fail(ctx, FS_ERR_OVERFLOW, "fs_occlusion: BVH traversal stack overflow (tree deeper than FS_STACK_SIZE): the results are invalid");
     return FS_OK;
 }
 

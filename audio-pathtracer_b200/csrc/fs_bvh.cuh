@@ -258,4 +258,52 @@ __device__ __forceinline__ bool fs_any_hit(const fs_bvh_view& bv, const float4* 
     return false;
 }
 
+// Every hit with 0 < t < tmax (fs_occlusion): the walk of fs_any_hit without the early exit, over the BVH2 `nodes`, which
+// every node format keeps and whose leaves address `tris` (the 8-wide format copies the records into tris8).
+// on_hit(t, original id, material) is called once per hit in traversal order; the walk stops when it returns false.
+template <class F>
+__device__ __forceinline__ void fs_all_hits(const fs_bvh_view& bv, fs_vec3 o, fs_vec3 d, float tmax, F&& on_hit,
+                                            uint32_t* overflow)
+{
+    if (bv.n_tris == 0) return;
+    const fs_ray_prep r = fs_prep_ray(o, d);
+    int stack[FS_STACK_SIZE];
+    int sp = 0;
+    const int SENTINEL = 0x7fffffff;
+    int node = 0;
+    FS_GUARD_DECL
+    while (node != SENTINEL) {
+        while (node >= 0 && node != SENTINEL) {
+            FS_GUARD_STEP
+            const float4* p = bv.nodes + (size_t)node * 4;
+            const float4 n0 = fs_ldg4(p), n1 = fs_ldg4(p + 1), n2 = fs_ldg4(p + 2), n3 = fs_ldg4(p + 3);
+            bool h0, h1; float t0, t1;
+            fs_slab2(r, n0, n1, n2, tmax, h0, h1, t0, t1);
+            int c0 = __float_as_int(n3.x), c1 = __float_as_int(n3.y);
+            if (!h0 && !h1) {
+                node = sp ? stack[--sp] : SENTINEL;
+            } else {
+                node = h0 ? c0 : c1;
+                if (h0 && h1) {
+                    if (sp < FS_STACK_SIZE) stack[sp++] = c1; else *overflow = 1u;
+                }
+            }
+        }
+        while (node < 0) {
+            uint32_t payload = (uint32_t)(~node);
+            uint32_t first = payload >> 3, count = (payload & 7u) + 1u;
+            for (uint32_t i = 0; i < count; ++i) {
+                const float4* tp = bv.tris + (size_t)(first + i) * 4;
+                const float4 a = fs_ldg4(tp), b = fs_ldg4(tp + 1), c = fs_ldg4(tp + 2);
+                float t;
+                if (fs_intersect_tri(o, d, fs_mk(a.x, a.y, a.z), fs_mk(b.x, b.y, b.z), fs_mk(c.x, c.y, c.z), t) && t < tmax) {
+                    const float4 e = fs_ldg4(tp + 3);
+                    if (!on_hit(t, __float_as_uint(e.x), __float_as_uint(e.y))) return;
+                }
+            }
+            node = sp ? stack[--sp] : SENTINEL;
+        }
+    }
+}
+
 #endif  // __CUDACC__

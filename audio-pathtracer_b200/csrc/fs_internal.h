@@ -222,6 +222,10 @@ struct fs_ctx {
     // (float4: unit forward, bits(pattern)); dir_sources = 0: none installed, every source omni
     float* d_dir_gain; uint32_t dir_patterns;
     float4* d_dir_orient; uint32_t dir_sources, dir_orient_cap;
+    // fs_occlusion: transmitted factor tau_eff [M][B] of every material (built by every fs_scene_commit), and the scratch of
+    // one call: [S][B+1] u64 sums, the call's own overflow flag (one u64 slot), [S] float4 sources, [S+1] u32 ray offsets
+    float* d_occl_tau;
+    void* d_occl; uint32_t occl_cap;
     fs_dev_counters* d_counters;
     // traversal-stack overflow of the last trace: one 4-byte async copy into pinned memory after every fs_trace*, looked at
     // by the next call that can (sticky until reported)
@@ -266,6 +270,11 @@ cudaError_t fs_wave_trace_batch(fs_ctx* ctx, fs_lane* lane, const fs_trace_param
 cudaError_t fs_wave_reset_counters(fs_ctx* ctx, int reset_overflow);
 cudaError_t fs_wave_debug_rays(fs_ctx* ctx, const fs_trace_params& tp, const float* d_rays, const float* d_tmax,
                                uint64_t n, float* d_t, uint32_t* d_tri, uint8_t* d_hit);
+
+// fs_occlusion.cu: k_occlusion over n_rays = d_off[n_src] flat rays; d_acc [n_src][n_bands+1] must be zeroed
+cudaError_t fs_occlusion_run(const fs_bvh_view& bv, const float4* d_src, const uint32_t* d_off, uint32_t n_src, uint32_t n_rays,
+                             const float lis[3], const float* d_tau, uint32_t n_bands, uint32_t max_crossings, float eps_connect,
+                             float eps_offset, uint64_t seed, unsigned long long* d_acc, uint32_t* d_overflow, cudaStream_t st);
 
 // fs_ir.cu
 struct fs_scale_table { double v[FS_PTR_TABLE]; };   // per-source 1 / n_paths, passed by value

@@ -46,6 +46,7 @@ ABI_SYMBOLS = [
     "fs_multi_trace", "fs_multi_trace_sources", "fs_multi_last_ms", "fs_multi_synchronize",
     "fs_set_directivity_patterns", "fs_set_source_directivity", "fs_directivity_polar",
     "fs_multi_set_directivity_patterns", "fs_multi_set_source_directivity",
+    "fs_occlusion",
 ]
 
 
@@ -193,6 +194,30 @@ def noise_stats_array(d):
     return arr
 
 
+class OcclusionSource(C.Structure):
+    """fs_occlusion_source: one emitter of a direct-path occlusion query (radius 0 = a point: one ray)"""
+    _fields_ = [("pos", C.c_float * 3), ("radius", C.c_float), ("n_rays", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class OcclusionResult(C.Structure):
+    """fs_occlusion_result: visible fraction and mean per-band transmitted gain of one emitter's sample rays"""
+    _fields_ = [("visible", C.c_float), ("transmission", C.c_float * MAX_BANDS), ("n_rays", C.c_uint32),
+                ("reserved", C.c_uint32)]
+
+
+def occlusion_sources(src_pos, radius, n_rays):
+    """fs_occlusion_source[S] from centres [S][3], radii [S] and ray counts [S] (scalars broadcast)"""
+    src = np.ascontiguousarray(src_pos, dtype=np.float32).reshape(-1, 3)
+    r = np.broadcast_to(np.asarray(radius, dtype=np.float32), (len(src),))
+    n = np.broadcast_to(np.asarray(n_rays, dtype=np.uint64), (len(src),))
+    arr = (OcclusionSource * max(len(src), 1))()
+    for s in range(len(src)):
+        arr[s].pos[:] = [float(v) for v in src[s]]
+        arr[s].radius = float(r[s])
+        arr[s].n_rays = int(n[s])
+    return arr, len(src)
+
+
 class FrequenSeeError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__("frequensee error %d: %s" % (code, msg))
@@ -287,6 +312,7 @@ def load():
     L.fs_directivity_polar.argtypes = [vp, vp, u32, vp]
     L.fs_multi_set_directivity_patterns.argtypes = [vp, vp, u32]
     L.fs_multi_set_source_directivity.argtypes = [vp, vp, u32]
+    L.fs_occlusion.argtypes = [vp, vp, u32, vp, u32, u64, vp]
     for n in ABI_SYMBOLS:
         if n not in ("fs_default_config", "fs_destroy", "fs_last_error", "fs_multi_destroy", "fs_multi_last_error",
                      "fs_multi_device_count", "fs_multi_context"):
@@ -529,6 +555,18 @@ class Context:
         """fs_set_source_directivity: forward axes [S][3] and pattern indices [S] (OMNI: omni); S = 0 (forward = []) clears"""
         arr, S = _orients(forward, pattern)
         self._ck(self.L.fs_set_source_directivity(self.h, arr, S))
+
+    def occlusion(self, src_pos, radius, n_rays, lis_pos, max_crossings=4, seed=0):
+        """fs_occlusion: direct-path occlusion of every emitter (centres [S][3], radii [S], ray counts [S]; scalars
+        broadcast).  Returns (visible [S] float32, transmission [S][B] float32)"""
+        arr, S = occlusion_sources(src_pos, radius, n_rays)
+        lis = np.ascontiguousarray(lis_pos, dtype=np.float32).reshape(3)
+        out = (OcclusionResult * max(S, 1))()
+        self._ck(self.L.fs_occlusion(self.h, arr, S, lis.ctypes.data, max_crossings, seed, out))
+        B = self.cfg.n_bands
+        vis = np.array([out[s].visible for s in range(S)], np.float32)
+        tr = np.array([list(out[s].transmission)[:B] for s in range(S)], np.float32).reshape(S, B)
+        return vis, tr
 
     def noise_stats(self):
         """fs_get_noise: per-source noise of the last update as a dict of numpy arrays -- n_paths [S], no_energy [S] bool,

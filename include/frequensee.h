@@ -385,6 +385,55 @@ int fs_set_source_directivity(fs_ctx* ctx, const fs_source_orient* o, uint32_t n
  * non-finite input */
 int fs_directivity_polar(const float* dipole_weight, const float* power, uint32_t n_bands, fs_directivity* out);
 
+/* ---- direct-path occlusion and transmission -------------------------------------------------------
+ * replaces: OcclusionAttenuation of the legacy per-frame tracer's CastDirectAudioRay (COMP.cpp:209-280, stored at :297-299: a
+ * direct ray that passes through up to RaycastBounces occluders, whose result nothing reads) and the value the registered
+ * occlusion plugin is given and ignores (OCC.cpp:46-49).  Answers, per emitter: how much of it reaches the listener straight
+ * through the geometry, per band -- what the host's dry path (its attenuation and occlusion plugin) needs.
+ * For source s with n rays (n = 1 when radius = 0):
+ *   sample points: q_0 = the centre exactly; q_j (j >= 1) = centre + rho sample_sphere(u1, u2), rho = radius u3^(1/3) (0 when
+ *     u3 = 0), u1..u3 = the first three words of Philox4x32-10 block (key seed, counter (j, s, 0, 'OCCL')) as 24-bit uniforms:
+ *     uniform in the ball.
+ *   ray j: built like the endpoint connection ray of the trace, from q_j to the listener: dl = lis - q, len = |dl|,
+ *     tmax = len - eps_connect; tmax <= 0 -> visible with gain 1, nothing traced; else direction dl (1 / len).  So for a point
+ *     emitter `visible` is the visibility of the direct (1,1) connection of the trace.
+ *   crossings: every triangle hit with t < tmax, ordered by (t, original triangle id); a hit of the same material as the last
+ *     counted crossing and less than eps_offset further along is that crossing again (a shared edge or vertex of a
+ *     tessellated wall counts once).  At most 32 raw hits are kept: a ray with more is blocked (gain 0, not visible).
+ *   per ray, k counted crossings: visible_j = (k == 0); gain_jb = 0 if k > max_crossings, else the float product, in
+ *     crossing order from 1.0f, of tau_eff[m][b] of the crossed materials.  max_crossings plays the part of the legacy ray's
+ *     RaycastBounces; with 0 the query is pure occlusion (transmission == visible).
+ *   tau_eff[m][b] = the material model's transmitted factor (Transmission limited to 1 - Refl, raised to ThicknessCm / 2.5),
+ *     built at fs_scene_commit for every context, with or without FS_FLAG_MATERIAL_MODEL.  Materials set with
+ *     fs_scene_set_materials have tau = 0: their surfaces block.
+ *   result: visible = (visible rays) / n in double, rounded to float; transmission[b] = (sum_j trunc(gain_jb 2^32)) 2^-32 / n,
+ *     the sum exact in 64-bit integers and the division in double, so the value does not depend on ray order or the tree.
+ * State and errors, all checked before anything is enqueued (a rejected call changes nothing): FS_ERR_STATE before
+ * fs_scene_commit or while moved vertices await fs_scene_refit; FS_ERR_INVALID for NULL pointers, n_sources 0 or > 4096, a
+ * non-finite or > 1e18 position, a negative or non-finite radius, n_rays 0 or > 65536 with radius > 0, max_crossings > 16,
+ * a non-zero reserved field.  FS_ERR_OVERFLOW: the traversal stack overflowed and the results are invalid; reported by this
+ * call from a flag of its own (the trace's sticky flag is neither set nor cleared).
+ * Runs on the context stream after the work already enqueued there and synchronises.  Reads and writes nothing of the
+ * histogram, the noise moments, the IRs, the convolver, the directivity state or fs_stats (except kernel_launches);
+ * directivity does not weight it (a transmitted fraction, not an energy).
+ * Several GPUs: the scene of an fs_multi is replicated, so call fs_occlusion(fs_multi_context(m, 0), ...). */
+typedef struct fs_occlusion_source {
+    float    pos[3];        /* emitter centre, metres */
+    float    radius;        /* >= 0; 0 = point emitter: one ray, n_rays ignored */
+    uint32_t n_rays;        /* 1..65536 sample rays when radius > 0 */
+    uint32_t reserved;      /* 0 */
+} fs_occlusion_source;      /* 24 bytes */
+
+typedef struct fs_occlusion_result {
+    float    visible;                       /* fraction of sample rays that cross no surface */
+    float    transmission[FS_MAX_BANDS];    /* mean per-band gain of the rays (visible rays count 1); bands >= n_bands: 0 */
+    uint32_t n_rays;                        /* rays actually used (1 for radius 0) */
+    uint32_t reserved;
+} fs_occlusion_result;      /* 44 bytes */
+
+int fs_occlusion(fs_ctx* ctx, const fs_occlusion_source* src, uint32_t n_sources, const float lis_pos[3],
+                 uint32_t max_crossings /* 0..16 */, uint64_t seed, fs_occlusion_result* out /* [n_sources] */);
+
 /* single rays through the device BVH (parity tests of the intersector):
  * rays: [n][6] (origin, direction); out_t [n] (inf on miss), out_tri [n] (0xffffffff on miss) */
 int fs_debug_closest_hits(fs_ctx* ctx, const float* rays, uint64_t n, float* out_t, uint32_t* out_tri);

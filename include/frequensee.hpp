@@ -83,6 +83,12 @@ public:
     // index into the patterns of UAudioRayTracingSubsystem::SetDirectivityPatterns, or FS_OMNI (radiates alike everywhere)
     FVector3f Forward{1.f, 0.f, 0.f};
     uint32_t DirectivityPattern = FS_OMNI;
+    // direct-path occlusion (UAudioRayTracingSubsystem::UpdateOcclusion, fs_occlusion): the emitter as a ball of this radius
+    // in metres (0 = a point, one ray) sampled by OcclusionRays rays, and the result of the last query -- visible fraction and
+    // per-band transmission, what the host's occlusion plugin turns into the dry sound's volume and low-pass
+    float OcclusionRadius = 0.0f;
+    uint32_t OcclusionRays = 64;
+    fs_occlusion_result LastOcclusion{};
 
     std::vector<float> EnergyBuffer;   // COMP.h:70
     void FlushEnergyBuffer() { EnergyBuffer.assign(NumBins, 0.0f); bUseDeviceHistogram = false; }          // COMP.h:76-79
@@ -273,6 +279,30 @@ public:
         }
     }
     uint64_t LastConnected = 0;
+
+    // Direct-path occlusion of every active source in ONE fs_occlusion call (the OcclusionAttenuation the legacy tracer's
+    // CastDirectAudioRay computes, COMP.cpp:209-280, with MaxCrossings in the part of its RaycastBounces): each component's
+    // LastOcclusion is filled.  Uses each component's OcclusionRadius / OcclusionRays; no histogram or IR is touched.  RegisterGeometry
+    // commits Absorption only (FAcousticMaterial's other fields are carried and ignored), so here every surface blocks and
+    // transmission equals visible; a host that sets Transmission through fs_scene_set_materials_ex gets the per-band gains.
+    void UpdateOcclusion(uint32_t MaxCrossings, uint64_t OcclusionSeed)
+    {
+        if (ActiveSources.empty() || !Commit()) return;
+        const float lis[3] = {PawnLocation.X, PawnLocation.Y, PawnLocation.Z};
+        const uint32_t S = (uint32_t)ActiveSources.size();
+        std::vector<fs_occlusion_source> desc(S);
+        for (uint32_t s = 0; s < S; ++s) {
+            const UFrequenSeeAudioComponent& c = *ActiveSources[s];
+            const FVector3f L = c.GetActorLocation();
+            desc[s] = fs_occlusion_source{};
+            desc[s].pos[0] = L.X; desc[s].pos[1] = L.Y; desc[s].pos[2] = L.Z;
+            desc[s].radius = c.OcclusionRadius;
+            desc[s].n_rays = c.OcclusionRays;
+        }
+        std::vector<fs_occlusion_result> res(S);
+        if (Ctx->Check(fs_occlusion(Ctx->Get(), desc.data(), S, lis, MaxCrossings, OcclusionSeed, res.data())) != FS_OK) return;
+        for (uint32_t s = 0; s < S; ++s) ActiveSources[s]->LastOcclusion = res[s];
+    }
 
 private:
     // the orientations of the sources a trace is about to trace (slot s = Src[s]), or none when every one is omni
