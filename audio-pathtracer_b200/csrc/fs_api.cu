@@ -198,7 +198,7 @@ void fs_destroy(fs_ctx* ctx)
     cudaFree(ctx->d_bsdf_tab); cudaFree(ctx->d_lobes);
     fs_bvh_free(&ctx->bvh);
     cudaFree(ctx->d_verts); cudaFree(ctx->d_tri_mat); cudaFree(ctx->d_refl_over_pi);
-    cudaFree(ctx->d_hist); cudaFree(ctx->d_m2); cudaFree(ctx->d_noise); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
+    cudaFree(ctx->d_hist); cudaFree(ctx->d_m2); cudaFree(ctx->d_noise); cudaFree(ctx->d_acou); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
     cudaFree(ctx->d_dir_gain); cudaFree(ctx->d_dir_orient);
     cudaFree(ctx->d_occl_tau); cudaFree(ctx->d_occl);
     cudaFree(ctx->d_amp); cudaFree(ctx->d_energy);
@@ -1475,6 +1475,43 @@ int fs_get_histogram_m2(fs_ctx* ctx, uint64_t* out)
     const size_t n = (size_t)ctx->hist_cur_sources * (ctx->cfg.n_bands + 1u) * ctx->cfg.n_bins;
     CK(cudaMemcpyAsync(out, ctx->d_m2, sizeof(ulonglong2) * n, cudaMemcpyDeviceToHost, ctx->stream));
     return finish_stats(ctx);
+}
+
+// ---- room-acoustic parameters ---------------------------------------------------------------------
+int fs_get_acoustic_params(fs_ctx* ctx, fs_acoustic_params* out, uint32_t n_sources, float* edc_db_out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (!out) return fail(ctx, FS_ERR_INVALID, "fs_get_acoustic_params: null output");
+    if (!ctx->d_hist || ctx->hist_cur_sources == 0)
+        return fail(ctx, FS_ERR_STATE, "fs_get_acoustic_params: no histogram (trace or fs_set_histogram first)");
+    const uint32_t S = ctx->hist_cur_sources, B = ctx->cfg.n_bands, K = ctx->cfg.n_bins, W = B + 1u;
+    if (n_sources != S) return fail(ctx, FS_ERR_INVALID, "fs_get_acoustic_params: n_sources differs from fs_get_histogram_sources");
+    dev_guard g(ctx->device);
+    const size_t n_rec = (size_t)S * W, rec_bytes = (sizeof(fs_acoustic_slot) * n_rec + 255u) & ~(size_t)255u;
+    const size_t need = rec_bytes + (edc_db_out ? sizeof(float) * n_rec * K : 0u);
+    if (ctx->acou_cap < need) {
+        cudaFree(ctx->d_acou); ctx->d_acou = nullptr; ctx->acou_cap = 0;
+        CK(cudaMalloc(&ctx->d_acou, need));
+        ctx->acou_cap = need;
+    }
+    fs_acoustic_slot* d_rec = (fs_acoustic_slot*)ctx->d_acou;
+    float* d_edc = edc_db_out ? (float*)((char*)ctx->d_acou + rec_bytes) : nullptr;
+    std::vector<fs_acoustic_slot> h(n_rec);
+    CK(fs_acoustics_run(ctx->d_hist, S, B, K, ctx->cfg.bin_ms, d_rec, d_edc, ctx->stream));
+    ctx->launches.fetch_add(1);
+    CK(cudaMemcpyAsync(h.data(), d_rec, sizeof(fs_acoustic_slot) * n_rec, cudaMemcpyDeviceToHost, ctx->stream));
+    if (edc_db_out) CK(cudaMemcpyAsync(edc_db_out, d_edc, sizeof(float) * n_rec * K, cudaMemcpyDeviceToHost, ctx->stream));
+    const int rc = finish_stats(ctx);
+    if (rc != FS_OK && rc != FS_ERR_OVERFLOW) return rc;
+    for (uint32_t s = 0; s < S; ++s) {
+        fs_acoustic_params& o = out[s];
+        memset(&o, 0, sizeof(o));
+        const fs_acoustic_slot* r = h.data() + (size_t)s * W;
+        for (uint32_t b = 0; b < B; ++b) o.band[b] = r[b];
+        o.broadband = r[B];
+        o.no_energy = r[B].onset_bin == 0xffffffffu ? 1u : 0u;
+    }
+    return rc;
 }
 
 // ---- directional sources ------------------------------------------------------------------------

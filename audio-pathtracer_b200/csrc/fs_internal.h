@@ -217,6 +217,7 @@ struct fs_ctx {
     // fs_trace / fs_trace_sources / fs_update* / fs_multi_trace*, cleared by every other call that writes d_hist)
     ulonglong2* d_m2; uint32_t m2_sources; bool m2_valid;
     double* d_noise; uint32_t noise_cap;    // fs_get_noise scratch: [S] path counts (u64), then [S][B+1] (signal, variance)
+    void* d_acou; size_t acou_cap;          // fs_get_acoustic_params scratch: [S][B+1] records, then the [S][B+1][K] float EDC
     void* d_src_tab; uint32_t src_tab_cap;  // per-source budgets on the device: [S+1] u64 offsets, then [S] u32 depths
     // directional sources: the installed pattern table [P][FS_MAX_BANDS][FS_DIR_POINTS] and orientations [dir_sources]
     // (float4: unit forward, bits(pattern)); dir_sources = 0: none installed, every source omni
@@ -290,6 +291,11 @@ cudaError_t fs_ir_build(fs_ctx* ctx, const unsigned long long* d_hist_src, uint6
 // moments and the per-source pair counts d_n [S]; out [S][B+1][2] (signal, variance), energy units.  Fixed-order double sums.
 cudaError_t fs_noise_reduce(const unsigned long long* d_hist, const ulonglong2* d_m2, const uint64_t* d_n, uint32_t n_sources,
                             uint32_t n_bands, uint32_t n_bins, double* d_out, cudaStream_t st);
+
+// fs_acoustics.cu: k_acoustics, one CTA per (source, band or broadband slot) of the histogram [S][B][K]; records d_out
+// [S][B+1] and, when d_edc is not null, the decay curves d_edc [S][B+1][K] in dB
+cudaError_t fs_acoustics_run(const unsigned long long* d_hist, uint32_t n_sources, uint32_t n_bands, uint32_t n_bins, float bin_ms,
+                             fs_acoustic_slot* d_out, float* d_edc, cudaStream_t st);
 
 // fs_conv.cu
 cudaError_t fs_conv_setup(fs_ctx* ctx);

@@ -9,3 +9,4 @@ from . import capi, scenes  # noqa: F401
 from .capi import Context, MultiContext, FrequenSeeError, default_config, load_float_array, save_float_array, allocate_paths  # noqa: F401
 from .capi import directivity_polar, OMNI  # noqa: F401
 from .capi import OcclusionSource, OcclusionResult  # noqa: F401
+from .capi import AcousticParams, AcousticSlot, DecayFit  # noqa: F401

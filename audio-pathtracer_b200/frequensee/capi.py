@@ -47,6 +47,7 @@ ABI_SYMBOLS = [
     "fs_set_directivity_patterns", "fs_set_source_directivity", "fs_directivity_polar",
     "fs_multi_set_directivity_patterns", "fs_multi_set_source_directivity",
     "fs_occlusion",
+    "fs_get_acoustic_params",
 ]
 
 
@@ -218,6 +219,27 @@ def occlusion_sources(src_pos, radius, n_rays):
     return arr, len(src)
 
 
+AP_EDT, AP_T20, AP_T30, AP_C50, AP_C80, AP_TS = 1, 2, 4, 8, 16, 32    # FS_AP_*: valid bits of an AcousticSlot
+NO_ONSET = 0xFFFFFFFF
+
+
+class DecayFit(C.Structure):
+    """fs_decay_fit: one least-squares fit of the Schroeder decay curve (time_s = -60 / slope; NaN unless valid)"""
+    _fields_ = [("time_s", C.c_double), ("r", C.c_double), ("first_bin", C.c_uint32), ("n_points", C.c_uint32)]
+
+
+class AcousticSlot(C.Structure):
+    """fs_acoustic_slot: EDT / T20 / T30, C50 / C80 / D50 and centre time of one band or the broadband sum"""
+    _fields_ = [("edt", DecayFit), ("t20", DecayFit), ("t30", DecayFit), ("c50_db", C.c_double), ("c80_db", C.c_double),
+                ("d50", C.c_double), ("ts_s", C.c_double), ("onset_bin", C.c_uint32), ("valid", C.c_uint32)]
+
+
+class AcousticParams(C.Structure):
+    """fs_acoustic_params: the room-acoustic parameters of one source, broadband and per band"""
+    _fields_ = [("no_energy", C.c_uint32), ("reserved", C.c_uint32), ("broadband", AcousticSlot),
+                ("band", AcousticSlot * MAX_BANDS)]
+
+
 class FrequenSeeError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__("frequensee error %d: %s" % (code, msg))
@@ -313,6 +335,7 @@ def load():
     L.fs_multi_set_directivity_patterns.argtypes = [vp, vp, u32]
     L.fs_multi_set_source_directivity.argtypes = [vp, vp, u32]
     L.fs_occlusion.argtypes = [vp, vp, u32, vp, u32, u64, vp]
+    L.fs_get_acoustic_params.argtypes = [vp, vp, u32, vp]
     for n in ABI_SYMBOLS:
         if n not in ("fs_default_config", "fs_destroy", "fs_last_error", "fs_multi_destroy", "fs_multi_last_error",
                      "fs_multi_device_count", "fs_multi_context"):
@@ -586,6 +609,17 @@ class Context:
             "band_variance": np.array([list(arr[s].band_variance)[:B] for s in range(S)]).reshape(S, B),
             "band_snr_db": np.array([list(arr[s].band_snr_db)[:B] for s in range(S)]).reshape(S, B),
         }
+
+    def acoustic_params(self, edc=False):
+        """fs_get_acoustic_params: the AcousticParams[S] of the current histogram, and with edc=True also the decay curves as
+        float32 [S][B+1][K] in dB (slot B is broadband)"""
+        n = C.c_uint32(0)
+        self._ck(self.L.fs_get_histogram_sources(self.h, C.byref(n)))
+        S = n.value
+        arr = (AcousticParams * max(S, 1))()
+        curves = np.empty((S, self.cfg.n_bands + 1, self.cfg.n_bins), np.float32) if edc else None
+        self._ck(self.L.fs_get_acoustic_params(self.h, arr, S, curves.ctypes.data if edc else None))
+        return (arr, curves) if edc else arr
 
     def histogram_m2(self):
         """fs_get_histogram_m2: second moments of the last update, uint64 [S][B+1][K][2] (lo, hi); slot B is broadband"""

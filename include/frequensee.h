@@ -339,6 +339,72 @@ int fs_get_histogram_m2(fs_ctx* ctx, uint64_t* out);
 int fs_allocate_paths(const fs_noise_stats* st, uint32_t n_sources, uint64_t total, uint64_t min_paths, uint64_t max_paths,
                       const float* weight, uint64_t* n_out);
 
+/* ---- room-acoustic parameters of the energy histogram ----------------------------------------------
+ * EXTENDS the reference, which turns the histogram into a convolution IR only.  A parametric reverb (a decay time per band
+ * and an early / late balance), game logic and checks of the simulation itself need what the histogram means acoustically:
+ * the ISO 3382-1 parameters EDT, T20, T30, C50, C80, D50 and the centre time Ts, per band and broadband.
+ * Input: the histogram fs_get_histogram would return (S = fs_get_histogram_sources sources, B = n_bands, K = n_bins), after
+ * any call that leaves one (fs_trace*, fs_update*, fs_set_histogram*, fs_multi_trace* on context 0), in every connection
+ * mode.  Each source has B + 1 slots: band b, and broadband = the band sum formed exactly in 128 bits.  Every value is a
+ * ratio or a slope, so nothing is normalised by the path count.  Per slot, E_k = the integer energy of bin k and
+ * delta = (double)bin_ms * 1e-3 s:
+ *   overflow bin: every arrival at or after (K-1) delta is counted in bin K-1.  It is in every energy sum, but it is never a
+ *     fit point and never a time.  Bins 0 .. K-2 are the regular bins.
+ *   onset: k0 = the first k with E_k > 0 (the first arrival: the histogram has no background noise).  None: the slot has no
+ *     energy, every value is NaN, valid = 0, onset_bin = 0xffffffff, first_bin = n_points = 0 (and no_energy = 1 for the
+ *     broadband slot).  Times are relative to the start of bin k0: t_k = (k - k0) delta.
+ *   decay curve (Schroeder): S0 = sum_k E_k, R_k = sum_{j >= k} E_j (exact), as doubles (double)hi 2^64 + (double)lo;
+ *     L_k = 10 log10(R_k / S0) dB: 0 for k <= k0, -inf where R_k = 0.
+ *   fits EDT [0, -10] dB, T20 [-5, -25] dB, T30 [-5, -35] dB: with C_x the double nearest 10^(x/10), ka = the first k >= k0
+ *     with (double)R_k <= (double)S0 C_hi (K if none), kb = the last regular k with (double)R_k >= (double)S0 C_lo; the points
+ *     are ka .. kb (contiguous: the curve is monotone), n = kb - ka + 1 (0 when kb < ka).  Least squares of L_k on t_k with
+ *     w_k = 2k - ka - kb: slope m = 6 sum w_k L_k / (delta n (n^2 - 1)) dB/s (summed over L_k - L_ka from the exact integer
+ *     drop R_ka - R_k: the same line, with the digits of a nearly flat curve kept), time_s = -60 / m, r = the correlation
+ *     coefficient of the same fit (negative for a decay; ISO 3382-1 Annex B reports 1000 (1 - r^2)).  Valid iff the curve
+ *     has fallen below lo before the overflow bin ((double)R_{K-1} < (double)S0 C_lo), n >= 3 and m < 0; otherwise time_s
+ *     and r are NaN, first_bin and n_points are reported either way.
+ *   clarity and definition: nX = (uint32)(X / (double)bin_ms + 0.5) bins for X = 50, 80 ms (exact at bin edges only when
+ *     bin_ms divides X, otherwise rounded to the nearest bin); early_X = sum_{k0 <= k < k0 + nX} E_k, late_X = S0 - early_X
+ *     (exact); C_X = 10 log10(early_X / late_X) dB (+inf when late_X = 0, e.g. in free field: a valid value); D50 =
+ *     early_50 / S0.  Valid iff nX >= 1 and k0 + nX <= K - 1 (the window lies in regular bins).
+ *   centre time: Ts = delta (sum_k (k - k0) E_k) / S0, the sum exact in 128 bits.  Valid iff E_{K-1} = 0.
+ *   EDC (optional): float [S][B+1][K] of (float)L_k (0 for k < k0, -inf where R_k = 0; NaN throughout a slot without energy).
+ * State and errors: n_sources must equal fs_get_histogram_sources and out must not be NULL (FS_ERR_INVALID); FS_ERR_STATE
+ * when there is no histogram; a rejected call writes nothing.  FS_ERR_OVERFLOW is the sticky flag of the last trace, as for
+ * every fs_get_*: the results are filled, from the histogram that trace left incomplete.  One kernel and one copy (two with
+ * the EDC) on the context stream after the work already enqueued there; synchronises.  Reads and writes nothing of the
+ * histogram, the noise moments, the IRs, the convolver or fs_stats (except kernel_launches); results are bit-identical for
+ * a given histogram.  Several GPUs: call it on fs_multi_context(m, 0), which holds the reduced histogram. */
+typedef struct fs_decay_fit {
+    double   time_s;     /* -60 / slope; NaN unless valid */
+    double   r;          /* correlation coefficient of the fit; NaN unless valid */
+    uint32_t first_bin;  /* ka */
+    uint32_t n_points;   /* kb - ka + 1, 0 if none */
+} fs_decay_fit;          /* 24 bytes */
+
+#define FS_AP_EDT 1u
+#define FS_AP_T20 2u
+#define FS_AP_T30 4u
+#define FS_AP_C50 8u     /* C50 and D50 */
+#define FS_AP_C80 16u
+#define FS_AP_TS  32u
+
+typedef struct fs_acoustic_slot {
+    fs_decay_fit edt, t20, t30;
+    double   c50_db, c80_db, d50, ts_s;   /* NaN unless the matching valid bit is set */
+    uint32_t onset_bin;                   /* k0; 0xffffffff: no energy */
+    uint32_t valid;                       /* FS_AP_* */
+} fs_acoustic_slot;                       /* 112 bytes */
+
+typedef struct fs_acoustic_params {
+    uint32_t no_energy, reserved;         /* no_energy: the broadband slot has no energy */
+    fs_acoustic_slot broadband;
+    fs_acoustic_slot band[FS_MAX_BANDS];  /* bands >= n_bands: all zero, valid 0 */
+} fs_acoustic_params;                     /* 1016 bytes */
+
+int fs_get_acoustic_params(fs_ctx* ctx, fs_acoustic_params* out /* [n_sources] */, uint32_t n_sources,
+                           float* edc_db_out /* [S][B+1][K] or NULL */);
+
 /* ---- directional sources ----------------------------------------------------------------------
  * EXTENDS the reference: its emitters radiate the same energy in every direction (node 0 of the source subpath samples a
  * uniform sphere, VRand at SUB.cpp:306-311, and EvaluatePath starts every path at Energy = 1, SUB.cpp:367).  A directional

@@ -89,6 +89,9 @@ public:
     float OcclusionRadius = 0.0f;
     uint32_t OcclusionRays = 64;
     fs_occlusion_result LastOcclusion{};
+    // room-acoustic parameters of this source's histogram in the last UpdateSources() (UpdateAcousticParams,
+    // fs_get_acoustic_params): decay times, clarity and centre time per band and broadband, the inputs of a parametric reverb
+    fs_acoustic_params LastAcoustics{};
 
     std::vector<float> EnergyBuffer;   // COMP.h:70
     void FlushEnergyBuffer() { EnergyBuffer.assign(NumBins, 0.0f); bUseDeviceHistogram = false; }          // COMP.h:76-79
@@ -214,6 +217,7 @@ public:
         const float src[3] = {S.X, S.Y, S.Z}, lis[3] = {PawnLocation.X, PawnLocation.Y, PawnLocation.Z};
         // one source per call: the device histogram of source slot 0 belongs to Src until the next update
         UFrequenSeeAudioComponent* One[1] = {&Src};
+        HistSources.clear();
         if (!InstallOrientations(One, 1)) return;
         if (Ctx->Check(fs_trace(Ctx->Get(), src, 1, lis, (uint64_t)Src.RaycastsPerTick, (uint32_t)Src.RaycastBounces,
                                 Seed++, nullptr)) != FS_OK) return;
@@ -259,8 +263,10 @@ public:
             desc[s].n_paths = budget[s];
         }
         NoiseSources.clear();
+        HistSources.clear();
         if (!InstallOrientations(ActiveSources.data(), S)) return;
         if (Ctx->Check(fs_trace_sources(Ctx->Get(), desc.data(), S, lis, Seed++, nullptr)) != FS_OK) return;
+        HistSources = ActiveSources;
         fs_stats st;
         if (fs_get_stats(Ctx->Get(), &st) == FS_OK) LastConnected = st.connected;
         if (noise) {
@@ -304,7 +310,22 @@ public:
         for (uint32_t s = 0; s < S; ++s) ActiveSources[s]->LastOcclusion = res[s];
     }
 
+    // The room-acoustic parameters of every source of the last UpdateSources() in ONE fs_get_acoustic_params call: each
+    // component's LastAcoustics is filled (DecayTime from T30, else T20, else EDT by the valid bits; see INTEGRATION.md).
+    // Reads the histogram only.  Returns false, and leaves every LastAcoustics as it was, when the call fails or when the set
+    // of active sources has changed since that update (its histogram slots no longer belong to them: FS_ERR_STATE).
+    bool UpdateAcousticParams()
+    {
+        if (HistSources.empty() || HistSources != ActiveSources) { Ctx->Check(FS_ERR_STATE); return false; }
+        const uint32_t S = (uint32_t)ActiveSources.size();
+        std::vector<fs_acoustic_params> ap(S);
+        if (Ctx->Check(fs_get_acoustic_params(Ctx->Get(), ap.data(), S, nullptr)) != FS_OK) return false;
+        for (uint32_t s = 0; s < S; ++s) ActiveSources[s]->LastAcoustics = ap[s];
+        return true;
+    }
+
 private:
+    std::vector<UFrequenSeeAudioComponent*> HistSources;    // the sources whose histogram slots the last UpdateSources() filled
     // the orientations of the sources a trace is about to trace (slot s = Src[s]), or none when every one is omni
     bool InstallOrientations(UFrequenSeeAudioComponent* const* Src, uint32_t S)
     {
