@@ -1,6 +1,7 @@
 // fs_api.cu -- the extern "C" boundary (include/frequensee.h).  No CPU fallback anywhere: every
 // entry point either runs the CUDA path or returns an error.
 #include "fs_internal.h"
+#include "fs_diffraction.h"
 
 #include <nvtx3/nvToolsExt.h>          // header-only NVTX 3: named ranges per stage for nsys / ncu --nvtx (SURVEY section 5)
 #include <algorithm>
@@ -201,6 +202,7 @@ void fs_destroy(fs_ctx* ctx)
     cudaFree(ctx->d_hist); cudaFree(ctx->d_m2); cudaFree(ctx->d_noise); cudaFree(ctx->d_acou); cudaFree(ctx->d_counters); cudaFree(ctx->d_src_pos); cudaFree(ctx->d_dbg); cudaFree(ctx->d_src_tab);
     cudaFree(ctx->d_dir_gain); cudaFree(ctx->d_dir_orient);
     cudaFree(ctx->d_occl_tau); cudaFree(ctx->d_occl);
+    cudaFree(ctx->d_diff_edges); cudaFree(ctx->d_diff); cudaFree(ctx->d_diff_cand);
     cudaFree(ctx->d_amp); cudaFree(ctx->d_energy);
     for (cudaEvent_t e : ctx->kev) cudaEventDestroy(e);
     for (cudaEvent_t e : ctx->tev) cudaEventDestroy(e);
@@ -257,7 +259,7 @@ int fs_scene_set_triangles(fs_ctx* ctx, const float* verts, const uint32_t* tri_
         if (!(verts[i] == verts[i]) || fabsf(verts[i]) > 1e18f) return fail(ctx, FS_ERR_INVALID, "non-finite vertex");
     cudaFree(ctx->d_verts); cudaFree(ctx->d_tri_mat);
     ctx->d_verts = nullptr; ctx->d_tri_mat = nullptr;
-    ctx->n_tris = n_tris; ctx->committed = false; ctx->tris_set = false; ctx->verts_dirty = false;
+    ctx->n_tris = n_tris; ctx->committed = false; ctx->tris_set = false; ctx->verts_dirty = false; ctx->diff_valid = false;
     if (n_tris) {
         CK(cudaMalloc(&ctx->d_verts, sizeof(float) * 9 * n_tris));
         CK(cudaMalloc(&ctx->d_tri_mat, sizeof(uint32_t) * n_tris));
@@ -463,6 +465,7 @@ int fs_scene_commit(fs_ctx* ctx)
     apply_l2_policy(ctx);
     ctx->committed = true;
     ctx->verts_dirty = false;
+    ctx->diff_valid = false;
     return FS_OK;
 }
 
@@ -505,6 +508,7 @@ int fs_scene_refit(fs_ctx* ctx, float* cost_ratio_out)
     ctx->launches.fetch_add(launches);
     ctx->trav = fs_choose_traversal(ctx->tune, ctx->bvh);
     ctx->verts_dirty = false;
+    ctx->diff_valid = false;
     if (cost_ratio_out) *cost_ratio_out = ratio;
     return FS_OK;
 }
@@ -1659,6 +1663,122 @@ int fs_occlusion(fs_ctx* ctx, const fs_occlusion_source* src, uint32_t n_sources
     }
     if ((uint32_t)h[(size_t)S * W])
         return fail(ctx, FS_ERR_OVERFLOW, "fs_occlusion: BVH traversal stack overflow (tree deeper than FS_STACK_SIZE): the results are invalid");
+    return FS_OK;
+}
+
+// ---- first-order edge diffraction -----------------------------------------------------------------
+static_assert(sizeof(fs_diffraction_result) == 68, "fs_diffraction_result is part of the ABI");
+static_assert(sizeof(fs_diff_edge) == 64, "fs_diff_edge is read as four 16-byte words");
+
+// the checks every diffraction entry point shares; nothing is enqueued before they pass
+static int diffraction_state(fs_ctx* ctx, const char* who, float min_fold_deg)
+{
+    if (!ctx->committed) return fail(ctx, FS_ERR_STATE, (std::string(who) + ": call fs_scene_commit first").c_str());
+    if (ctx->verts_dirty)
+        return fail(ctx, FS_ERR_STATE, (std::string(who) + ": triangles were moved; call fs_scene_refit (or fs_scene_commit) first").c_str());
+    if (!std::isfinite(min_fold_deg) || min_fold_deg < 0.0f || min_fold_deg > 180.0f)
+        return fail(ctx, FS_ERR_INVALID, (std::string(who) + ": min_fold_deg must be finite and in [0, 180]").c_str());
+    return FS_OK;
+}
+
+// the edge set for min_fold_deg: built on first use after a commit, refit or threshold change
+static int diffraction_edges(fs_ctx* ctx, float min_fold_deg)
+{
+    if (ctx->diff_valid && ctx->diff_fold_deg == min_fold_deg) return FS_OK;
+    cudaFree(ctx->d_diff_edges); ctx->d_diff_edges = nullptr; ctx->n_diff_edges = 0; ctx->diff_valid = false;
+    const float c_min = (float)(-cos((double)min_fold_deg * (M_PI / 180.0)));
+    uint64_t launches = 0;
+    const cudaError_t e = fs_diffraction_edges(ctx->stream, ctx->d_verts, (uint32_t)ctx->n_tris, c_min, &ctx->d_diff_edges,
+                                               &ctx->n_diff_edges, &launches);
+    ctx->launches.fetch_add(launches);
+    CK(e);
+    ctx->diff_fold_deg = min_fold_deg;
+    ctx->diff_valid = true;
+    return FS_OK;
+}
+
+int fs_diffraction(fs_ctx* ctx, const float* src_pos, uint32_t n_sources, const float lis_pos[3], float min_fold_deg,
+                   const float* band_hz, fs_diffraction_result* out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (int rc = diffraction_state(ctx, "fs_diffraction", min_fold_deg)) return rc;
+    if (!src_pos || !lis_pos || !out) return fail(ctx, FS_ERR_INVALID, "fs_diffraction: null argument");
+    if (n_sources == 0 || n_sources > FS_MAX_SOURCES) return fail(ctx, FS_ERR_INVALID, "fs_diffraction: n_sources must be 1..4096");
+    auto bad_pos = [](const float* p) {
+        for (int a = 0; a < 3; ++a) if (!std::isfinite(p[a]) || fabsf(p[a]) > 1e18f) return true;
+        return false;
+    };
+    if (bad_pos(lis_pos)) return fail(ctx, FS_ERR_INVALID, "fs_diffraction: non-finite or > 1e18 listener position");
+    const uint32_t S = n_sources, B = ctx->cfg.n_bands;
+    for (uint32_t s = 0; s < S; ++s)
+        if (bad_pos(src_pos + 3ull * s))
+            return fail(ctx, FS_ERR_INVALID, ("fs_diffraction: source " + std::to_string(s) + ": non-finite or > 1e18 position").c_str());
+    fs_diff_run a;
+    memset(&a, 0, sizeof(a));
+    for (uint32_t b = 0; b < B; ++b) {
+        if (band_hz && !(std::isfinite(band_hz[b]) && band_hz[b] > 0.0f))
+            return fail(ctx, FS_ERR_INVALID, "fs_diffraction: band_hz entries must be finite and > 0");
+        a.band_hz[b] = band_hz ? band_hz[b] : fs_diff_default_hz(b);
+    }
+    dev_guard g(ctx->device);
+    if (int rc = diffraction_edges(ctx, min_fold_deg)) return rc;
+    // scratch: [S] float4 sources | [S] u64 best | [S] u32 path counts | u64 candidates, u64 rays, u32 overflow | [S] results
+    const size_t o_best = 16ull * FS_MAX_SOURCES, o_np = o_best + 8ull * FS_MAX_SOURCES, o_misc = o_np + 4ull * FS_MAX_SOURCES,
+                 o_out = o_misc + 32ull, cap = o_out + sizeof(fs_diffraction_result) * FS_MAX_SOURCES;   // 0.4 MB: the largest call
+    if (!ctx->d_diff) {
+        CK(cudaMalloc(&ctx->d_diff, cap));
+        ctx->diff_cap = cap;
+    }
+    char* base = (char*)ctx->d_diff;
+    std::vector<float4> hsrc(S);
+    for (uint32_t s = 0; s < S; ++s) hsrc[s] = make_float4(src_pos[3 * s], src_pos[3 * s + 1], src_pos[3 * s + 2], 0.0f);
+    fs_trace_params tp;
+    fill_params(ctx, &tp, nullptr, 1, 1, 0);
+    a.bv = tp.bv;
+    a.edges = ctx->d_diff_edges; a.n_edges = ctx->n_diff_edges;
+    a.src = (const float4*)base; a.n_src = S;
+    for (int i = 0; i < 3; ++i) a.lis[i] = lis_pos[i];
+    a.eps_offset = ctx->cfg.eps_offset; a.eps_connect = ctx->cfg.eps_connect; a.sound_speed = ctx->cfg.sound_speed;
+    a.n_bands = B;
+    a.cand = &ctx->d_diff_cand; a.cand_cap = &ctx->diff_cand_cap;
+    a.best = (unsigned long long*)(base + o_best);
+    a.n_paths = (uint32_t*)(base + o_np);
+    a.d_count = (unsigned long long*)(base + o_misc);
+    a.rays = a.d_count + 1;
+    a.overflow = (uint32_t*)(a.d_count + 2);
+    a.out = (fs_diffraction_result*)(base + o_out);
+    CK(cudaMemcpyAsync(base, hsrc.data(), sizeof(float4) * S, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(a.best, 0xff, 8ull * S, ctx->stream));
+    CK(cudaMemsetAsync(a.n_paths, 0, 4ull * S, ctx->stream));
+    CK(cudaMemsetAsync(a.d_count, 0, 32, ctx->stream));
+    uint64_t launches = 0;
+    const cudaError_t e = fs_diffraction_run(a, ctx->stream, &launches, nullptr);
+    ctx->launches.fetch_add(launches);
+    CK(e);
+    uint32_t overflow = 0;
+    CK(cudaMemcpyAsync(out, a.out, sizeof(fs_diffraction_result) * S, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&overflow, a.overflow, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (overflow)
+        return fail(ctx, FS_ERR_OVERFLOW, "fs_diffraction: BVH traversal stack overflow (tree deeper than FS_STACK_SIZE): the results are invalid");
+    return FS_OK;
+}
+
+int fs_debug_diffraction_edges(fs_ctx* ctx, float min_fold_deg, uint32_t* out, uint64_t cap, uint64_t* n_out)
+{
+    if (!ctx) return FS_ERR_INVALID;
+    if (int rc = diffraction_state(ctx, "fs_debug_diffraction_edges", min_fold_deg)) return rc;
+    if (!n_out) return fail(ctx, FS_ERR_INVALID, "fs_debug_diffraction_edges: null n_out");
+    dev_guard g(ctx->device);
+    if (int rc = diffraction_edges(ctx, min_fold_deg)) return rc;
+    const uint64_t n = ctx->n_diff_edges, m = out ? std::min<uint64_t>(n, cap) : 0;
+    if (m) {
+        std::vector<fs_diff_edge> h(m);
+        CK(cudaMemcpyAsync(h.data(), ctx->d_diff_edges, sizeof(fs_diff_edge) * m, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        for (uint64_t i = 0; i < m; ++i) { out[2 * i] = h[i].tri; out[2 * i + 1] = h[i].k & 3u; }
+    }
+    *n_out = n;
     return FS_OK;
 }
 

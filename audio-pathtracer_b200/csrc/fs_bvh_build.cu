@@ -1251,13 +1251,31 @@ __global__ void k_ri_apply(uint32_t n_inner, const int* __restrict__ parent, con
 
 }  // namespace
 
+uint32_t fs_radix_sort_blocks(uint32_t n) { return (n + SORT_TILE - 1) / SORT_TILE; }
 
+void fs_radix_sort_u64(cudaStream_t st, uint64_t* keys, uint32_t* vals, uint64_t* keys_tmp, uint32_t* vals_tmp, uint32_t n,
+                       uint32_t* block_hist, uint64_t* launches)
+{
+    const uint32_t n_blocks = fs_radix_sort_blocks(n);
+    uint64_t *ki = keys, *ko = keys_tmp;
+    uint32_t *vi = vals, *vo = vals_tmp;
+    for (int pass = 0; pass < 8; ++pass) {
+        int shift = pass * 8;
+        k_sort_hist<<<n_blocks, SORT_THREADS, 0, st>>>(ki, n, shift, block_hist, n_blocks);
+        k_sort_scan<<<1, 1024, 0, st>>>(block_hist, 256u * n_blocks);
+        k_sort_scatter<<<n_blocks, SORT_THREADS, 0, st>>>(ki, vi, ko, vo, n, shift, block_hist, n_blocks);
+        *launches += 3;
+        uint64_t* tk = ki; ki = ko; ko = tk;
+        uint32_t* tv = vi; vi = vo; vo = tv;
+    }
+    // 8 passes: the result is back in keys / vals
+}
 
 #define BCHECK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { err = e_; goto fail; } } while (0)
 
 // exclusive scan helper (device arrays); tile_sums must hold ceil(n/1024) + 1 entries
-static void scan_u32(cudaStream_t st, const uint32_t* in, uint32_t* out, uint32_t n, uint32_t* tile_sums,
-                     uint32_t* total, uint64_t* launches)
+void fs_scan_u32(cudaStream_t st, const uint32_t* in, uint32_t* out, uint32_t n, uint32_t* tile_sums,
+                 uint32_t* total, uint64_t* launches)
 {
     const uint32_t tiles = (n + SCAN_TILE - 1) / SCAN_TILE;
     k_scan_tiles<<<tiles, SCAN_TILE, 0, st>>>(in, out, n, tile_sums);
@@ -1294,8 +1312,8 @@ static cudaError_t ploc_build(cudaStream_t st, uint32_t n, const float4* bb_lo, 
         k_ploc_nn<<<g, TPB, 0, st>>>(cur, lo[pp], hi[pp], nn, radius);
         k_ploc_flags<<<g, TPB, 0, st>>>(cur, nn, keep, mflag);
         *launches += 2;
-        scan_u32(st, keep, keep_scan, cur, tile_sums, totals, launches);
-        scan_u32(st, mflag, merge_scan, cur, tile_sums, totals + 1, launches);
+        fs_scan_u32(st, keep, keep_scan, cur, tile_sums, totals, launches);
+        fs_scan_u32(st, mflag, merge_scan, cur, tile_sums, totals + 1, launches);
         k_ploc_merge<<<g, TPB, 0, st>>>(cur, nn, keep_scan, merge_scan, keep, mflag, made, n_inner, lo[pp], hi[pp], ref[pp],
                                         lo[pp ^ 1], hi[pp ^ 1], ref[pp ^ 1], nodes);
         ++*launches;
@@ -1338,7 +1356,7 @@ static cudaError_t bvh2_rotate(cudaStream_t st, uint32_t n_inner, float4* nodes,
             const uint32_t g = (nf + TPB - 1) / TPB;
             uint32_t next = 0;
             k_bvh2_count<<<g, TPB, 0, st>>>(nodes, order + base, nf, cnt); ++*launches;
-            scan_u32(st, cnt, off, nf, tile_sums, total, launches);
+            fs_scan_u32(st, cnt, off, nf, tile_sums, total, launches);
             BCHECK(cudaMemcpyAsync(&next, total, 4, cudaMemcpyDeviceToHost, st));
             BCHECK(cudaStreamSynchronize(st));
             if (base + nf + next > n_inner) { err = cudaErrorUnknown; goto fail; }
@@ -1464,7 +1482,7 @@ static cudaError_t wide_compact(cudaStream_t st, uint32_t n_inner, const uint4* 
         const uint32_t g = (nf + TPB - 1) / TPB;
         uint32_t next = 0;
         k_wide_count<<<g, TPB, 0, st>>>(sparse, fr[pp], nf, cnt); ++*launches;
-        scan_u32(st, cnt, off, nf, tile_sums, total, launches);
+        fs_scan_u32(st, cnt, off, nf, tile_sums, total, launches);
         k_wide_place<<<g, TPB, 0, st>>>(sparse, dense, sparse_prov, dense_prov, fr[pp], nf, off, base, fr[pp ^ 1]); ++*launches;
         BCHECK(cudaMemcpyAsync(&next, total, 4, cudaMemcpyDeviceToHost, st));
         BCHECK(cudaStreamSynchronize(st));
@@ -1516,8 +1534,8 @@ static cudaError_t w8_build(cudaStream_t st, uint32_t n, uint32_t n_inner, const
         const uint32_t g = (nf + TPB - 1) / TPB;
         uint32_t next[2] = {0, 0};
         k_w8_count<<<g, TPB, 0, st>>>(tmp, fr[pp], nf, cnt_in, cnt_leaf); ++*launches;
-        scan_u32(st, cnt_in, off_in, nf, tile_sums, total, launches);
-        scan_u32(st, cnt_leaf, off_leaf, nf, tile_sums, total + 1, launches);
+        fs_scan_u32(st, cnt_in, off_in, nf, tile_sums, total, launches);
+        fs_scan_u32(st, cnt_leaf, off_leaf, nf, tile_sums, total + 1, launches);
         k_w8_place<<<g, TPB, 0, st>>>(tmp, ref, dense, fr[pp], nf, off_in, off_leaf, base, tri_base, fr[pp ^ 1], tris, tris8, map);
         ++*launches;
         BCHECK(cudaMemcpyAsync(next, total, 8, cudaMemcpyDeviceToHost, st));
@@ -1550,7 +1568,7 @@ cudaError_t fs_bvh_build(cudaStream_t st, const float* d_verts, const uint32_t* 
     out->n_tris = n;
     if (n == 0) return cudaSuccess;
     const uint32_t n_inner = n > 1 ? n - 1 : 1;
-    const uint32_t n_blocks_sort = (n + SORT_TILE - 1) / SORT_TILE;
+    const uint32_t n_blocks_sort = fs_radix_sort_blocks(n);
     float4 *tlo = nullptr, *thi = nullptr, *bb_lo = nullptr, *bb_hi = nullptr;
     uint64_t *keys0 = nullptr, *keys1 = nullptr;
     uint32_t *vals0 = nullptr, *vals1 = nullptr, *block_hist = nullptr, *misc = nullptr, *arrive = nullptr;
@@ -1592,20 +1610,7 @@ cudaError_t fs_bvh_build(cudaStream_t st, const float* d_verts, const uint32_t* 
     k_init_bounds<<<1, 32, 0, st>>>(misc); ++*launches;
     k_tri_bounds<<<gb, TPB, 0, st>>>(d_verts, n, tlo, thi, misc, misc + 6); ++*launches;
     k_morton<<<gb, TPB, 0, st>>>(tlo, thi, n, misc, keys0, vals0); ++*launches;
-    {
-        uint64_t *ki = keys0, *ko = keys1;
-        uint32_t *vi = vals0, *vo = vals1;
-        for (int pass = 0; pass < 8; ++pass) {
-            int shift = pass * 8;
-            k_sort_hist<<<n_blocks_sort, SORT_THREADS, 0, st>>>(ki, n, shift, block_hist, n_blocks_sort);
-            k_sort_scan<<<1, 1024, 0, st>>>(block_hist, 256u * n_blocks_sort);
-            k_sort_scatter<<<n_blocks_sort, SORT_THREADS, 0, st>>>(ki, vi, ko, vo, n, shift, block_hist, n_blocks_sort);
-            *launches += 3;
-            uint64_t* tk = ki; ki = ko; ko = tk;
-            uint32_t* tv = vi; vi = vo; vo = tv;
-        }
-        // 8 passes: result is back in keys0/vals0
-    }
+    fs_radix_sort_u64(st, keys0, vals0, keys1, vals1, n, block_hist, launches);
     k_pack<<<gb, TPB, 0, st>>>(d_verts, d_mats, vals0, n, tlo, thi, out->tris, out->tri_orig, out->tri_mat, out->tri_nm, bb_lo, bb_hi);
     ++*launches;
     if (n == 1) {

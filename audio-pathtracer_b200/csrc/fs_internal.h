@@ -17,6 +17,8 @@
 
 #define FS_TOP_CAP 1024          // nodes of the shared-memory treelet (64 KB)
 
+struct fs_diff_edge;             // fs_diffraction.h
+
 struct fs_bvh_device {
     float4* nodes;
     float4* tris;
@@ -227,6 +229,12 @@ struct fs_ctx {
     // one call: [S][B+1] u64 sums, the call's own overflow flag (one u64 slot), [S] float4 sources, [S+1] u32 ray offsets
     float* d_occl_tau;
     void* d_occl; uint32_t occl_cap;
+    // fs_diffraction: the edge set, built by the first call after a commit, refit or threshold change (diff_valid false
+    // until then), for diff_fold_deg; and the scratch of one call: [S] float4 sources, [S] u64 best, [S] u32 path counts,
+    // u64 candidate count, u64 rays, u32 overflow, [S] results; the candidate pairs
+    fs_diff_edge* d_diff_edges; uint32_t n_diff_edges; float diff_fold_deg; bool diff_valid;
+    void* d_diff; size_t diff_cap;
+    uint2* d_diff_cand; unsigned long long diff_cand_cap;
     fs_dev_counters* d_counters;
     // traversal-stack overflow of the last trace: one 4-byte async copy into pinned memory after every fs_trace*, looked at
     // by the next call that can (sticky until reported)
@@ -276,6 +284,37 @@ cudaError_t fs_wave_debug_rays(fs_ctx* ctx, const fs_trace_params& tp, const flo
 cudaError_t fs_occlusion_run(const fs_bvh_view& bv, const float4* d_src, const uint32_t* d_off, uint32_t n_src, uint32_t n_rays,
                              const float lis[3], const float* d_tau, uint32_t n_bands, uint32_t max_crossings, float eps_connect,
                              float eps_offset, uint64_t seed, unsigned long long* d_acc, uint32_t* d_overflow, cudaStream_t st);
+
+// fs_bvh_build.cu: the stable LSD radix sort of the build (8 passes of 8 bits over (u64 key, u32 value); the result is back in
+// keys / vals; block_hist holds 256 fs_radix_sort_blocks(n) words) and the exclusive scan (tile_sums: ceil(n / 1024) + 1
+// words, *total = the sum)
+uint32_t fs_radix_sort_blocks(uint32_t n);
+void fs_radix_sort_u64(cudaStream_t st, uint64_t* keys, uint32_t* vals, uint64_t* keys_tmp, uint32_t* vals_tmp, uint32_t n,
+                       uint32_t* block_hist, uint64_t* launches);
+void fs_scan_u32(cudaStream_t st, const uint32_t* in, uint32_t* out, uint32_t n, uint32_t* tile_sums, uint32_t* total,
+                 uint64_t* launches);
+
+// fs_diffraction.cu: the edge set of the triangles d_verts [n_tris][3][3] for the fold threshold c_min, in ascending
+// (tri, k) (cudaMalloc'ed into *d_edges when not empty), and one query over it
+cudaError_t fs_diffraction_edges(cudaStream_t st, const float* d_verts, uint32_t n_tris, float c_min, fs_diff_edge** d_edges,
+                                 uint32_t* n_out, uint64_t* launches);
+#define FS_DIFF_CAND_MAX (1ull << 27)   // candidate pairs held at once (1 GB); a larger edge range is split
+struct fs_diff_run {
+    fs_bvh_view bv;
+    const fs_diff_edge* edges; uint32_t n_edges;
+    const float4* src; uint32_t n_src;            // [S] (position, -)
+    float lis[3];
+    float eps_offset, eps_connect, sound_speed;
+    float band_hz[FS_MAX_BANDS]; uint32_t n_bands;
+    uint2** cand; unsigned long long* cand_cap;   // the context's candidate buffer, grown on demand
+    unsigned long long* d_count;                  // candidates of one edge range
+    unsigned long long* best;                     // [S] min (bits(length) << 32 | edge rank), set to ~0 by the caller
+    uint32_t* n_paths;                            // [S] zeroed by the caller
+    unsigned long long* rays;                     // leg rays traced
+    uint32_t* overflow;
+    fs_diffraction_result* out;                   // [S] device
+};
+cudaError_t fs_diffraction_run(const fs_diff_run& a, cudaStream_t st, uint64_t* launches, uint64_t* n_cand_out);
 
 // fs_ir.cu
 struct fs_scale_table { double v[FS_PTR_TABLE]; };   // per-source 1 / n_paths, passed by value

@@ -10,3 +10,4 @@ from .capi import Context, MultiContext, FrequenSeeError, default_config, load_f
 from .capi import directivity_polar, OMNI  # noqa: F401
 from .capi import OcclusionSource, OcclusionResult  # noqa: F401
 from .capi import AcousticParams, AcousticSlot, DecayFit  # noqa: F401
+from .capi import DIFFRACTION_DTYPE  # noqa: F401

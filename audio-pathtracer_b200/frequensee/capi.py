@@ -48,6 +48,7 @@ ABI_SYMBOLS = [
     "fs_multi_set_directivity_patterns", "fs_multi_set_source_directivity",
     "fs_occlusion",
     "fs_get_acoustic_params",
+    "fs_diffraction", "fs_debug_diffraction_edges",
 ]
 
 
@@ -240,6 +241,13 @@ class AcousticParams(C.Structure):
                 ("band", AcousticSlot * MAX_BANDS)]
 
 
+# fs_diffraction_result (68 bytes): the shortest first-order diffraction path of one source
+DIFFRACTION_DTYPE = np.dtype([
+    ("found", np.uint32), ("n_paths", np.uint32), ("edge_tri", np.uint32), ("edge_k", np.uint32),
+    ("apex", np.float32, (3,)), ("length", np.float32), ("path_difference", np.float32),
+    ("gain", np.float32, (MAX_BANDS,))])
+
+
 class FrequenSeeError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__("frequensee error %d: %s" % (code, msg))
@@ -336,6 +344,8 @@ def load():
     L.fs_multi_set_source_directivity.argtypes = [vp, vp, u32]
     L.fs_occlusion.argtypes = [vp, vp, u32, vp, u32, u64, vp]
     L.fs_get_acoustic_params.argtypes = [vp, vp, u32, vp]
+    L.fs_diffraction.argtypes = [vp, vp, u32, vp, C.c_float, vp, vp]
+    L.fs_debug_diffraction_edges.argtypes = [vp, C.c_float, vp, u64, C.POINTER(C.c_uint64)]
     for n in ABI_SYMBOLS:
         if n not in ("fs_default_config", "fs_destroy", "fs_last_error", "fs_multi_destroy", "fs_multi_last_error",
                      "fs_multi_device_count", "fs_multi_context"):
@@ -590,6 +600,27 @@ class Context:
         vis = np.array([out[s].visible for s in range(S)], np.float32)
         tr = np.array([list(out[s].transmission)[:B] for s in range(S)], np.float32).reshape(S, B)
         return vis, tr
+
+    def diffraction(self, src_pos, lis_pos, min_fold_deg=30.0, band_hz=None):
+        """fs_diffraction: the shortest first-order diffraction path of every source (positions [S][3]) to the listener
+        around the scene's edges whose fold is at least min_fold_deg; band_hz [B] centre frequencies (None: 62.5 2^b Hz).
+        Returns a DIFFRACTION_DTYPE array [S]"""
+        src = np.ascontiguousarray(src_pos, dtype=np.float32).reshape(-1, 3)
+        lis = np.ascontiguousarray(lis_pos, dtype=np.float32).reshape(3)
+        hz = None if band_hz is None else np.ascontiguousarray(band_hz, dtype=np.float32).reshape(self.cfg.n_bands)
+        out = np.zeros(max(len(src), 1), DIFFRACTION_DTYPE)
+        self._ck(self.L.fs_diffraction(self.h, src.ctypes.data, len(src), lis.ctypes.data, float(min_fold_deg),
+                                       None if hz is None else hz.ctypes.data, out.ctypes.data))
+        return out[:len(src)]
+
+    def debug_diffraction_edges(self, min_fold_deg=30.0):
+        """fs_debug_diffraction_edges: the edge set for a fold threshold as (tri, k) pairs [n][2] uint32, ascending"""
+        n = C.c_uint64(0)
+        self._ck(self.L.fs_debug_diffraction_edges(self.h, float(min_fold_deg), None, 0, C.byref(n)))
+        out = np.zeros((n.value, 2), np.uint32)
+        if n.value:
+            self._ck(self.L.fs_debug_diffraction_edges(self.h, float(min_fold_deg), out.ctypes.data, n.value, C.byref(n)))
+        return out
 
     def noise_stats(self):
         """fs_get_noise: per-source noise of the last update as a dict of numpy arrays -- n_paths [S], no_energy [S] bool,

@@ -500,6 +500,66 @@ typedef struct fs_occlusion_result {
 int fs_occlusion(fs_ctx* ctx, const fs_occlusion_source* src, uint32_t n_sources, const float lis_pos[3],
                  uint32_t max_crossings /* 0..16 */, uint64_t seed, fs_occlusion_result* out /* [n_sources] */);
 
+/* ---- first-order edge diffraction of the direct path -----------------------------------------------
+ * Where fs_occlusion reports the straight path blocked, sound still bends around the obstacle's edges: it arrives from the
+ * edge, later and duller.  For every source this finds the shortest path S -> P -> L via one point P on one edge of the
+ * scene, counts such paths, and gives the per-band energy attenuation of the shortest.
+ * Edges, a pure function of the current triangle positions and min_fold_deg:
+ *   triangle edge k of triangle tri = (v_k, v_(k+1) mod 3).  Two triangle edges are the same scene edge iff their endpoints
+ *     are equal as float positions (unordered; -0.0 equals +0.0; compared exactly, no welding tolerance).  Degenerate
+ *     triangles (zero cross product) and zero-length edges hold no edge.  An edge is named by (tri, k) of the lowest triangle
+ *     id that holds it; edges are ordered by ascending (tri, k), the tie-break everywhere.
+ *   held by exactly two triangles: a wedge.  u1, u2 = the unit vectors from the edge into each face, perpendicular to it; the
+ *     fold phi = pi - angle(u1, u2) (0: a flat seam, pi: a fin).  Kept iff dot(u1, u2) >= c_min, c_min = (float)(-cos(phi_min))
+ *     computed in double.  The wedge's solid is the smaller sector between u1 and u2 (no winding needed): concave corners,
+ *     such as the inside of a room, never diffract.
+ *   held by one triangle (a boundary edge or a T-junction): a thin screen with the one face half-line u1; always kept.
+ *   held by three or more triangles: non-manifold, never diffracts.
+ * Path via the edge A -> B (A = the lexicographically smaller endpoint) for source S and listener L:
+ *   r_S, r_L = the distances of S and L from the edge line, both > eps_offset.
+ *   apex P = A + x u_hat, x = s_a + (l_a - s_a) r_S / (r_S + r_L) (s_a, l_a the projections onto the line; the minimiser of
+ *     |SP| + |PL| along it), valid iff 0 <= x <= |AB|.
+ *   shadow: in the plane perpendicular to the edge, the segment between the projections of S - A and L - A strictly crosses
+ *     every face half-line (u1 and u2 of a wedge, u1 of a screen): S and L are both outside the solid and their angular
+ *     separation through the exterior exceeds 180 degrees.  Sign tests on cross products, no trigonometry.
+ *   legs: one any-hit ray from S toward P and one from L toward P, tmax = |leg| - eps_connect (<= 0: clear), like the
+ *     trace's connection ray; both must be clear.
+ *   length = |SP| + |PL|, path difference z = max(length - |SL|, 0),
+ *   gain_b = max(1 / (3 + ((40 z) f_b) / c), 0.01): Maekawa's 10 lg(3 + 20 N), N = 2 z / lambda, limited to 20 dB (ISO
+ *     9613-2, single diffraction).  c = fs_config.sound_speed; f_b = band_hz[b], or 62.5 2^b Hz when band_hz is NULL.
+ *   The float arithmetic, in its fixed order, is that of audio-pathtracer_b200/csrc/fs_diffraction.h.
+ * Result: among every valid path the one with the smallest length (the smallest z, so the largest gain in every band), ties
+ *   to the lower (tri, k).
+ * Edge cache: the edge set is built by the first fs_diffraction or fs_debug_diffraction_edges after an fs_scene_commit or
+ * fs_scene_refit, or after a change of min_fold_deg, and kept until then (commit and refit cost what they did before).
+ * Not modelled: paths over two or more edges (a thick obstacle seen from opposite sides gives found = 0), diffraction inside
+ * the histogram or the IR, phase-accurate UTD / BTM edge models, vertex welding with a tolerance; combining the result with
+ * fs_occlusion is the host's policy.
+ * State and errors, all checked before anything is enqueued (a rejected call changes nothing): FS_ERR_STATE before
+ * fs_scene_commit or while moved vertices await fs_scene_refit; FS_ERR_INVALID for NULL pointers, n_sources 0 or > 4096, a
+ * non-finite or > 1e18 position, min_fold_deg non-finite or outside [0, 180], a band_hz entry non-finite or <= 0.
+ * FS_ERR_OVERFLOW: the traversal stack overflowed and the results are invalid; from a flag of this call's own (the trace's
+ * sticky flag is neither set nor cleared).
+ * Runs on the context stream after the work already enqueued there and synchronises.  Reads and writes nothing of the
+ * histogram, the noise moments, the IRs, the convolver, the directivity state or fs_stats (except kernel_launches).
+ * Several GPUs: call fs_diffraction(fs_multi_context(m, 0), ...). */
+typedef struct fs_diffraction_result {
+    uint32_t found;              /* 1: at least one valid path; 0: everything below is 0 */
+    uint32_t n_paths;            /* valid first-order paths of this source (edges passing every test) */
+    uint32_t edge_tri, edge_k;   /* the shortest path's edge */
+    float    apex[3];            /* P */
+    float    length;             /* |SP| + |PL|, metres: the host's distance attenuation and delay use it */
+    float    path_difference;    /* z */
+    float    gain[FS_MAX_BANDS]; /* bands >= n_bands: 0 */
+} fs_diffraction_result;         /* 68 bytes */
+
+int fs_diffraction(fs_ctx* ctx, const float* src_pos /* [n_sources][3] */, uint32_t n_sources, const float lis_pos[3],
+                   float min_fold_deg /* [0, 180] */, const float* band_hz /* [n_bands] or NULL */,
+                   fs_diffraction_result* out /* [n_sources] */);
+/* debug / parity: the edge set for a threshold as (tri, k) pairs in ascending order; *n_out = the number of edges, of which
+ * the first min(n, cap) are written to out [cap][2] when out is not NULL (the sizing convention of fs_load_float_array) */
+int fs_debug_diffraction_edges(fs_ctx* ctx, float min_fold_deg, uint32_t* out, uint64_t cap, uint64_t* n_out);
+
 /* single rays through the device BVH (parity tests of the intersector):
  * rays: [n][6] (origin, direction); out_t [n] (inf on miss), out_tri [n] (0xffffffff on miss) */
 int fs_debug_closest_hits(fs_ctx* ctx, const float* rays, uint64_t n, float* out_t, uint32_t* out_tri);

@@ -89,6 +89,10 @@ public:
     float OcclusionRadius = 0.0f;
     uint32_t OcclusionRays = 64;
     fs_occlusion_result LastOcclusion{};
+    // first-order edge diffraction of the direct path (UAudioRayTracingSubsystem::UpdateDiffraction, fs_diffraction): the
+    // shortest path around one edge of the scene -- where the dry sound arrives from (Apex), how far it travels (Length) and
+    // its per-band filter (Gain) when LastOcclusion reports the straight path blocked
+    fs_diffraction_result LastDiffraction{};
     // room-acoustic parameters of this source's histogram in the last UpdateSources() (UpdateAcousticParams,
     // fs_get_acoustic_params): decay times, clarity and centre time per band and broadband, the inputs of a parametric reverb
     fs_acoustic_params LastAcoustics{};
@@ -308,6 +312,24 @@ public:
         std::vector<fs_occlusion_result> res(S);
         if (Ctx->Check(fs_occlusion(Ctx->Get(), desc.data(), S, lis, MaxCrossings, OcclusionSeed, res.data())) != FS_OK) return;
         for (uint32_t s = 0; s < S; ++s) ActiveSources[s]->LastOcclusion = res[s];
+    }
+
+    // First-order edge diffraction of every active source in ONE fs_diffraction call: each component's LastDiffraction is
+    // filled, over the edges whose fold is at least MinFoldDeg, with the default band centres 62.5 2^b Hz.  No histogram or
+    // IR is touched.
+    void UpdateDiffraction(float MinFoldDeg)
+    {
+        if (ActiveSources.empty() || !Commit()) return;
+        const float lis[3] = {PawnLocation.X, PawnLocation.Y, PawnLocation.Z};
+        const uint32_t S = (uint32_t)ActiveSources.size();
+        std::vector<float> pos(3 * (size_t)S);
+        for (uint32_t s = 0; s < S; ++s) {
+            const FVector3f L = ActiveSources[s]->GetActorLocation();
+            pos[3 * s] = L.X; pos[3 * s + 1] = L.Y; pos[3 * s + 2] = L.Z;
+        }
+        std::vector<fs_diffraction_result> res(S);
+        if (Ctx->Check(fs_diffraction(Ctx->Get(), pos.data(), S, lis, MinFoldDeg, nullptr, res.data())) != FS_OK) return;
+        for (uint32_t s = 0; s < S; ++s) ActiveSources[s]->LastDiffraction = res[s];
     }
 
     // The room-acoustic parameters of every source of the last UpdateSources() in ONE fs_get_acoustic_params call: each
