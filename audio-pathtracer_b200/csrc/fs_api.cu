@@ -111,6 +111,9 @@ int fs_create(const fs_config* cfg, fs_ctx** out)
     if ((uint32_t)((double)cfg->bin_ms * 1e-3 * cfg->sample_rate + 0.5) < 1u)
         return fail(nullptr, FS_ERR_INVALID, "bin_ms * sample_rate / 1000 must be at least one sample");
     if (!(cfg->ir_lowpass > 0.0f) || cfg->ir_lowpass > 1.0f) return fail(nullptr, FS_ERR_INVALID, "ir_lowpass must be in (0,1]");
+    // an empty bin passes a threshold <= 0 and maps to 0 / sqrt(0) = NaN; a NaN threshold silently zeroes the IR
+    if (!(cfg->ir_threshold > 0.0f) || !isfinite(cfg->ir_threshold))
+        return fail(nullptr, FS_ERR_INVALID, "ir_threshold must be finite and > 0");
     if ((cfg->flags & FS_FLAG_NOISE_STATS) && (cfg->flags & (FS_FLAG_CONNECT_ALL | FS_FLAG_MIS)))
         return fail(nullptr, FS_ERR_INVALID, "FS_FLAG_NOISE_STATS needs the endpoint connection (not with FS_FLAG_CONNECT_ALL / "
                                              "FS_FLAG_MIS: a pair adds to several bins there)");
@@ -1294,6 +1297,10 @@ int fs_build_ir_from_energy(fs_ctx* ctx, uint32_t source, const float* energy, f
 {
     if (!ctx) return FS_ERR_INVALID;
     if (!energy) return fail(ctx, FS_ERR_INVALID, "fs_build_ir_from_energy: null energy");
+    // a negative entry at or above the threshold maps to NaN, which the low-pass spreads over the rest of the IR
+    for (uint32_t k = 0; k < ctx->cfg.n_bins; ++k)
+        if (!(energy[k] >= 0.0f) || !isfinite(energy[k]))
+            return fail(ctx, FS_ERR_INVALID, "fs_build_ir_from_energy: energy entries must be finite and >= 0");
     dev_guard g(ctx->device);
     return ir_common(ctx, 0, source, energy, ir_out);
 }

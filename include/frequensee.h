@@ -138,7 +138,9 @@ typedef struct fs_config {
     float    air_absorption[FS_MAX_BANDS]; /* per metre per band (AIR_ABSORPTION_FACTOR, SUB.cpp:395) */
     uint32_t sample_rate;      /* SampleRate = 48000 (COMP.h:133) */
     uint32_t n_channels;       /* NumChannels = 2 (COMP.h:135) */
-    float    ir_threshold;     /* kEnergyThreshold = 1e-6 (COMP.cpp:322) */
+    float    ir_threshold;     /* kEnergyThreshold = 1e-6 (COMP.cpp:322).  Must be finite and > 0 (fs_create returns
+                                  FS_ERR_INVALID otherwise): a bin with |E| >= threshold maps to E / sqrt(E sqrt(4 pi)), so
+                                  at 0 every empty bin is 0 / 0 = NaN, and a NaN threshold would zero the whole IR */
     float    ir_lowpass;       /* FilterCoefficient = 0.25 (COMP.cpp:366) */
     uint32_t conv_block;       /* AudioCallbackBufferFrameSize = 1024 (Config/DefaultEngine.ini:15) */
     uint32_t conv_clamp;       /* clamp to +-1 (REV.cpp:162-168) */
@@ -582,7 +584,9 @@ int fs_build_ir_all(fs_ctx* ctx, uint32_t n_sources, float* ir_out);
  * octave-band noise carrier (f_b = 62.5 * 2^b Hz, Philox noise keyed by noise_seed through two RBJ band-pass biquads);
  * ir[c][t] = sum_b ramp_b[t] * carrier[c][b][t], no low-pass.  Publishes to conv_source's convolver like fs_build_ir_to. */
 int fs_build_ir_bands(fs_ctx* ctx, uint32_t hist_source, uint32_t conv_source, uint64_t noise_seed, float* ir_out);
-/* seam 1 of the reference taken literally: EnergyBuffer float[K] -> IR (AddEnergyAtDelay users) */
+/* seam 1 of the reference taken literally: EnergyBuffer float[K] -> IR (AddEnergyAtDelay users).  Every entry must be
+ * finite and >= 0: otherwise FS_ERR_INVALID, checked on the host before anything is enqueued, so the source's IR and
+ * convolver are left as they were (a negative entry would map to NaN and the low-pass would carry it through the IR). */
 int fs_build_ir_from_energy(fs_ctx* ctx, uint32_t source, const float* energy /*[K]*/, float* ir_out);
 /* install an already reduced histogram (host [S][B][K]) and its path count, e.g. after an NCCL reduce */
 int fs_set_histogram(fs_ctx* ctx, const uint64_t* hist, uint32_t n_sources, uint64_t n_paths);
